@@ -12,6 +12,9 @@ Own arm (default):  python bench.py --gpus N --steps K --warmup W
     windows -> cutoff -> coverage -> ROH, fused) -> ROH records to the host.  Sharded by individual: every rank holds
     2,000 individuals (weak scaling).
     `value` has the packed matrix resident in HBM; `e2e` goes through the C ABI with pinned HOST buffers.
+    --dump-outputs DIR writes what the last resident step returned (freq, keep mask, thinned KDE windows, ROH records)
+    as DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output.  Under N ranks every rank
+    writes its ROH records as roh_rank<r>.npy, with individuals counted within the rank.
 
 Reference arm:      python bench.py --impl reference --gpus N --steps K --warmup W
     The reference's own calcLODWindows + assembleROHWindows (oracle/_ref/ref_driver, compiled from
@@ -258,6 +261,22 @@ class CpuSample:
         return time.perf_counter() - t0, sorted(sum(parts, []))
 
 
+def dump_outputs(out_dir, arrays, limit=64 << 20, seed=0):
+    """Writes each array as out_dir/<name>.npy, in float64 (bool as float32).  If together they would exceed `limit`
+    bytes, every array keeps the same fixed, seeded fraction of its rows, and the row indices kept go to <name>_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, np.float32 if v.dtype == np.bool_ else np.float64) for k, v in arrays.items() if v is not None}
+    total = sum(v.nbytes for v in arrays.values())
+    frac = 1.0 if total <= limit else (limit - (1 << 16)) / (total + sum(8 * len(v) for v in arrays.values()))
+    rng = np.random.default_rng(seed)
+    for k, v in arrays.items():
+        if frac < 1.0:
+            rows = np.sort(rng.choice(len(v), min(len(v), max(1, int(len(v) * frac))), replace=False))
+            np.save(os.path.join(out_dir, k + "_rows.npy"), rows.astype(np.float64))
+            v = v[rows]
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -272,7 +291,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--exact", action="store_true", help="whole-segment chains in pass 2")
     ap.add_argument("--no-configs", action="store_true", help="skip the full-size C4 / C3 runs that follow the headline at N=1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     a.warmup = max(a.warmup, 0)
     # exactly one JSON line on stdout: libraries (NCCL prints its version) get stderr
     sys.stdout.flush()
@@ -445,6 +469,9 @@ def main():
 
     g.put_packed_dev(rows_dev.data_ptr(), row_bytes)
     ms_res, (kms, sqms), launches, clocks = timed(True, a.steps, a.warmup, True)
+    # copied now: the steps that follow overwrite the page-locked buffers these arrays live in
+    last_outputs = {name: None if state[k] is None else np.array(state[k])
+                    for name, k in (("freq", "freq"), ("keep", "keep"), ("kde_windows", "thin"), ("roh", "roh"))}
     units_local = state["stats"]["units"]
     units_total = units_local * world
     value = units_total * a.steps / (ms_res / 1e3)
@@ -598,6 +625,11 @@ def main():
         except Exception as e:
             cfgs["error"] = repr(e)[:300]
         line["configs"] = cfgs
+    if a.dump_outputs:
+        # ROH records are (individual, chromosome, first kept SNP, last kept SNP), the individual counted within this rank
+        # (rank r holds the global individuals r * n_ind ...); freq / keep / kde_windows reach rank 0 only
+        suffix = "_rank%d" % rank if world > 1 else ""
+        dump_outputs(a.dump_outputs, {k + suffix: v for k, v in last_outputs.items()})
     if rank == 0:
         emit(line)
     if dist is not None:
