@@ -311,4 +311,27 @@ GHD uint32_t plan_window(const uint4& hd, uint32_t x0, uint32_t x1, uint32_t x2)
     return lo;
 }
 
+// Output half-word q of one row, gathered from the row's uncompacted half-words hin by its plan head hd and segments sg
+GHD uint32_t plan_gather(const uint4& hd, const uint4* sg, const uint32_t* hin)
+{
+    if (hd.x & 0x100u) return plan_window(hd, hin[hd.y], plan_need1(hd) ? hin[hd.y + 1] : 0u, plan_need2(hd) ? hin[hd.y + 2] : 0u);
+    uint32_t h = hd.w;
+    for (uint32_t k = 0; k < hd.x; ++k) { const uint4 g = sg[k]; h |= ((hin[g.x] >> g.y) & g.z) << g.w; }
+    return h;
+}
+
+// Compacted words [wlo, wlo + n) of one row into out[0 .. n): what K3 writes there, built from the uncompacted row hin
+// (32-bit view) by the plan (head / segs of every output half-word, bound.cuh:plan_half).  Half-words from SNP L on read
+// as missing calls.  The plan is the same for every row: on the GPU a warp's lanes read it with uniform loads and
+// only the row loads differ between lanes (the pruned walker, kernels.cu:walk_units_kernel).
+GHD void plan_slice(const uint4* head, const uint4* segs, long long L, const uint32_t* hin, long long wlo, int n, uint64_t* out)
+{
+    for (int j = 0; j < n; ++j) {
+        const long long q = 2 * (wlo + j);
+        const uint32_t lo = 16 * q < L ? plan_gather(head[q], segs + q * kPlanSegMax, hin) : 0xffffffffu;
+        const uint32_t hi = 16 * (q + 1) < L ? plan_gather(head[q + 1], segs + (q + 1) * kPlanSegMax, hin) : 0xffffffffu;
+        out[j] = (uint64_t)hi << 32 | lo;
+    }
+}
+
 }  // namespace garlic

@@ -81,7 +81,7 @@ struct garlic_gpu {
     std::vector<Segment> p2_segs;
     std::vector<Item> p2_items;
     Item* d_items_p2 = nullptr;
-    int p2_W = 0, p2_tile = 0, p2_chunk = 0;
+    int p2_W = 0, p2_tile = 0, p2_chunk = 0, p2_slice = 0;
     uint64_t tables_gen = 0, p2_gen = 0;
     size_t sorted_cap = 0;
     unsigned out_cap = 0, amb_cap = 0;
@@ -98,7 +98,8 @@ struct garlic_gpu {
     uint32_t* d_badbits = nullptr; // bit i: no window may hold SNPs i-1 and i (gap / centromere pair, chromosome start)
     int* d_thin = nullptr;         // segment + chromosome tables of the thinned pass 1
     // K3 is deferred to the first consumer of the compacted rows so that it can run fused with the pruning bound
-    // (squeeze.cu): filter() only builds the plan
+    // (squeeze.cu): filter() only builds the plan.  The pruned pass 2 of window sizes from 32 on never needs them: its
+    // bound reads the uncompacted rows and its walker compacts its candidates' slices (kernels.cu:walk_units_kernel)
     bool geno_pending = false;
     uint4 *d_plan_head = nullptr, *d_plan_seg = nullptr;
     int2* d_plan_rng = nullptr;
@@ -114,7 +115,7 @@ struct garlic_gpu {
     int2* d_units = nullptr;       // work queue of the pruned pass 2: (item, first candidate)
     unsigned* d_nunits = nullptr;  // [0] units appended, [1] candidate pairs (inside the block of d_cnt: ensure_zero_block)
     size_t zero_cap = 0, zero_n = 0;
-    cudaEvent_t ev_sq0 = nullptr, ev_sq1 = nullptr;   // around the last fused compaction + bound launch
+    cudaEvent_t ev_sq0 = nullptr, ev_sq1 = nullptr;   // around the last compaction and / or bound launch
     bool sq_timed = false;
     int item_pieces = 1;           // pieces per item of the pruned pass (GARLIC_ITEM_PIECES)
     bool prune = true;             // GARLIC_NO_PRUNE=1 disables the pruning pass
@@ -977,13 +978,8 @@ int garlic_gpu_filter(garlic_gpu_t* h, int oob, const int32_t* chr_param, const 
     if (n_kept) *n_kept = L;
     if (L < 1) FAIL("filter: no polymorphic loci left");
     h->row_words = (((L + kPad + 31) >> 5) + 3) & ~(int64_t)1;   // even: rows are whole 16-byte quads
-    // the slack words behind each row are only ever over-read (their lookups are masked), so they need
-    // no defined content; a fresh allocation is filled once so that dumps stay reproducible
-    const bool fresh = h->cap.find((void*)&h->d_geno) == h->cap.end() || !h->d_geno ||
-                       h->cap[(void*)&h->d_geno] < (size_t)h->n_ind * h->row_words * 8;
-    if (dev_alloc(h, &h->d_geno, (size_t)h->n_ind * h->row_words)) return 1;
-    if (fresh) CK(cudaMemsetAsync(h->d_geno, 0xff, (size_t)h->n_ind * h->row_words * 8, h->stream));
-    // the compaction itself waits for its first consumer (ensure_geno): here only its plan, from the gather list
+    // the compaction itself, and the compacted matrix, wait for their first consumer (ensure_geno): here only its plan,
+    // from the gather list
     h->n_pieces = (int)((L + kPiece - 1) / kPiece);
     {
         const long long n_q = 16ll * (h->n_pieces + 4);
@@ -1265,6 +1261,16 @@ static bool can_bound(const garlic_gpu* h, int W)
     return h->prune && h->tables && !h->have_gl && W >= kBoundMinW && W <= 1280;   // (a piece plus its lead-in must fit the walker's table tile)
 }
 
+// Will the pruned pass 2 of window size W run as work units (walk_units_kernel)?  That walker builds its candidates'
+// compacted slices itself, so the pass in front of it is the bound alone.  Conservative in the item table's tile (the
+// largest an item of kPiece * item_pieces owned SNPs and its W - 1 lead-in windows can need): a false "no" only costs
+// the compaction the pass did before.
+static bool units_walk(const garlic_gpu* h, int W)
+{
+    const int span = kPiece * h->item_pieces + W - 2;          // slide steps of the longest item
+    return can_bound(h, W) && !bound_partial(W) && 32 * ((span + 31) / 32) + W <= kTileSnpsMax;
+}
+
 static int ensure_bound_tables(garlic_gpu* h, int W)
 {
     if (h->bound_tables_W == W) return 0;
@@ -1307,15 +1313,21 @@ static int alloc_pmax(garlic_gpu* h)
 static int ensure_geno(garlic_gpu* h, int W_hint)
 {
     if (!h->geno_pending) return 0;
+    // the slack words behind each row are only ever over-read (their lookups are masked), so they need
+    // no defined content; a fresh allocation is filled once so that dumps stay reproducible
+    const bool fresh = h->cap.find((void*)&h->d_geno) == h->cap.end() || !h->d_geno ||
+                       h->cap[(void*)&h->d_geno] < (size_t)h->n_ind * h->row_words * 8;
+    if (dev_alloc(h, &h->d_geno, (size_t)h->n_ind * h->row_words)) return 1;
+    if (fresh) CK(cudaMemsetAsync(h->d_geno, 0xff, (size_t)h->n_ind * h->row_words * 8, h->stream));
     int c2 = 0;
-    if (W_hint > 0 && can_bound(h, W_hint)) {
+    if (W_hint > 0 && can_bound(h, W_hint) && h->bound_W != W_hint) {
         if (ensure_bound_tables(h, W_hint)) return 1;
         if (alloc_pmax(h)) return 1;
         c2 = bound_c2(W_hint);
     }
     const SqueezeParams Q = squeeze_params(h, true, W_hint);
     CK(cudaEventRecord(h->ev_sq0, h->stream));
-    LAUNCH(launch_squeeze_bound(Q, true, c2, h->stream));
+    LAUNCH(launch_squeeze_bound(Q, true, true, c2, h->stream));
     CK(cudaEventRecord(h->ev_sq1, h->stream));
     h->sq_timed = true;
     h->geno_pending = false;
@@ -1334,6 +1346,7 @@ static int prepare_p2_items(garlic_gpu* h, int W)
     h->p2_chunk = 0;
     for (const Item& it : h->p2_items) h->p2_chunk = std::max(h->p2_chunk, it.own_hi - it.own_lo);
     h->p2_tile = items_tile_snps(h->p2_items, W);
+    h->p2_slice = items_slice_words(h->p2_items, W);
     if (dev_alloc(h, &h->d_items_p2, h->p2_items.size() + 1)) return 1;
     if (!h->p2_items.empty())
         CK(cudaMemcpyAsync(h->d_items_p2, h->p2_items.data(), h->p2_items.size() * sizeof(Item), cudaMemcpyHostToDevice, h->stream));
@@ -1341,16 +1354,19 @@ static int prepare_p2_items(garlic_gpu* h, int W)
     return 0;
 }
 
-// piece maxima for window size W present (fused with the compaction if that is still pending)
+// Piece maxima for window size W present, without compacting rows where it can: over the compacted rows if they
+// exist, else over the uncompacted ones, compacted in registers only.  Window sizes below 32 whose rows are not
+// compacted yet take the fused pass instead: their pruned walker (launch_walk) reads compacted rows.
 static int ensure_bound(garlic_gpu* h, int W)
 {
-    if (ensure_geno(h, W)) return 1;
     if (h->bound_W == W) return 0;
+    if (h->geno_pending && bound_partial(W)) return ensure_geno(h, W);
     if (ensure_bound_tables(h, W)) return 1;
     if (alloc_pmax(h)) return 1;
-    const SqueezeParams Q = squeeze_params(h, false, W);
+    const bool raw = h->geno_pending;
+    const SqueezeParams Q = squeeze_params(h, raw, W);
     CK(cudaEventRecord(h->ev_sq0, h->stream));
-    LAUNCH(launch_squeeze_bound(Q, false, bound_c2(W), h->stream));
+    LAUNCH(launch_squeeze_bound(Q, raw, false, bound_c2(W), h->stream));
     CK(cudaEventRecord(h->ev_sq1, h->stream));
     h->sq_timed = true;
     h->bound_W = W;
@@ -1487,7 +1503,9 @@ static int windows_common(garlic_gpu_t* h, int winsize, int step, int weighted, 
         if (side) {
             if (begin_side(h)) return 1;                           // the side stream takes over behind the windows …
             ws = h->aux_stream;
-            if (ensure_geno(h, winsize)) return 1;                 // … and the main stream goes on with the compaction
+            // … and the main stream goes on with the bound for pass 2, fused with the compaction unless pass 2 will
+            // not need compacted rows
+            if (units_walk(h, W) ? ensure_bound(h, W) : ensure_geno(h, winsize)) return 1;
         }
         tl_mark(h, "windows:squeeze-enqueued");
         // the GPU is busy: the host gets pass 2's items ready meanwhile
@@ -1586,7 +1604,8 @@ int garlic_gpu_call_roh(garlic_gpu_t* h, int winsize, double cutoff, double over
     int cut_ok = 0;
     bound_cut_store(cutoff, 1.0, &cut_ok);
     bool prune = !exact && !weighted && can_bound(h, W) && cut_ok;
-    if (ensure_geno(h, prune ? W : 0)) return 1;
+    // the bound, and the compacted rows unless the pruned walker will build its own slices (checked again below)
+    if (prune && units_walk(h, W) ? ensure_bound(h, W) : ensure_geno(h, prune ? W : 0)) return 1;
     // garlic-roh.cpp:422-424, compared against integers at :466 and :477
     double thr_d = overlap_frac * W;
     thr_d = (thr_d >= 1) ? thr_d : 1;
@@ -1608,6 +1627,7 @@ int garlic_gpu_call_roh(garlic_gpu_t* h, int winsize, double cutoff, double over
         prune = h->p2_tile <= kTileSnpsMax && (int64_t)h->p2_items.size() * h->n_ind < (1ll << 31);
         if (prune) chunk = h->p2_chunk;
     }
+    if (!(prune && !bound_partial(W)) && ensure_geno(h, 0)) return 1;   // every walker but the work units reads compacted rows
     const Item* d_its = h->d_items;                    // the items in use: the cached piece-aligned ones, or `items`
     const std::vector<Item>* its = &items;
     if (prune) {
@@ -1685,7 +1705,12 @@ int garlic_gpu_call_roh(garlic_gpu_t* h, int winsize, double cutoff, double over
         P.hist = h->d_hist;
         // window sizes below 32 leave a quarter of the pairs (a short window is homozygous by chance often enough): eight-warp
         // CTAs over the candidate lists share one table tile among 256 candidates, where a work unit would stage it for 64
-        if (prune_now && !bound_partial(W)) LAUNCH(launch_walk_units(P, d_its, h->d_units, h->d_nunits, unit_cap, tile_snps, cl, h->stream));
+        if (prune_now && !bound_partial(W)) {
+            RawRows R;                                 // (the compacted rows, if another consumer has made them)
+            R.rows = h->geno_pending ? h->d_geno0 : nullptr; R.row_words = h->row_words0;
+            R.head = h->d_plan_head; R.segs = h->d_plan_seg; R.L = h->L;
+            LAUNCH(launch_walk_units(P, R, d_its, h->d_units, h->d_nunits, unit_cap, tile_snps, h->p2_slice, cl, h->stream));
+        }
         else if (prune_now) LAUNCH(launch_walk(P, d_its, n_its, false, true, false, tile_snps, cl, h->stream));
         else if (launch_any_walk(h, P, d_its, n_its, weighted, true, false, tile_snps)) return 1;
         CK(cudaEventRecord(h->ev1, h->stream));
@@ -1719,6 +1744,7 @@ int garlic_gpu_call_roh(garlic_gpu_t* h, int winsize, double cutoff, double over
         }
         if (n_amb > h->amb_cap) {   // pathological: (nearly) everything ambiguous → exact everywhere
             exact = 1; prune = false;
+            if (ensure_geno(h, 0)) return 1;
             build_items(h->chr_off, W, segs, 0, 0, items);
             if (upload_items(h, items)) return 1;
             d_its = h->d_items; its = &items;
@@ -1741,6 +1767,7 @@ int garlic_gpu_call_roh(garlic_gpu_t* h, int winsize, double cutoff, double over
     // distance of the cutoff: one whole-segment launch per distinct segment
     int64_t n_amb_pairs = 0;
     if (!ambs.empty()) {
+        if (ensure_geno(h, 0)) return 1;                  // whole-segment chains read compacted rows
         std::map<int, std::vector<int>> by_seg;
         for (const RohRec& a : ambs) by_seg[a.tag].push_back(a.ind);
         std::vector<RohRec> fixed;

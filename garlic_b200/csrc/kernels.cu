@@ -8,6 +8,7 @@
 #include <algorithm>
 #include "common.cuh"
 #include "walk.cuh"
+#include "bound.cuh"
 #include "kernels.h"
 
 namespace garlic {
@@ -111,16 +112,22 @@ walk_kernel(const WalkParams P, const Item* __restrict__ items, int n_items, int
 // K5 pass 2 on the candidates the bound left (squeeze.cu:select_kernel): one CTA of two warps per work unit = up to 64
 // candidate individuals of one piece-sized item, taken from a device-resident queue (the host never learns its length).
 // The item's slice of the per-SNP table (about 14 KB at W = 50) is staged by one bulk copy per unit; two-warp CTAs keep
-// the barrier around it cheap and let some twenty units share an SM.
+// the barrier around it cheap and let some ten units share an SM.  The compacted matrix is never written on this path:
+// while the copy lands, every lane builds its candidate's compacted words of the item (about 14 at W = 50) from the
+// uncompacted row by the compaction plan (bound.cuh:plan_slice) into its own stretch of shared memory — a few percent of
+// the rows are read, where the compaction would have written all of them.  Where a compacted matrix exists already
+// (R.rows == nullptr: another consumer needed it) the lanes read their rows from there, as the other walkers do.
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kUnitThreads, 16)
-walk_units_kernel(const WalkParams P, const Item* __restrict__ items, const int2* __restrict__ units,
-                  const unsigned* __restrict__ n_units, unsigned unit_cap, int tile_bytes, const int* __restrict__ cand_list,
-                  const unsigned* __restrict__ cand_cnt, int cand_stride)
+walk_units_kernel(const WalkParams P, const RawRows R, const Item* __restrict__ items, const int2* __restrict__ units,
+                  const unsigned* __restrict__ n_units, unsigned unit_cap, int tile_bytes, int slice_stride,
+                  const int* __restrict__ cand_list, const unsigned* __restrict__ cand_cnt, int cand_stride)
 {
     extern __shared__ __align__(128) unsigned char walk_smem[];
+    // layout: [tile (tile_bytes)] [slices: slice_stride words per thread] [ring: NW words per thread] [mbarrier]
     unsigned char* tile_s = walk_smem;
-    uint32_t* ring_smem = reinterpret_cast<uint32_t*>(walk_smem + tile_bytes);
+    uint64_t* slice_s = reinterpret_cast<uint64_t*>(walk_smem + tile_bytes) + (size_t)threadIdx.x * slice_stride;
+    uint32_t* ring_smem = reinterpret_cast<uint32_t*>(walk_smem + tile_bytes + (size_t)slice_stride * kUnitThreads * 8);
     const int NW = ((P.W + 31) >> 5) + 1;
     uint64_t* bar = reinterpret_cast<uint64_t*>(ring_smem + NW * kUnitThreads);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -141,33 +148,40 @@ walk_units_kernel(const WalkParams P, const Item* __restrict__ items, const int2
             mbar_expect_tx(bar, bytes);
             tma_load_1d(tile_s, P.lut + (int64_t)it.w0 * 4, bytes, bar);
         }
+        const bool busy = warp * 32 < n_lanes;
+        const int k = warp * 32 + lane;
+        const bool active = k < n_lanes;
+        const int kk = active ? k : n_lanes - 1;
+        const int ind = busy ? list[kk] : 0;
+        const int wlo = it.w0 >> 5;
+        if (busy && R.rows) {
+            const int n_w = ((it.w0 + P.W) >> 5) + nblk + 2 - wlo;   // (items_slice_words)
+            plan_slice(R.head, R.segs, R.L, reinterpret_cast<const uint32_t*>(R.rows + (int64_t)ind * R.row_words), wlo, n_w, slice_s);
+        }
         mbar_wait(bar, phase);
         phase ^= 1u;
-        if (warp * 32 < n_lanes) {
-            const int k = warp * 32 + lane;
-            const bool active = k < n_lanes;
-            const int kk = active ? k : n_lanes - 1;
+        if (busy)
             walk_item<0, true, false>(P, it, kk, active, ring_smem + threadIdx.x, kUnitThreads,
-                                      reinterpret_cast<const char*>(tile_s), it.w0, list[kk]);
-        }
+                                      reinterpret_cast<const char*>(tile_s), it.w0, ind, R.rows ? slice_s : nullptr, wlo);
         __syncthreads();   // both warps are done with the tile before the next copy lands
     }
 }
 
-cudaError_t launch_walk_units(const WalkParams& P, const Item* items, const int2* units, const unsigned* n_units,
-                              unsigned unit_cap, int tile_snps, const CandList& cl, cudaStream_t st)
+cudaError_t launch_walk_units(const WalkParams& P, const RawRows& R, const Item* items, const int2* units, const unsigned* n_units,
+                              unsigned unit_cap, int tile_snps, int slice_words, const CandList& cl, cudaStream_t st)
 {
     const int NW = ((P.W + 31) >> 5) + 1;
     const int tile_bytes = tile_snps * 32;
-    const size_t smem = (size_t)tile_bytes + (size_t)NW * kUnitThreads * sizeof(uint32_t) + 16;
+    const int slice_stride = R.rows ? slice_words | 1 : 0;   // odd: the lanes' 8-byte reads of the same word k fall in distinct banks
+    const size_t smem = (size_t)tile_bytes + (size_t)slice_stride * kUnitThreads * 8 + (size_t)NW * kUnitThreads * sizeof(uint32_t) + 16;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(walk_units_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
     int per_sm = (int)((227 * 1024) / (smem + 1024));
     per_sm = per_sm > 16 ? 16 : (per_sm < 1 ? 1 : per_sm);
-    walk_units_kernel<<<148 * per_sm, kUnitThreads, smem, st>>>(P, items, units, n_units, unit_cap, tile_bytes, cl.list, cl.cnt,
-                                                               cl.stride);
+    walk_units_kernel<<<148 * per_sm, kUnitThreads, smem, st>>>(P, R, items, units, n_units, unit_cap, tile_bytes, slice_stride,
+                                                               cl.list, cl.cnt, cl.stride);
     return cudaGetLastError();
 }
 

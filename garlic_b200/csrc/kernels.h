@@ -21,9 +21,20 @@ struct CandList {
 // tile_snps > 0: every item touches at most tile_snps SNPs → stage its table slice in shared memory
 cudaError_t launch_walk(const WalkParams& P, const Item* items, int n_items, bool gl_mode, bool roh,
                         bool dump, int tile_snps, const CandList& cl, cudaStream_t st);
-// the walker over the queue of (item, 64 candidates) work units left by the bound (squeeze.cu)
-cudaError_t launch_walk_units(const WalkParams& P, const Item* items, const int2* units, const unsigned* n_units,
-                              unsigned unit_cap, int tile_snps, const CandList& cl, cudaStream_t st);
+// The uncompacted rows and the compaction plan (bound.cuh:plan_half), from which the pruned walker builds the
+// compacted slices of its candidates (bound.cuh:plan_slice)
+struct RawRows {
+    const uint64_t* rows;      // [n_ind][row_words] uncompacted
+    int64_t row_words;
+    const uint4* head;         // plan head per output half-word
+    const uint4* segs;         // [n_q][kPlanSegMax] plan segments
+    long long L;               // kept SNPs
+};
+// the walker over the queue of (item, 64 candidates) work units left by the bound (squeeze.cu); every lane reads its
+// candidate's compacted words [w0 >> 5, that + slice_words) from a slice it builds out of R first (R.rows == nullptr:
+// from the compacted rows P.geno instead)
+cudaError_t launch_walk_units(const WalkParams& P, const RawRows& R, const Item* items, const int2* units, const unsigned* n_units,
+                              unsigned unit_cap, int tile_snps, int slice_words, const CandList& cl, cudaStream_t st);
 
 // K3 + pruning bound, fused (squeeze.cu, bound.cuh)
 struct SqueezeParams {
@@ -50,8 +61,9 @@ struct SqueezeParams {
 cudaError_t launch_bound_tables(const double* lut, long long n_tab, long long n_hw, long long L, int W, uint4* hw, int* invalid, cudaStream_t st);
 cudaError_t launch_plan(const int* src, const int* n_kept, long long n_q, uint4* head, uint4* segs, uint16_t* fast,
                         int2* piece_rng, cudaStream_t st);
-// c2 > 0: with the bound for that window size class; squeeze = false: bound only, over compacted rows
-cudaError_t launch_squeeze_bound(SqueezeParams P, bool squeeze, int c2, cudaStream_t st);
+// c2 > 0: with the bound for that window size class; squeeze = false: bound only, over compacted rows;
+// squeeze and not store: bound only, over the uncompacted rows (compacted in registers, nothing written)
+cudaError_t launch_squeeze_bound(SqueezeParams P, bool squeeze, bool store, int c2, cudaStream_t st);
 cudaError_t launch_select(const Item* items, int n_items, const uint32_t* pmax, int64_t stride, int n_ind, int cut_store,
                           const int* invalid, int* cand_list, int cand_stride, unsigned* cand_cnt, int2* units, unsigned* n_units,
                           unsigned unit_cap, int lanes_per_unit, int c2, cudaStream_t st);

@@ -82,6 +82,16 @@ inline int items_tile_snps(const std::vector<Item>& items, int W)
     return m;
 }
 
+// packed words of a row the walker reads for an item (walk.cuh:walk_item): from word w0 >> 5 through the slide-in
+// stream's two-word lookahead behind its last block; the largest over the items
+inline int items_slice_words(const std::vector<Item>& items, int W)
+{
+    int m = 0;
+    for (const Item& it : items)
+        m = std::max(m, ((it.w0 + W) >> 5) + ((it.own_hi - 1 - it.w0 + 31) >> 5) + 2 - (it.w0 >> 5));
+    return m;
+}
+
 // chunk = 0: one item per segment (exact chains).  step > 0: thinning slots for window dumps.
 inline void build_items(const std::vector<int64_t>& chr_off, int W, const std::vector<Segment>& segs, int chunk,
                         int step, std::vector<Item>& items)

@@ -10,6 +10,9 @@
 // 128-byte row stores and (b), still in its register, into the bound (three POPC and a dozen integer operations).
 // SQUEEZE = false: bound only, over rows that are already compacted (another window size on the same data).
 // BOUND = false: compaction only (GL / weighted modes, window sizes outside the bound's range).
+// STORE = false (with SQUEEZE): the bound over the uncompacted rows, compacted in registers only and never written —
+// when the only consumer is the pruned walker (walk_units_kernel), which compacts its few candidates' slices itself.
+// Without the output tile a CTA needs 36 KB instead of 54 KB of shared memory: five CTAs per SM instead of four.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <algorithm>
@@ -20,7 +23,7 @@
 namespace garlic {
 
 namespace {
-constexpr int kSqWarps = 4;                               // 54 KB of shared memory per CTA: four CTAs = sixteen warps per SM
+constexpr int kSqWarps = 4;                               // 54 KB (36 KB without the output tile) of shared memory per CTA
 constexpr int kSqStages = 4;                              // ring = 4 stages of 16 input half-words (64 B) per row
 constexpr int kSqStageHw = 16, kSqStageShift = 4;
 constexpr int kSqRingHw = kSqStages * kSqStageHw;         // input half-word a of a row sits at ring position a & 63
@@ -30,6 +33,11 @@ constexpr int kSqOutRowBytes = 144;                       // output staging: 16 
 constexpr int kSqOutBytes = 32 * kSqOutRowBytes;
 constexpr int kSqStashBytes = 32 + 256 + 256;             // the current piece's plan codes, bound tables, full plan heads
 constexpr int kSqWarpBytes = kSqRingBytes + kSqOutBytes + kSqStashBytes;
+constexpr int kSqWarpBytesNoTile = kSqRingBytes + kSqStashBytes;
+// CTAs per SM: the tiled layout is held to four by shared memory (and runs at up to 128 registers); without the tile six
+// would fit, but the bound's register state (two 16-entry prefix rings, the 20-register input window, 16 half-words)
+// spills below 96 registers, which allow five
+constexpr int kSqCtasPerSm = 4, kSqCtasPerSmNoTile = 5;
 
 __device__ __forceinline__ uint32_t sq_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void cp_async8(uint32_t dst_smem, const void* src)
@@ -183,26 +191,27 @@ cudaError_t launch_plan(const int* src, const int* n_kept, long long n_q, uint4*
 // ------------------------------------------------------------------------------------------
 // the fused pass
 // ------------------------------------------------------------------------------------------
-template <bool SQUEEZE, bool BOUND, int C2, int LAG, bool PARTIAL>
-__global__ void __launch_bounds__(kSqWarps * 32)
+template <bool SQUEEZE, bool STORE, bool BOUND, int C2, int LAG, bool PARTIAL>
+__global__ void __launch_bounds__(kSqWarps * 32, SQUEEZE && STORE ? 0 : kSqCtasPerSmNoTile)
 squeeze_bound_kernel(const SqueezeParams P)
 {
+    constexpr bool TILE = SQUEEZE && STORE;               // the output staging tile exists
     extern __shared__ __align__(16) unsigned char sq_smem[];
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);   // warp-uniform for the compiler
     const int lane = threadIdx.x & 31;
-    unsigned char* ring_s = sq_smem + (size_t)warp * kSqWarpBytes;
+    unsigned char* ring_s = sq_smem + (size_t)warp * (TILE ? kSqWarpBytes : kSqWarpBytesNoTile);
     unsigned char* out_s = ring_s + kSqRingBytes;
     const uint32_t* my_ring = reinterpret_cast<const uint32_t*>(ring_s + lane * kSqRowBytes);
     const uint2* my_ring64 = reinterpret_cast<const uint2*>(ring_s + lane * kSqRowBytes);
     uint32_t* my_out = reinterpret_cast<uint32_t*>(out_s + lane * kSqOutRowBytes);   // this lane's 32 output half-words
-    uint32_t* sh_fast = reinterpret_cast<uint32_t*>(out_s + kSqOutBytes);   // the piece's 16 two-byte plan codes
+    uint32_t* sh_fast = reinterpret_cast<uint32_t*>(out_s + (TILE ? kSqOutBytes : 0));   // the piece's 16 two-byte plan codes
     uint4* sh_tab = reinterpret_cast<uint4*>(sh_fast + 8);                 // its 16 bound table entries (lanes 0..15)
     uint4* sh_head = sh_tab + 16;                                          // its 16 full plan heads (lanes 16..31): slow path
     const int c4 = lane & 7, rsel4 = lane >> 3;           // copies and flushes: a quarter-warp covers one row
     const uint32_t ring_u32 = sq_smem_u32(ring_s);
     const int n_rg = (P.n_ind + 31) >> 5;
-    const long long n_kept = SQUEEZE ? (long long)*P.n_kept : 0;
-    const long long n_out_words = SQUEEZE ? (n_kept + 31) >> 5 : 0;
+    const long long n_kept = TILE ? (long long)*P.n_kept : 0;
+    const long long n_out_words = TILE ? (n_kept + 31) >> 5 : 0;
     const long long n_tasks = (long long)n_rg * P.n_col_tasks;
     for (long long task = (long long)blockIdx.x * kSqWarps + warp; task < n_tasks; task += (long long)gridDim.x * kSqWarps) {
         const int rg = (int)(task % n_rg), ct = (int)(task / n_rg);
@@ -305,8 +314,10 @@ squeeze_bound_kernel(const SqueezeParams P)
                     const uint32_t m = __funnelshift_lc(0xffffffffu, 0u, p2);             // the fields below the dropped one
                     hreg[I] = (lo & m) | (__funnelshift_r(lo, hi, 2u) & ~m);
                 }
+                if (TILE) {
 #pragma unroll
-                for (int I = 0; I < 16; I += 4) *reinterpret_cast<uint4*>(dst + I) = make_uint4(hreg[I], hreg[I + 1], hreg[I + 2], hreg[I + 3]);
+                    for (int I = 0; I < 16; I += 4) *reinterpret_cast<uint4*>(dst + I) = make_uint4(hreg[I], hreg[I + 1], hreg[I + 2], hreg[I + 3]);
+                }
                 unsigned slow = ring_ok ? ((unsigned)rng.y & 0xffffu) : 0xffffu;
                 if (slow) {                                // several dropped SNPs, long dropped runs, the end of the data
 #pragma unroll 1
@@ -329,11 +340,18 @@ squeeze_bound_kernel(const SqueezeParams P)
                                 h |= ((x >> g.y) & g.z) << g.w;
                             }
                         }
-                        dst[I] = h;
-                    }
-                    __syncwarp();
+                        if (TILE) {
+                            dst[I] = h;
+                        } else {                           // (warp-uniform I: a select per register, no divergence)
 #pragma unroll
-                    for (int I = 0; I < 16; ++I) hreg[I] = dst[I];
+                            for (int J = 0; J < 16; ++J) hreg[J] = J == I ? h : hreg[J];
+                        }
+                    }
+                    if (TILE) {
+                        __syncwarp();
+#pragma unroll
+                        for (int I = 0; I < 16; ++I) hreg[I] = dst[I];
+                    }
                 }
             } else {
                 const uint4* hsrc = reinterpret_cast<const uint4*>(my_ring + (qb & (kSqRingHw - 1)));   // a piece = one stage
@@ -355,7 +373,7 @@ squeeze_bound_kernel(const SqueezeParams P)
                 }
             }
             // ---- two pieces = 16 output words per row: flush through shared memory, 128 B per row and quarter-warp
-            if (SQUEEZE && pi < pc_hi && ((pi & 1) || pi == pc_hi - 1)) {
+            if (TILE && pi < pc_hi && ((pi & 1) || pi == pc_hi - 1)) {
                 __syncwarp();
                 const long long wd = 16ll * (pi >> 1) + 2 * c4;
                 if (2 * c4 < ((pi & 1) ? 16 : 8) && wd < n_out_words) {
@@ -374,51 +392,51 @@ squeeze_bound_kernel(const SqueezeParams P)
     }
 }
 
-template <bool SQUEEZE, bool BOUND, int C2, int LAG, bool PARTIAL>
+template <bool SQUEEZE, bool STORE, bool BOUND, int C2, int LAG, bool PARTIAL>
 static cudaError_t launch_sq_t(const SqueezeParams& P, unsigned grid, size_t smem, cudaStream_t st)
 {
-    auto kern = squeeze_bound_kernel<SQUEEZE, BOUND, C2, LAG, PARTIAL>;
+    auto kern = squeeze_bound_kernel<SQUEEZE, STORE, BOUND, C2, LAG, PARTIAL>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kern<<<grid, kSqWarps * 32, smem, st>>>(P);
     return cudaGetLastError();
 }
 
-template <bool SQUEEZE, int LAG>
+template <bool SQUEEZE, bool STORE, int LAG>
 static cudaError_t launch_sq_c2(const SqueezeParams& P, int c2, unsigned grid, size_t smem, cudaStream_t st)
 {
     switch (c2) {
-        case 2: return launch_sq_t<SQUEEZE, true, 2, LAG, false>(P, grid, smem, st);
-        case 3: return launch_sq_t<SQUEEZE, true, 3, LAG, false>(P, grid, smem, st);
-        case 4: return launch_sq_t<SQUEEZE, true, 4, LAG, false>(P, grid, smem, st);
-        case 5: return launch_sq_t<SQUEEZE, true, 5, LAG, false>(P, grid, smem, st);
-        case 6: return launch_sq_t<SQUEEZE, true, 6, LAG, false>(P, grid, smem, st);
-        case 7: return launch_sq_t<SQUEEZE, true, 7, LAG, false>(P, grid, smem, st);
-        case 8: return launch_sq_t<SQUEEZE, true, 8, LAG, false>(P, grid, smem, st);
-        case 9: return launch_sq_t<SQUEEZE, true, 9, LAG, false>(P, grid, smem, st);
-        case 10: return launch_sq_t<SQUEEZE, true, 10, LAG, false>(P, grid, smem, st);
-        case 11: return launch_sq_t<SQUEEZE, true, 11, LAG, false>(P, grid, smem, st);
-        case 12: return launch_sq_t<SQUEEZE, true, 12, LAG, false>(P, grid, smem, st);
-        case 13: return launch_sq_t<SQUEEZE, true, 13, LAG, false>(P, grid, smem, st);
+        case 2: return launch_sq_t<SQUEEZE, STORE, true, 2, LAG, false>(P, grid, smem, st);
+        case 3: return launch_sq_t<SQUEEZE, STORE, true, 3, LAG, false>(P, grid, smem, st);
+        case 4: return launch_sq_t<SQUEEZE, STORE, true, 4, LAG, false>(P, grid, smem, st);
+        case 5: return launch_sq_t<SQUEEZE, STORE, true, 5, LAG, false>(P, grid, smem, st);
+        case 6: return launch_sq_t<SQUEEZE, STORE, true, 6, LAG, false>(P, grid, smem, st);
+        case 7: return launch_sq_t<SQUEEZE, STORE, true, 7, LAG, false>(P, grid, smem, st);
+        case 8: return launch_sq_t<SQUEEZE, STORE, true, 8, LAG, false>(P, grid, smem, st);
+        case 9: return launch_sq_t<SQUEEZE, STORE, true, 9, LAG, false>(P, grid, smem, st);
+        case 10: return launch_sq_t<SQUEEZE, STORE, true, 10, LAG, false>(P, grid, smem, st);
+        case 11: return launch_sq_t<SQUEEZE, STORE, true, 11, LAG, false>(P, grid, smem, st);
+        case 12: return launch_sq_t<SQUEEZE, STORE, true, 12, LAG, false>(P, grid, smem, st);
+        case 13: return launch_sq_t<SQUEEZE, STORE, true, 13, LAG, false>(P, grid, smem, st);
         default: return cudaErrorInvalidValue;
     }
 }
 
 // window sizes below 32: the core is a partial half-word (bound.cuh: bound_step<…, true>), C2 = LAG = 1 or 2
-template <bool SQUEEZE>
+template <bool SQUEEZE, bool STORE>
 static cudaError_t launch_sq_partial(const SqueezeParams& P, int c2, unsigned grid, size_t smem, cudaStream_t st)
 {
-    if (c2 == 1) return launch_sq_t<SQUEEZE, true, 1, 1, true>(P, grid, smem, st);
-    if (c2 == 2) return launch_sq_t<SQUEEZE, true, 2, 2, true>(P, grid, smem, st);
+    if (c2 == 1) return launch_sq_t<SQUEEZE, STORE, true, 1, 1, true>(P, grid, smem, st);
+    if (c2 == 2) return launch_sq_t<SQUEEZE, STORE, true, 2, 2, true>(P, grid, smem, st);
     return cudaErrorInvalidValue;
 }
 
-// pieces per warp task: enough tasks for a few waves of 12 warps per SM, an even number of pieces (the output
+// pieces per warp task: enough tasks for three waves of the warps an SM holds, an even number of pieces (the output
 // staging tile holds two), and long enough that the extra piece the bound drains costs a few percent
-int squeeze_pieces_per_task(int n_ind, int n_pieces)
+int squeeze_pieces_per_task(int n_ind, int n_pieces, int warps_per_sm)
 {
     const int n_rg = (n_ind + 31) / 32;
-    const int want_tasks = 148 * 16 * 3;
+    const int want_tasks = 148 * warps_per_sm * 3;
     int n_col = std::max(1, (want_tasks + n_rg - 1) / n_rg);
     int ppt = (n_pieces + n_col - 1) / n_col;
     ppt = std::max(ppt, 16);
@@ -426,24 +444,27 @@ int squeeze_pieces_per_task(int n_ind, int n_pieces)
     return ppt;
 }
 
-cudaError_t launch_squeeze_bound(SqueezeParams P, bool squeeze, int c2, cudaStream_t st)
+cudaError_t launch_squeeze_bound(SqueezeParams P, bool squeeze, bool store, int c2, cudaStream_t st)
 {
     if (!P.n_ind || !P.n_pieces) return cudaSuccess;
-    P.pieces_per_task = squeeze_pieces_per_task(P.n_ind, P.n_pieces);
+    if (!squeeze) store = false;                           // bound over compacted rows: nothing to write
+    if (c2 <= 0 && !(squeeze && store)) return cudaErrorInvalidValue;
+    if (squeeze && !store && P.partial) return cudaErrorInvalidValue;   // (window sizes below 32 walk compacted rows)
+    const int ctas_per_sm = store ? kSqCtasPerSm : kSqCtasPerSmNoTile;
+    P.pieces_per_task = squeeze_pieces_per_task(P.n_ind, P.n_pieces, ctas_per_sm * kSqWarps);
     P.n_col_tasks = (P.n_pieces + P.pieces_per_task - 1) / P.pieces_per_task;
     const int n_rg = (P.n_ind + 31) / 32;
     const long long n_tasks = (long long)n_rg * P.n_col_tasks;
     long long grid = (n_tasks + kSqWarps - 1) / kSqWarps;
-    if (grid > 148ll * 4 * 8) grid = 148ll * 4 * 8;
-    const size_t smem = (size_t)kSqWarps * kSqWarpBytes;
-    if (c2 <= 0) {
-        if (!squeeze) return cudaErrorInvalidValue;
-        return launch_sq_t<true, false, 2, 1, false>(P, (unsigned)grid, smem, st);
-    }
-    if (P.partial) return squeeze ? launch_sq_partial<true>(P, c2, (unsigned)grid, smem, st) : launch_sq_partial<false>(P, c2, (unsigned)grid, smem, st);
-    if (P.lag == 1) return squeeze ? launch_sq_c2<true, 1>(P, c2, (unsigned)grid, smem, st) : launch_sq_c2<false, 1>(P, c2, (unsigned)grid, smem, st);
-    if (P.lag == 2) return squeeze ? launch_sq_c2<true, 2>(P, c2, (unsigned)grid, smem, st) : launch_sq_c2<false, 2>(P, c2, (unsigned)grid, smem, st);
-    return cudaErrorInvalidValue;
+    if (grid > 148ll * ctas_per_sm * 8) grid = 148ll * ctas_per_sm * 8;
+    const unsigned g = (unsigned)grid;
+    const size_t smem = (size_t)kSqWarps * (store ? kSqWarpBytes : kSqWarpBytesNoTile);
+    if (c2 <= 0) return launch_sq_t<true, true, false, 2, 1, false>(P, g, smem, st);
+    if (P.partial) return squeeze ? launch_sq_partial<true, true>(P, c2, g, smem, st) : launch_sq_partial<false, false>(P, c2, g, smem, st);
+    if (P.lag != 1 && P.lag != 2) return cudaErrorInvalidValue;
+    if (!squeeze) return P.lag == 1 ? launch_sq_c2<false, false, 1>(P, c2, g, smem, st) : launch_sq_c2<false, false, 2>(P, c2, g, smem, st);
+    if (!store) return P.lag == 1 ? launch_sq_c2<true, false, 1>(P, c2, g, smem, st) : launch_sq_c2<true, false, 2>(P, c2, g, smem, st);
+    return P.lag == 1 ? launch_sq_c2<true, true, 1>(P, c2, g, smem, st) : launch_sq_c2<true, true, 2>(P, c2, g, smem, st);
 }
 
 // ------------------------------------------------------------------------------------------

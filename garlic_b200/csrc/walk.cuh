@@ -44,7 +44,8 @@ GHD double lod_eval(int g, double f, double e)
 // SRC 1: per-genotype LOD values (GL mode; lod() of each genotype's own error rate, evaluated at compaction).
 template <int SRC>
 struct LaneCtx {
-    const uint64_t* row;
+    const uint64_t* row;    // word k of the row sits at row[k - row_base]
+    int row_base;
     const char* tile;
     int tile_lo;
     const double* freq;
@@ -257,14 +258,16 @@ GHD void walk_block(const WalkParams& P, const Item& it, const LaneCtx<SRC>& C, 
 }
 
 // Walk one item for one individual.  ring: this lane's flag-history ring (NW words, stride rstride).
+// row: the words [row_base, …) of the individual's compacted row, if the caller holds them (else P.geno's row).
 template <int SRC, bool ROH, bool DUMP>
 GHD void walk_item(const WalkParams& P, const Item& it, int k_slot, bool active, uint32_t* ring, int rstride,
-                   const char* tile, int tile_lo, int ind_in = -1)
+                   const char* tile, int tile_lo, int ind_in = -1, const uint64_t* row = nullptr, int row_base = 0)
 {
     const int W = P.W;
     const int ind = ind_in >= 0 ? ind_in : (P.ind_list ? P.ind_list[k_slot] : k_slot);
     LaneCtx<SRC> C;
-    C.row = P.geno + (int64_t)ind * P.row_words;
+    C.row = row ? row : P.geno + (int64_t)ind * P.row_words;
+    C.row_base = row ? row_base : 0;
     C.tile = tile;
     C.tile_lo = tile_lo;
     C.freq = P.freq;
@@ -276,7 +279,7 @@ GHD void walk_item(const WalkParams& P, const Item& it, int k_slot, bool active,
     double win = 0.0;
     for (int i = 0; i < W; ++i) {
         const int s = it.w0 + i;
-        const int g = (int)(C.row[s >> 5] >> (2 * (s & 31))) & 3;
+        const int g = (int)(C.row[(s >> 5) - C.row_base] >> (2 * (s & 31))) & 3;
         win += C.aval(s, g);
     }
     LaneState S;
@@ -294,8 +297,8 @@ GHD void walk_item(const WalkParams& P, const Item& it, int k_slot, bool active,
 
     const int M = it.own_hi - 1 - it.w0;   // number of slide steps
     const int sa = 2 * ((it.w0 + W) & 31), sb = 2 * (it.w0 & 31);
-    const uint64_t* pa = C.row + ((it.w0 + W) >> 5);   // slide-in stream
-    const uint64_t* pb = C.row + (it.w0 >> 5);         // slide-out stream
+    const uint64_t* pa = C.row + (((it.w0 + W) >> 5) - C.row_base);   // slide-in stream
+    const uint64_t* pb = C.row + ((it.w0 >> 5) - C.row_base);         // slide-out stream
     uint64_t a_lo = pa[0], b_lo = pb[0];
     uint64_t a_hi = pa[1], b_hi = pb[1];
     pa += 2; pb += 2;

@@ -198,8 +198,8 @@ int garlic_gpu_set_prune(garlic_gpu_t *h, int on);
 /* statistics of the last call_roh, 8 doubles: [0] items, [1] individual-windows decided (N·Σ_c(L_c-W+1)),
  * [2] ambiguous (individual, segment) pairs re-evaluated exactly, [3] kernel milliseconds of pass 2 (candidate
  * selection + walker), [4] of which selection, [5] (individual, item) pairs that went to the walker (-1: no
- * pruning), [6] all (individual, item) pairs, [7] milliseconds of the last compaction (K3) launch — fused with the
- * pruning bound when the first consumer of the compacted rows was an unweighted table-mode pass */
+ * pruning), [6] all (individual, item) pairs, [7] milliseconds of the last compaction (K3) or pruning-bound launch —
+ * the bound alone, over the uncompacted rows, when the pruned pass 2 needs no compacted matrix */
 int garlic_gpu_last_stats(garlic_gpu_t *h, double *stats8);
 /* the pruning bound of pass 2 (a sufficient test that an individual has NO window >= cutoff in a 256-SNP piece,
  * evaluated from the packed genotypes alone): out [n_pieces][n_ind], per entry two int16 — low = maximum over the
