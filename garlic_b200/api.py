@@ -28,6 +28,7 @@ EXPORTS = [
     "garlic_gpu_windows_dev", "garlic_gpu_windows_gather", "garlic_gpu_comm_id", "garlic_gpu_comm_init",
     "garlic_gpu_call_roh", "garlic_gpu_last_stats", "garlic_gpu_n_kept", "garlic_gpu_get_kept_index",
     "garlic_gpu_get_genotypes", "garlic_gpu_get_piece_bounds", "garlic_gpu_set_prune", "garlic_gpu_kde", "garlic_gpu_put_tgls_text", "garlic_gpu_get_gl",
+    "garlic_gpu_put_bed", "garlic_gpu_put_bed_dev",
 ]
 
 
@@ -133,6 +134,15 @@ class GarlicGPU:
         self._ck(self.lib.garlic_gpu_put_tped_text(self.h, _p(buf), _p(off), C.c_int64(snp0), C.c_int(n),
                                                    C.c_char(missing.encode()), _p(nb)))
         return nb
+
+    def put_bed(self, rows, snp0=0):
+        """rows: uint8[n_snp, ceil(N_total/4)] SNP-major .bed rows of the whole fileset (no magic bytes); this handle keeps
+        its own individuals' columns and records the first-allele keys and counters (phase a)."""
+        r = np.ascontiguousarray(rows, np.uint8)
+        self._ck(self.lib.garlic_gpu_put_bed(self.h, _p(r), C.c_int64(r.shape[1]), C.c_int64(snp0), C.c_int(r.shape[0])))
+
+    def put_bed_dev(self, ptr, stride, n_snp, snp0=0):
+        self._ck(self.lib.garlic_gpu_put_bed_dev(self.h, C.c_void_p(ptr), C.c_int64(stride), C.c_int64(snp0), C.c_int(n_snp)))
 
     def code_alleles(self):
         self._ck(self.lib.garlic_gpu_code_alleles(self.h))

@@ -55,6 +55,11 @@ struct garlic_gpu {
     // device
     uint8_t* d_alleles = nullptr;
     unsigned long long* d_key = nullptr;
+    uint8_t* d_bed = nullptr;         // put_bed staging: [L0][bed_stride] bytes, SNP-major, this rank's byte columns
+    uint8_t* d_bed_rows = nullptr;    // put_bed: whole rows of one block as the caller passed them (handle spans every column)
+    uint32_t* d_a1 = nullptr;         // per 32-SNP word: SNPs whose "1" allele is the .bim's A1
+    int64_t bed_stride = 0;
+    bool bed_input = false;           // the genotypes came from a .bed (no allele characters, no phase)
     uint64_t *d_geno0 = nullptr, *d_geno = nullptr;
     int64_t row_words0 = 0, row_words = 0;
     int* d_counts = nullptr;
@@ -493,7 +498,8 @@ void garlic_gpu_destroy(garlic_gpu_t* h)
     cudaStreamSynchronize(h->stream);
     tl_dump(h);
     xchg_teardown(h);
-    dev_free(h->d_alleles); dev_free(h->d_key); dev_free(h->d_geno0); dev_free(h->d_geno); free_counts(h);
+    dev_free(h->d_alleles); dev_free(h->d_key); dev_free(h->d_bed); dev_free(h->d_bed_rows); dev_free(h->d_a1); dev_free(h->d_geno0); dev_free(h->d_geno);
+    free_counts(h);
     dev_free(h->d_gl0); dev_free(h->d_gl); dev_free(h->d_freq0); dev_free(h->d_freq); dev_free(h->d_lut);
     dev_free(h->d_ldplanes); dev_free(h->d_ldpairs); dev_free(h->d_text); dev_free(h->d_textoff); dev_free(h->d_nonblank);
     dev_free(h->d_gpos); dev_free(h->d_nomut); dev_free(h->d_norec); dev_free(h->d_wlut); dev_free(h->d_invld);
@@ -593,7 +599,8 @@ int garlic_gpu_set_shape(garlic_gpu_t* h, int n_ind, int ind_offset, int64_t n_l
     CK(cudaMemcpyAsync(h->d_chr_of0, chr_of.data(), n_loci * sizeof(int), cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->have_geno0 = false; h->filtered = false; h->tables = false; h->have_gl = false; h->have_ld = false;
-    dev_free(h->d_alleles); dev_free(h->d_key);
+    dev_free(h->d_alleles); dev_free(h->d_key); dev_free(h->d_bed);
+    h->bed_input = false;
     return 0;
 }
 
@@ -602,6 +609,7 @@ int garlic_gpu_put_alleles(garlic_gpu_t* h, const uint8_t* alleles, int64_t snp0
     CK(cudaSetDevice(h->device));
     if (!h->L0) FAIL("put_alleles: call set_shape first");
     if (snp0 % 32 != 0 || snp0 < 0 || snp0 + n_snp > h->L0) FAIL("put_alleles: bad SNP range (snp0 must be a multiple of 32)");
+    if (h->bed_input) FAIL("put_alleles: this handle holds .bed input");
     if (!h->d_alleles) {
         if (dev_alloc(h, &h->d_alleles, (size_t)h->L0 * h->n_ind * 2)) return 1;
         if (dev_alloc(h, &h->d_key, (size_t)h->L0)) return 1;
@@ -622,6 +630,7 @@ int garlic_gpu_put_tped_text(garlic_gpu_t* h, const char* text, const int64_t* l
     if (!h->L0) FAIL("put_tped_text: call set_shape first");
     if (snp0 % 32 != 0 || snp0 < 0 || snp0 + n_snp > h->L0) FAIL("put_tped_text: bad SNP range (snp0 must be a multiple of 32)");
     if (n_snp <= 0) return 0;
+    if (h->bed_input) FAIL("put_tped_text: this handle holds .bed input");
     if (!h->d_alleles) {
         if (dev_alloc(h, &h->d_alleles, (size_t)h->L0 * h->n_ind * 2)) return 1;
         if (dev_alloc(h, &h->d_key, (size_t)h->L0)) return 1;
@@ -648,14 +657,70 @@ int garlic_gpu_put_tped_text(garlic_gpu_t* h, const char* text, const int64_t* l
 
 void* garlic_gpu_first_allele_keys_dev(garlic_gpu_t* h) { return h ? (void*)h->d_key : nullptr; }
 
+// .bed rows of the whole file → this handle's byte columns of SNPs [snp0, snp0 + n_snp), then phase a (bed.cu)
+static int put_bed_common(garlic_gpu* h, const void* rows, int64_t stride, int64_t snp0, int n_snp, cudaMemcpyKind kind)
+{
+    CK(cudaSetDevice(h->device));
+    if (!h->L0) FAIL("put_bed: call set_shape first");
+    if (snp0 % 32 != 0 || snp0 < 0 || n_snp < 0 || snp0 + n_snp > h->L0) FAIL("put_bed: bad SNP range (snp0 must be a multiple of 32)");
+    if (h->d_alleles) FAIL("put_bed: this handle holds allele input");
+    const int64_t byte0 = h->ind_offset / 4, sh = h->ind_offset % 4;
+    const int64_t width = (sh + h->n_ind + 3) / 4;
+    if (stride < byte0 + width) FAIL("put_bed: SNP row stride smaller than the bytes of this handle's individuals");
+    if (!h->d_bed) {
+        h->bed_stride = (width + 31) / 32 * 32;               // whole 32-byte sectors per row (bed_transpose_kernel)
+        if (dev_alloc(h, &h->d_bed, (size_t)h->L0 * h->bed_stride)) return 1;
+        if (dev_alloc(h, &h->d_key, (size_t)h->L0)) return 1;
+        h->bed_input = true;
+    }
+    if (n_snp == 0) return 0;
+    uint8_t* dst = h->d_bed + (size_t)snp0 * h->bed_stride;
+    if (kind == cudaMemcpyHostToDevice && width == stride) {
+        // a pitched host-to-device copy costs about 0.13 us per row (76 ms for the 600 k rows of a 2,000-individual file
+        // on a B200 box): a handle that keeps every column takes the rows in one piece and re-pitches them on the device
+        if (dev_alloc(h, &h->d_bed_rows, (size_t)n_snp * stride)) return 1;
+        CK(cudaMemcpyAsync(h->d_bed_rows, rows, (size_t)n_snp * stride, kind, h->stream));
+        rows = h->d_bed_rows;
+        kind = cudaMemcpyDeviceToDevice;
+    }
+    CK(cudaMemcpy2DAsync(dst, (size_t)h->bed_stride, (const uint8_t*)rows + byte0, (size_t)stride, (size_t)width, (size_t)n_snp,
+                         kind, h->stream));
+    CK(cudaEventRecord(h->ev_copy, h->stream));
+    LAUNCH(launch_bed_count(dst, h->bed_stride, n_snp, (int)sh, h->n_ind, h->ind_offset, h->d_counts + snp0, h->L0,
+                            h->d_key + snp0, h->stream));
+    h->counts_reduced = false; h->counts_hi_reduced = false;
+    CK(cudaEventSynchronize(h->ev_copy));   // the copy has left the caller's buffer (it may be page-locked and reused)
+    return 0;
+}
+
+int garlic_gpu_put_bed(garlic_gpu_t* h, const uint8_t* rows, int64_t snp_stride_bytes, int64_t snp0, int n_snp)
+{
+    return put_bed_common(h, rows, snp_stride_bytes, snp0, n_snp, cudaMemcpyHostToDevice);
+}
+int garlic_gpu_put_bed_dev(garlic_gpu_t* h, const void* rows_dev, int64_t snp_stride_bytes, int64_t snp0, int n_snp)
+{
+    return put_bed_common(h, rows_dev, snp_stride_bytes, snp0, n_snp, cudaMemcpyDeviceToDevice);
+}
+
 int garlic_gpu_code_alleles(garlic_gpu_t* h)
 {
     CK(cudaSetDevice(h->device));
-    if (!h->d_alleles) FAIL("code_alleles: no alleles uploaded");
+    if (!h->d_alleles && !h->d_bed) FAIL("code_alleles: no alleles uploaded");
     const int missing = h->missing_char;
     h->counts_reduced = false; h->counts_hi_reduced = false;
     // the "1" allele is the first non-missing character over ALL individuals: MIN over the shards' keys
     if (h->comm) NCK(ncclAllReduce(h->d_key, h->d_key, (size_t)h->L0, ncclUint64, ncclMin, h->comm, h->stream));
+    if (h->d_bed) {
+        // put_bed's phase a left the counters of every SNP; nothing reads the staged rows after the transpose
+        if (dev_alloc(h, &h->d_a1, (size_t)(h->L0 + 31) / 32)) return 1;
+        LAUNCH(launch_bed_code(h->d_bed, h->bed_stride, h->L0, h->ind_offset % 4, h->n_ind, h->d_key, h->d_counts, h->d_a1,
+                               h->d_geno0, h->row_words0, h->stream));
+        h->launches++;                     // (two kernels)
+        CK(cudaStreamSynchronize(h->stream));
+        dev_free(h->d_bed); dev_free(h->d_bed_rows);
+        h->have_geno0 = true;
+        return 0;
+    }
     CK(cudaMemsetAsync(h->d_counts, 0, (size_t)4 * h->L0 * sizeof(int), h->stream));
     // chunks of SNPs so the grid stays within limits; all chunks start on a 32-SNP boundary
     const int64_t chunk = 1 << 20;
@@ -1904,6 +1969,7 @@ int garlic_gpu_ld_band(garlic_gpu_t* h, int winsize, const int32_t* ld_individua
     CK(cudaMemsetAsync(h->d_invld, 0, (size_t)(L + kPad) * inv_stride(W) * sizeof(double), h->stream));
     LdPhase ph;
     if (h->phased) {
+        if (h->bed_input) FAIL("ld_band: --phased needs phased haplotypes, and a PLINK .bed stores unphased genotypes");
         if (!h->d_alleles || !h->d_key) FAIL("ld_band: --phased needs the allele characters (put_alleles / put_tped_text), not pre-packed genotypes");
         ph.alleles = h->d_alleles; ph.key = h->d_key; ph.src = h->d_src; ph.missing = h->missing_char; ph.freq = h->d_freq;
     }

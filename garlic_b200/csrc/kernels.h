@@ -82,6 +82,12 @@ cudaError_t launch_code_alleles(const uint8_t* alleles, int n_snp, int n_ind, in
                                 int64_t row_words, int* counts, long long L0, cudaStream_t st);
 cudaError_t launch_count_packed(const uint64_t* geno, int64_t row_words, int n_ind, long long L0,
                                 int* counts, cudaStream_t st);
+// bed.cu: PLINK .bed rows staged SNP-major ([n_snp][stride] bytes, this rank's individual i at field sh + i)
+cudaError_t launch_bed_count(const uint8_t* stage, int64_t stride, int n_snp, int sh, int n_ind, int ind_offset,
+                             int* counts, long long L0, unsigned long long* key, cudaStream_t st);
+cudaError_t launch_bed_code(const uint8_t* stage, int64_t stride, long long L0, int sh, int n_ind,
+                            const unsigned long long* key, int* counts, uint32_t* a1_words, uint64_t* geno,
+                            int64_t row_words, cudaStream_t st);
 cudaError_t launch_freq_keep(const int* counts, long long L0, const int* pos, const int* chr_of,
                              const int* chr_param, int oob, double* freq, uint8_t* keep, cudaStream_t st);
 cudaError_t launch_keep_scan(const uint8_t* keep, long long L0, const int* chr_of0, int n_chr, int* block_counts,

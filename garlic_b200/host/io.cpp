@@ -182,6 +182,65 @@ bool load_tfam(const std::string& path, Tfam& f)
     return true;
 }
 
+bool load_bim(const std::string& path, Tped& t, std::vector<std::string>& a1, std::vector<std::string>& a2)
+{
+    GzLines in;
+    if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
+    std::string line, prev_chr;
+    t = Tped();
+    t.chr_off.push_back(0);
+    a1.clear();
+    a2.clear();
+    int64_t cur = 0;
+    while (in.next(line)) {
+        if (count_fields(line) != 6) {
+            LOG.error("ERROR: line " + std::to_string(t.n_loci + 1) + " of " + path + " does not have 6 columns.");
+            return false;
+        }
+        std::istringstream ss(line);
+        std::string chr, id, cm, bp, x, y;
+        ss >> chr >> id >> cm >> bp >> x >> y;
+        if (t.n_loci == 0) prev_chr = chr;
+        if (chr != prev_chr) {
+            LOG.line("Chromosome " + chr_label(prev_chr) + ": " + std::to_string(cur) + " sites.");
+            t.chr_names.push_back(prev_chr);
+            t.chr_off.push_back(t.n_loci);
+            prev_chr = chr;
+            cur = 0;
+        }
+        ++cur;
+        t.snp_id.push_back(id);
+        t.pos.push_back((int32_t)strtod(bp.c_str(), nullptr));   // as load_tped reads the 4th column
+        a1.push_back(x);
+        a2.push_back(y);
+        ++t.n_loci;
+    }
+    if (t.n_loci == 0) { LOG.error("ERROR: " + path + " is empty."); return false; }
+    LOG.line("Chromosome " + chr_label(prev_chr) + ": " + std::to_string(cur) + " sites.");
+    t.chr_names.push_back(prev_chr);
+    t.chr_off.push_back(t.n_loci);
+    return true;
+}
+
+bool open_bed(const std::string& path, int n_ind, int64_t n_loci, FILE*& f)
+{
+    f = fopen(path.c_str(), "rb");
+    if (!f) { LOG.error("ERROR: Failed to open " + path); return false; }
+    unsigned char head[3] = {0, 0, 0};
+    const size_t got = fread(head, 1, 3, f);
+    auto bad = [&](const std::string& why) { LOG.error("ERROR: " + path + ": " + why); fclose(f); f = nullptr; return false; };
+    if (got < 3 || head[0] != 0x6c || head[1] != 0x1b) return bad("not a PLINK .bed file (the first bytes are not 6c 1b).");
+    if (head[2] == 0) return bad("individual-major .bed (mode byte 00) is not supported; rewrite it SNP-major with plink --make-bed.");
+    if (head[2] != 1) return bad("unknown .bed mode byte.");
+    fseeko(f, 0, SEEK_END);
+    const int64_t size = (int64_t)ftello(f), want = 3 + n_loci * (int64_t)((n_ind + 3) / 4);
+    fseeko(f, 3, SEEK_SET);
+    if (size != want)
+        return bad("has " + std::to_string(size) + " bytes, but " + std::to_string(n_loci) + " SNPs (.bim) x " + std::to_string(n_ind) +
+                   " individuals (.fam) need " + std::to_string(want) + ".");
+    return true;
+}
+
 // loadMapScaffold (garlic-data.cpp:760-839): <chr> <id> <cM> <bp>, exactly four columns.
 bool load_map(const std::string& path, std::vector<Scaffold>& out)
 {
@@ -263,7 +322,8 @@ int TglsBlocks::next(int max_lines, std::vector<char>& text, std::vector<int64_t
 }
 TglsBlocks::~TglsBlocks() { delete static_cast<GzLines*>(impl); }
 
-bool load_freq_file(const std::string& path, const Tped& t, const std::vector<uint8_t>& one, std::vector<double>& freq)
+bool load_freq_file(const std::string& path, const Tped& t, const std::vector<std::string>& one, bool by_name,
+                    std::vector<double>& freq)
 {
     GzLines in;
     if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
@@ -280,10 +340,11 @@ bool load_freq_file(const std::string& path, const Tped& t, const std::vector<ui
         if (cols != prev_cols && prev_cols != -1) { LOG.error("ERROR: Differing number of columns across rows found in " + path); return false; }
         prev_cols = cols;
         std::istringstream ss(line);
-        std::string chr, id;
+        std::string chr, id, name;
         double pos, f;
         char allele;
-        ss >> chr >> id >> pos >> allele >> f;
+        if (by_name) ss >> chr >> id >> pos >> name >> f;
+        else ss >> chr >> id >> pos >> allele >> f;
         if (id != t.snp_id[l]) {
             LOG.error("ERROR: Loci appear mismatched in: " + path);
             LOG.error("ERROR: at line: " + std::to_string(line_no));
@@ -291,7 +352,7 @@ bool load_freq_file(const std::string& path, const Tped& t, const std::vector<ui
             LOG.error("ERROR: tped file locus name: " + t.snp_id[l]);
             return false;
         }
-        freq[l] = ((uint8_t)allele != one[l]) ? 1 - f : f;
+        freq[l] = (by_name ? name != one[l] : allele != one[l][0]) ? 1 - f : f;
     }
     if (in.next(line) && !line.empty()) { LOG.error("ERROR: " + path + " has more rows than the tped file has loci."); return false; }
     return true;
@@ -352,7 +413,7 @@ bool interpolate_map(const int32_t* pos, int64_t n, const Scaffold& s, double* g
 }
 
 // writeFreqData (garlic-data.cpp:1311-1343): all loci before filtering, 6 significant digits.
-bool write_freq_gz(const std::string& path, const Tped& t, const std::vector<uint8_t>& one, const std::vector<double>& freq)
+bool write_freq_gz(const std::string& path, const Tped& t, const std::vector<std::string>& one, const std::vector<double>& freq)
 {
     gzFile f = gzopen(path.c_str(), "wb");
     if (!f) { LOG.error("ERROR: Failed to open " + path); return false; }
@@ -361,7 +422,7 @@ bool write_freq_gz(const std::string& path, const Tped& t, const std::vector<uin
     for (size_t c = 0; c + 1 < t.chr_off.size(); ++c) {
         const std::string lab = chr_label(t.chr_names[c]);
         for (int64_t l = t.chr_off[c]; l < t.chr_off[c + 1]; ++l) {
-            row = lab + "\t" + t.snp_id[l] + "\t" + std::to_string(t.pos[l]) + "\t" + (char)one[l] + "\t" + fmt_g(freq[l]) + "\n";
+            row = lab + "\t" + t.snp_id[l] + "\t" + std::to_string(t.pos[l]) + "\t" + one[l] + "\t" + fmt_g(freq[l]) + "\n";
             gzwrite(f, row.data(), (unsigned)row.size());
         }
     }

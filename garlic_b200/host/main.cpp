@@ -292,10 +292,17 @@ int main(int argc, char** argv)
     LOG.line("Output file basename: " + o.out);
 
     // ---- validation and parameter log, in the reference's order (garlic-main.cpp:39-183) ----
-    if (o.tped == "none" || o.tfam == "none") { LOG.error("ERROR: Must provide both a tped and tfam file."); return -1; }
-    LOG.line("TPED file: " + o.tped);
-    LOG.line(std::string("TPED missing data code: ") + o.tped_missing);
-    LOG.line("TFAM file: " + o.tfam);
+    const bool bed = o.bfile != "none";
+    if (bed) {
+        if (o.tped != "none" || o.tfam != "none") { LOG.error("ERROR: Provide either --bfile or --tped and --tfam, not both."); return -1; }
+        if (o.phased) { LOG.error("ERROR: --phased cannot be used with --bfile: a PLINK .bed stores unphased genotypes."); return -1; }
+        LOG.line("PLINK binary fileset: " + o.bfile);
+    } else {
+        if (o.tped == "none" || o.tfam == "none") { LOG.error("ERROR: Must provide both a tped and tfam file."); return -1; }
+        LOG.line("TPED file: " + o.tped);
+        LOG.line(std::string("TPED missing data code: ") + o.tped_missing);
+        LOG.line("TFAM file: " + o.tfam);
+    }
     LOG.line("TGLS file: " + o.tgls);
     const bool use_gl = o.tgls != "none";
     if (use_gl && o.gl_type != "GQ" && o.gl_type != "GL" && o.gl_type != "PL") {
@@ -388,11 +395,15 @@ int main(int argc, char** argv)
 
     // ---- inputs ----
     if (!load_centromeres(o.build, o.centromere, c.cen)) return -1;
-    if (!load_tped(o.tped, o.tped_missing, c.tped, o.host_tokenize)) return 1;
+    std::vector<std::string> a1, a2;                   // .bim allele names (--bfile)
+    if (bed ? !load_bim(o.bfile + ".bim", c.tped, a1, a2) : !load_tped(o.tped, o.tped_missing, c.tped, o.host_tokenize)) return 1;
     Tped& t = c.tped;
     LOG.line("Total loci: " + std::to_string(t.n_loci));
-    if (!load_tfam(o.tfam, c.tfam)) return 1;
-    if ((int)c.tfam.ids.size() != t.n_ind) { LOG.error("ERROR: tfam and tped disagree on the number of individuals."); return 1; }
+    if (!load_tfam(bed ? o.bfile + ".fam" : o.tfam, c.tfam)) return 1;
+    if (bed) t.n_ind = (int)c.tfam.ids.size();
+    else if ((int)c.tfam.ids.size() != t.n_ind) { LOG.error("ERROR: tfam and tped disagree on the number of individuals."); return 1; }
+    FILE* bed_in = nullptr;
+    if (bed && !open_bed(o.bfile + ".bed", t.n_ind, t.n_loci, bed_in)) return 1;
     LOG.line("Population: " + c.tfam.pop);
     LOG.line("Total diploid individuals: " + std::to_string(t.n_ind));
     std::vector<double> gl;
@@ -436,7 +447,7 @@ int main(int argc, char** argv)
             if (!rank_ok(R, garlic_gpu_set_shape(R.g, n, R.lo, t.n_loci, C, t.chr_off.data(), t.pos.data()), "set_shape")) return false;
             std::vector<uint8_t> slice;
             std::vector<int32_t> nb;
-            for (int64_t s0 = 0; s0 < t.n_loci && !o.host_tokenize; s0 += blk) {
+            for (int64_t s0 = 0; s0 < t.n_loci && !bed && !o.host_tokenize; s0 += blk) {
                 // K0: the raw genotype columns go to every rank, which keeps its own individuals' characters
                 const int ns = (int)std::min(blk, t.n_loci - s0);
                 nb.resize(ns);
@@ -447,7 +458,7 @@ int main(int argc, char** argv)
                         return false;
                     }
             }
-            for (int64_t s0 = 0; s0 < t.n_loci && o.host_tokenize; s0 += blk) {
+            for (int64_t s0 = 0; s0 < t.n_loci && !bed && o.host_tokenize; s0 += blk) {
                 const int ns = (int)std::min(blk, t.n_loci - s0);
                 const uint8_t* src_ = t.alleles.data() + (size_t)s0 * t.n_ind * 2;
                 if (G > 1) {                                   // this rank's columns of the block
@@ -457,13 +468,39 @@ int main(int argc, char** argv)
                 }
                 if (!rank_ok(R, garlic_gpu_put_alleles(R.g, src_, s0, ns, o.tped_missing), "put_alleles")) return false;
             }
-            if (!rank_ok(R, garlic_gpu_code_alleles(R.g), "code_alleles")) return false;     // MIN all-reduce of the first-allele keys
+            if (!bed && !rank_ok(R, garlic_gpu_code_alleles(R.g), "code_alleles")) return false;     // MIN all-reduce of the first-allele keys
             if (use_gl && o.host_tokenize) {
                 const int type = o.gl_type == "GQ" ? GARLIC_GL_GQ : o.gl_type == "GL" ? GARLIC_GL_GL : GARLIC_GL_PL;
                 if (!rank_ok(R, garlic_gpu_put_gl(R.g, gl.data() + (size_t)R.lo * t.n_loci, type), "put_gl")) return false;
             }
             return true;
         })) return fail(1);
+    if (bed) {
+        // the .bed streams through two page-locked buffers of blk whole SNP rows: the next block is read while every rank
+        // copies its own byte columns of the current one (garlic_gpu_put_bed); the whole file is never held
+        const int64_t stride = (t.n_ind + 3) / 4;
+        uint8_t* buf[2] = {(uint8_t*)garlic_gpu_host_alloc((size_t)(blk * stride)), (uint8_t*)garlic_gpu_host_alloc((size_t)(blk * stride))};
+        auto rd = [&](int k, int64_t s0) {
+            const int64_t ns = std::min(blk, t.n_loci - s0);
+            return fread(buf[k], (size_t)stride, (size_t)ns, bed_in) == (size_t)ns;
+        };
+        bool have = buf[0] && buf[1] && rd(0, 0), put = true;
+        for (int64_t s0 = 0; have && put && s0 < t.n_loci; s0 += blk) {
+            const int k = (int)((s0 / blk) & 1), ns = (int)std::min(blk, t.n_loci - s0);
+            bool next = true;
+            std::thread reader;
+            if (s0 + blk < t.n_loci) reader = std::thread([&, k, s0] { next = rd(k ^ 1, s0 + blk); });
+            put = team.all([&](Rank& R) { return rank_ok(R, garlic_gpu_put_bed(R.g, buf[k], stride, s0, ns), "put_bed"); });
+            if (reader.joinable()) reader.join();
+            have = next;
+        }
+        fclose(bed_in);
+        garlic_gpu_host_free(buf[0]);
+        garlic_gpu_host_free(buf[1]);
+        if (!put) return fail(1);
+        if (!have) { LOG.error("ERROR: Failed to read " + o.bfile + ".bed"); team.stop(); return 1; }
+        if (!team.all([&](Rank& R) { return rank_ok(R, garlic_gpu_code_alleles(R.g), "code_alleles"); })) return fail(1);
+    }
     if (use_gl && !o.host_tokenize) {
         // K0-GL: the likelihood file goes to the GPUs as raw text, a block of lines at a time; every rank converts its
         // own individuals' columns (readTGLSData's parsing, garlic-data.cpp:1516-1554)
@@ -502,10 +539,13 @@ int main(int argc, char** argv)
     std::vector<double> freq0(t.n_loci);
     std::vector<uint8_t> one(t.n_loci);
     if (!gpu_ok(c, garlic_gpu_get_one_allele(c.g, one.data(), o.tped_missing), "get_one_allele")) return 1;
+    std::vector<std::string> one_name(t.n_loci);       // what .freq.gz prints and --freq-file is compared with
+    for (int64_t s = 0; s < t.n_loci; ++s)
+        one_name[s] = !bed ? std::string(1, (char)one[s]) : one[s] == 1 ? a1[s] : one[s] == 2 ? a2[s] : std::string("0");
     std::vector<double> panel;
     if (!auto_freq) {   // readFreqData (garlic-data.cpp:1345-1440): panel frequencies, flipped where the row names the other allele
         printf("Loading user provided allele frequencies from %s\n", o.freq_file.c_str());
-        if (!load_freq_file(o.freq_file, t, one, panel)) { team.stop(); return -1; }
+        if (!load_freq_file(o.freq_file, t, one_name, bed, panel)) { team.stop(); return -1; }
     }
     if (!team.all([&](Rank& R) {                               // SUM all-reduce of the per-SNP counters inside
             int64_t L = 0;
@@ -533,7 +573,7 @@ int main(int argc, char** argv)
                 return ok;
             })) return fail(1);
     }
-    if (auto_freq && !write_freq_gz(o.out + ".freq.gz", t, one, freq0)) { team.stop(); return 1; }
+    if (auto_freq && !write_freq_gz(o.out + ".freq.gz", t, one_name, freq0)) { team.stop(); return 1; }
     auto shutdown = [&]() { team.all([](Rank& R) { garlic_gpu_destroy(R.g); R.g = nullptr; return true; }); team.stop(); };
     if (o.freq_only) { shutdown(); return 0; }   // freqOnly (garlic-data.cpp:238-315): the .freq.gz is the output
     std::vector<int32_t> src(c.L);

@@ -81,6 +81,16 @@ void *garlic_gpu_first_allele_keys_dev(garlic_gpu_t *h);
  * nonblank (may be NULL): [n_snp] number of non-blank characters found per line, for the caller's column-count check. */
 int garlic_gpu_put_tped_text(garlic_gpu_t *h, const char *text, const int64_t *line_off, int64_t snp0, int n_snp,
                              char missing, int32_t *nonblank);
+/* PLINK 1 binary genotypes: rows = whole SNP-major .bed rows of SNPs [snp0, snp0+n_snp), snp0 % 32 == 0, of the WHOLE
+ * fileset (snp_stride_bytes = ceil(N_total/4): individual i at bits 2(i%4) of byte i/4, PLINK values 0 hom A1,
+ * 1 missing, 2 het, 3 hom A2), without the 3 magic bytes.  One cudaMemcpy2DAsync copies only the byte columns that hold
+ * this handle's individuals [ind_offset, ind_offset+n_ind); a kernel then records per SNP the first-allele key and the
+ * counters (phase a).  The calls are coded as the tped that writes hom A1 "A1 A1", het "A1 A2", hom A2 "A2 A2" and
+ * missing "0 0" would be: the "1" allele is A2 iff the first present call over all individuals is hom A2.
+ * garlic_gpu_code_alleles then runs the transpose (phase b) and frees the staging rows.  --phased is refused on such
+ * a handle (a .bed stores no phase).  _dev: rows on this GPU, complete before the call. */
+int garlic_gpu_put_bed(garlic_gpu_t *h, const uint8_t *rows, int64_t snp_stride_bytes, int64_t snp0, int n_snp);
+int garlic_gpu_put_bed_dev(garlic_gpu_t *h, const void *rows_dev, int64_t snp_stride_bytes, int64_t snp0, int n_snp);
 int garlic_gpu_code_alleles(garlic_gpu_t *h);
 
 /* ---- pre-coded input: packed 2-bit rows (codes 0/1/2, 3 = missing) -------------------------
@@ -98,7 +108,8 @@ int garlic_gpu_count_packed(garlic_gpu_t *h, const int32_t *nalleles_corr, const
  * GPUs before garlic_gpu_filter. */
 void *garlic_gpu_counts_dev(garlic_gpu_t *h);
 int garlic_gpu_get_counts(garlic_gpu_t *h, int32_t *nalleles, int32_t *total, int32_t *hom, int32_t *nonmiss);
-/* the "1" allele per SNP after code_alleles (missing char if all calls missing) */
+/* the "1" allele per SNP after code_alleles (missing char if all calls missing).  After put_bed: 1 = the .bim's A1
+ * (5th column), 2 = its A2 (6th column), missing if no call is present */
 int garlic_gpu_get_one_allele(garlic_gpu_t *h, uint8_t *allele, char missing);
 
 /* ---- optional per-genotype likelihoods (readTGLSData, src/garlic-data.cpp:1516-1586) -------
