@@ -28,7 +28,7 @@ EXPORTS = [
     "garlic_gpu_windows_dev", "garlic_gpu_windows_gather", "garlic_gpu_comm_id", "garlic_gpu_comm_init",
     "garlic_gpu_call_roh", "garlic_gpu_last_stats", "garlic_gpu_n_kept", "garlic_gpu_get_kept_index",
     "garlic_gpu_get_genotypes", "garlic_gpu_get_piece_bounds", "garlic_gpu_set_prune", "garlic_gpu_kde", "garlic_gpu_put_tgls_text", "garlic_gpu_get_gl",
-    "garlic_gpu_put_bed", "garlic_gpu_put_bed_dev",
+    "garlic_gpu_put_bed", "garlic_gpu_put_bed_dev", "garlic_gpu_put_vcf_text",
 ]
 
 
@@ -135,6 +135,17 @@ class GarlicGPU:
                                                    C.c_char(missing.encode()), _p(nb)))
         return nb
 
+    def put_vcf_text(self, text: bytes, line_off, snp0=0):
+        """VCF sample columns (the text after FORMAT's tab per record, vcf.sample_text) → allele index bytes on the device
+        (255 = missing).  Returns per record (sample columns, largest allele index or -1, first malformed column or -1)."""
+        off = np.ascontiguousarray(line_off, np.int64)
+        n = len(off) - 1
+        nc, mx, bad = np.empty(n, np.int32), np.empty(n, np.int32), np.empty(n, np.int32)
+        buf = np.frombuffer(text, np.uint8) if len(text) else np.zeros(1, np.uint8)
+        self._ck(self.lib.garlic_gpu_put_vcf_text(self.h, _p(buf), _p(off), C.c_int64(snp0), C.c_int(n), _p(nc), _p(mx),
+                                                  _p(bad)))
+        return nc, mx, bad
+
     def put_bed(self, rows, snp0=0):
         """rows: uint8[n_snp, ceil(N_total/4)] SNP-major .bed rows of the whole fileset (no magic bytes); this handle keeps
         its own individuals' columns and records the first-allele keys and counters (phase a)."""
@@ -171,8 +182,10 @@ class GarlicGPU:
         return out
 
     def get_one_allele(self, missing="0"):
+        """missing: the value for a SNP without a present allele, a one-character str or an int (255 for VCF input)."""
         a = np.empty(self.L0, np.uint8)
-        self._ck(self.lib.garlic_gpu_get_one_allele(self.h, _p(a), C.c_char(missing.encode())))
+        m = bytes([missing]) if isinstance(missing, int) else missing.encode()
+        self._ck(self.lib.garlic_gpu_get_one_allele(self.h, _p(a), C.c_char(m)))
         return a
 
     def put_gl(self, values_ind_major, gl_type):

@@ -6,8 +6,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libgarlic_b200.so")
-SOURCES = ["kernels.cu", "squeeze.cu", "wlod.cu", "kde.cu", "ingest.cu", "bed.cu", "xchg.cu", "capi.cu"]
-HEADERS = ["common.cuh", "walk.cuh", "bound.cuh", "segments.h", "kernels.h", "wlod.h", os.path.join("..", "..", "include", "garlic_b200.h")]
+SOURCES = ["kernels.cu", "squeeze.cu", "wlod.cu", "kde.cu", "ingest.cu", "bed.cu", "vcf.cu", "xchg.cu", "capi.cu"]
+HEADERS = ["common.cuh", "walk.cuh", "bound.cuh", "vcf_gt.cuh", "segments.h", "kernels.h", "wlod.h", os.path.join("..", "..", "include", "garlic_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-fmad=false",          # the reference is built without FMA; keep mul/add roundings separate
               "-Xcompiler", "-fPIC", "--shared"]

@@ -60,6 +60,7 @@ struct garlic_gpu {
     uint32_t* d_a1 = nullptr;         // per 32-SNP word: SNPs whose "1" allele is the .bim's A1
     int64_t bed_stride = 0;
     bool bed_input = false;           // the genotypes came from a .bed (no allele characters, no phase)
+    bool vcf_input = false;           // d_alleles holds VCF allele index bytes (put_vcf_text), not tped characters
     uint64_t *d_geno0 = nullptr, *d_geno = nullptr;
     int64_t row_words0 = 0, row_words = 0;
     int* d_counts = nullptr;
@@ -600,7 +601,7 @@ int garlic_gpu_set_shape(garlic_gpu_t* h, int n_ind, int ind_offset, int64_t n_l
     CK(cudaStreamSynchronize(h->stream));
     h->have_geno0 = false; h->filtered = false; h->tables = false; h->have_gl = false; h->have_ld = false;
     dev_free(h->d_alleles); dev_free(h->d_key); dev_free(h->d_bed);
-    h->bed_input = false;
+    h->bed_input = false; h->vcf_input = false;
     return 0;
 }
 
@@ -610,6 +611,7 @@ int garlic_gpu_put_alleles(garlic_gpu_t* h, const uint8_t* alleles, int64_t snp0
     if (!h->L0) FAIL("put_alleles: call set_shape first");
     if (snp0 % 32 != 0 || snp0 < 0 || snp0 + n_snp > h->L0) FAIL("put_alleles: bad SNP range (snp0 must be a multiple of 32)");
     if (h->bed_input) FAIL("put_alleles: this handle holds .bed input");
+    if (h->vcf_input) FAIL("put_alleles: this handle holds VCF input");
     if (!h->d_alleles) {
         if (dev_alloc(h, &h->d_alleles, (size_t)h->L0 * h->n_ind * 2)) return 1;
         if (dev_alloc(h, &h->d_key, (size_t)h->L0)) return 1;
@@ -631,6 +633,7 @@ int garlic_gpu_put_tped_text(garlic_gpu_t* h, const char* text, const int64_t* l
     if (snp0 % 32 != 0 || snp0 < 0 || snp0 + n_snp > h->L0) FAIL("put_tped_text: bad SNP range (snp0 must be a multiple of 32)");
     if (n_snp <= 0) return 0;
     if (h->bed_input) FAIL("put_tped_text: this handle holds .bed input");
+    if (h->vcf_input) FAIL("put_tped_text: this handle holds VCF input");
     if (!h->d_alleles) {
         if (dev_alloc(h, &h->d_alleles, (size_t)h->L0 * h->n_ind * 2)) return 1;
         if (dev_alloc(h, &h->d_key, (size_t)h->L0)) return 1;
@@ -651,6 +654,44 @@ int garlic_gpu_put_tped_text(garlic_gpu_t* h, const char* text, const int64_t* l
     LAUNCH(launch_first_allele(dst, n_snp, h->n_ind, h->ind_offset, (unsigned char)missing, h->d_key + snp0, h->stream));
     h->missing_char = (unsigned char)missing;
     if (nonblank) CK(cudaMemcpyAsync(nonblank, h->d_nonblank, (size_t)n_snp * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));   // the caller may reuse its text buffer
+    return 0;
+}
+
+int garlic_gpu_put_vcf_text(garlic_gpu_t* h, const char* text, const int64_t* line_off, int64_t snp0, int n_snp,
+                            int32_t* n_cols, int32_t* max_allele, int32_t* bad_col)
+{
+    CK(cudaSetDevice(h->device));
+    if (!h->L0) FAIL("put_vcf_text: call set_shape first");
+    if (snp0 % 32 != 0 || snp0 < 0 || snp0 + n_snp > h->L0) FAIL("put_vcf_text: bad SNP range (snp0 must be a multiple of 32)");
+    if (n_snp <= 0) return 0;
+    if (h->bed_input) FAIL("put_vcf_text: this handle holds .bed input");
+    if (h->d_alleles && !h->vcf_input) FAIL("put_vcf_text: this handle holds tped input");
+    if (!h->d_alleles) {
+        if (dev_alloc(h, &h->d_alleles, (size_t)h->L0 * h->n_ind * 2)) return 1;
+        if (dev_alloc(h, &h->d_key, (size_t)h->L0)) return 1;
+        h->vcf_input = true;
+    }
+    const int64_t bytes = line_off[n_snp] - line_off[0];
+    if (bytes < 0) FAIL("put_vcf_text: line offsets must ascend");
+    if (dev_alloc(h, &h->d_text, (size_t)bytes + 16)) return 1;
+    if (dev_alloc(h, &h->d_textoff, (size_t)n_snp + 1)) return 1;
+    if (dev_alloc(h, &h->d_nonblank, (size_t)3 * n_snp)) return 1;     // column count, largest index, first bad column
+    std::vector<long long> rel(n_snp + 1);
+    for (int i = 0; i <= n_snp; ++i) rel[i] = (long long)(line_off[i] - line_off[0]);
+    CK(cudaMemcpyAsync(h->d_text, text + line_off[0], (size_t)bytes, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->d_textoff, rel.data(), rel.size() * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+    uint8_t* dst = h->d_alleles + (size_t)snp0 * h->n_ind * 2;
+    // a short record leaves its tail untouched: pre-fill with the missing code so that nothing undefined is coded
+    CK(cudaMemsetAsync(dst, 255, (size_t)n_snp * h->n_ind * 2, h->stream));
+    int* diag = h->d_nonblank;
+    LAUNCH(launch_tokenize_vcf(h->d_text, h->d_textoff, n_snp, h->n_ind, h->ind_offset, dst, diag, diag + n_snp,
+                               diag + 2 * n_snp, h->stream));
+    LAUNCH(launch_first_allele(dst, n_snp, h->n_ind, h->ind_offset, 255, h->d_key + snp0, h->stream));
+    h->missing_char = 255;
+    int32_t* out[3] = {n_cols, max_allele, bad_col};
+    for (int k = 0; k < 3; ++k)
+        if (out[k]) CK(cudaMemcpyAsync(out[k], diag + (size_t)k * n_snp, (size_t)n_snp * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));   // the caller may reuse its text buffer
     return 0;
 }

@@ -75,6 +75,10 @@ cudaError_t launch_bucket_by_individual(RohRec* in, const unsigned* count, unsig
                                         RohRec* out, int thr, unsigned* kept, unsigned* total, cudaStream_t st);
 cudaError_t launch_tokenize_tped(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, uint8_t* alleles,
                                  int* nonblank, cudaStream_t st);
+// vcf.cu: VCF sample columns → allele index bytes (255 = missing) and per record the column count, the largest allele
+// index (-1 if none) and the first column whose GT is malformed (-1 if none)
+cudaError_t launch_tokenize_vcf(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, uint8_t* alleles,
+                                int* n_cols, int* max_allele, int* bad_col, cudaStream_t st);
 cudaError_t launch_first_allele(const uint8_t* alleles, int n_snp, int n_ind, int ind_offset, int missing,
                                 unsigned long long* key, cudaStream_t st);
 cudaError_t launch_code_alleles(const uint8_t* alleles, int n_snp, int n_ind, int missing,

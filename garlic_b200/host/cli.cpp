@@ -76,7 +76,12 @@ static const char* kHelp =
     "  --winsize --winsize-multi --auto-winsize --auto-winsize-step --overlap-frac --auto-overlap-frac --error\n"
     "  --max-gap --lod-cutoff --size-bounds --kde-subsample --ld-subsample --no-kde-thinning --nclust --M --mu\n"
     "  --build --centromere --tped-missing --threads --resample --out --raw-lod\n"
-    "Extensions: --bfile <prefix> (PLINK 1 binary fileset prefix.bed/.bim/.fam in place of --tped/--tfam; not with --phased), --gpus <n> (shard individuals over n GPUs), --exact (whole-segment chains), --device <n>, --seed <n> (subsample RNG seed), --device-lut, --kde-direct, --kde-gpu (the KDE itself on the GPU: exact Gauss transform of the thinned windows still in HBM), --host-tokenize (tped allele columns extracted on the host instead of the GPU tokeniser)\n";
+    "Extensions: --bfile <prefix> (PLINK 1 binary fileset prefix.bed/.bim/.fam in place of --tped/--tfam; not with --phased),\n"
+    "  --vcf <file> (VCF, plain, gzip or BGZF, in place of --tped; FORMAT must start with GT and every GT must be diploid, so\n"
+    "  restrict the input to the autosomes; QUAL, FILTER and INFO are ignored and no filter is applied; --tfam is optional:\n"
+    "  its IDs must equal the VCF samples in order and it names the population, which is VCF without it; not with\n"
+    "  --host-tokenize),\n"
+    "  --gpus <n> (shard individuals over n GPUs), --exact (whole-segment chains), --device <n>, --seed <n> (subsample RNG seed), --device-lut, --kde-direct, --kde-gpu (the KDE itself on the GPU: exact Gauss transform of the thinned windows still in HBM), --host-tokenize (tped allele columns extracted on the host instead of the GPU tokeniser)\n";
 
 int parse_cli(int argc, char** argv, Options& o, std::string& cmdline)
 {
@@ -93,7 +98,7 @@ int parse_cli(int argc, char** argv, Options& o, std::string& cmdline)
         {"--lod-cutoff", &o.lod_cutoff}, {"--mu", &o.mu}};
     std::map<std::string, std::string*> fs = {{"--tped", &o.tped}, {"--tfam", &o.tfam}, {"--tgls", &o.tgls},
         {"--gl-type", &o.gl_type}, {"--map", &o.map}, {"--out", &o.out}, {"--build", &o.build},
-        {"--centromere", &o.centromere}, {"--freq-file", &o.freq_file}, {"--bfile", &o.bfile}};
+        {"--centromere", &o.centromere}, {"--freq-file", &o.freq_file}, {"--bfile", &o.bfile}, {"--vcf", &o.vcf}};
     auto is_flag = [&](const std::string& s) {
         return fb.count(s) || fi.count(s) || fd.count(s) || fs.count(s) || s == "--winsize-multi" || s == "--size-bounds" ||
                s == "--tped-missing" || s == "--seed" || s == "--help";

@@ -33,6 +33,7 @@ struct Options {
     std::string tped = "none", tfam = "none", tgls = "none", gl_type = "none", map = "none", out = "outfile";
     std::string build = "none", centromere = "none", freq_file = "none";
     std::string bfile = "none";  // PLINK 1 binary fileset PREFIX.bed / .bim / .fam in place of --tped / --tfam
+    std::string vcf = "none";    // VCF in place of --tped (--tfam optional)
     bool weighted = false, cm = false, auto_winsize = false, auto_overlap = false, raw_lod = false;
     bool freq_only = false, phased = false, no_kde_thinning = false;
     int winsize = 0, auto_winsize_step = 10, max_gap = 200000, resample = 0, threads = 1, M = 7, nclust = 3;
@@ -74,6 +75,17 @@ bool load_tfam(const std::string& path, Tfam& f);
 bool load_bim(const std::string& path, Tped& t, std::vector<std::string>& a1, std::vector<std::string>& a2);
 // PLINK .bed header and size: magic 6c 1b, SNP-major mode 01, 3 + n_loci * ceil(n_ind/4) bytes; leaves f after the header
 bool open_bed(const std::string& path, int n_ind, int64_t n_loci, FILE*& f);
+// VCF (plain, gzip or BGZF — the last inflated block-parallel): the #CHROM line's samples take the place of the tfam's
+// individuals; per record CHROM / ID / POS fill the tped's columns 1 / 2 / 4 (same chromosome log lines as load_tped),
+// and the sample columns (the text after FORMAT's tab) go to Tped::text / text_off for the GPU (garlic_gpu_put_vcf_text).
+// FORMAT must be GT or start with GT:.  QUAL, FILTER and INFO are ignored.
+struct Vcf {
+    std::vector<std::string> samples;
+    std::vector<std::string> ref;                 // per record
+    std::vector<std::vector<std::string>> alts;   // per record, ALT split on ',' ('.' = none)
+    std::vector<int64_t> line;                    // per record, its line number in the file (for messages)
+};
+bool load_vcf(const std::string& path, Tped& t, Vcf& v);
 struct Scaffold { std::string chr; std::vector<int32_t> pos; std::vector<double> gen; };
 bool load_map(const std::string& path, std::vector<Scaffold>& s);
 // values individual-major [N][L0]

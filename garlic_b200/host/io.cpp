@@ -1,5 +1,5 @@
 // io.cpp — text loaders and writers of the GARLIC file formats (SURVEY.md §8b): tped / tfam / map / tgls /
-// centromere inputs (plain or gz, read through zlib), .freq.gz / .kde / .roh.bed outputs.
+// centromere inputs (plain or gz, read through zlib), VCF (plain, gz or BGZF), .freq.gz / .kde / .roh.bed outputs.
 #include <zlib.h>
 
 #include <algorithm>
@@ -7,7 +7,9 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <set>
 #include <sstream>
+#include <thread>
 
 #include "garlic_host.h"
 
@@ -62,6 +64,130 @@ struct GzLines {
     }
     ~GzLines() { if (f) gzclose(f); }
 };
+
+// BGZF, the blocked gzip of VCF files: a series of gzip members of at most 64 KiB each, whose total size is in the 'BC'
+// extra subfield (BSIZE = size - 1) and whose inflated size is in the ISIZE trailer.  So every block's input and output
+// offsets are known before any is inflated: a batch of blocks is read, inflated with raw zlib inflate on
+// min(hardware_concurrency, 16) threads, and each block's CRC32 and ISIZE are checked.  Lines are served like
+// GzLines::next_view serves them, across block and batch boundaries.
+struct BgzfLines {
+    FILE* f = nullptr;
+    std::string path, err;                     // err: why reading stopped early (truncated block, bad CRC, ...)
+    std::vector<unsigned char> in;             // the compressed blocks of the current batch
+    std::vector<char> buf;
+    size_t pos = 0, end = 0;
+    bool eof = false;
+    int threads = 1;
+    static constexpr size_t kBatch = 1024;     // blocks per batch: at most 64 MiB inflated
+
+    // true if the file starts with a BGZF block header (gzip, FEXTRA, first subfield 'BC' of length 2)
+    static bool sniff(const std::string& p)
+    {
+        FILE* g = fopen(p.c_str(), "rb");
+        if (!g) return false;
+        unsigned char h[16];
+        const bool ok = fread(h, 1, 16, g) == 16 && h[0] == 31 && h[1] == 139 && h[2] == 8 && (h[3] & 4) &&
+                        h[12] == 'B' && h[13] == 'C' && h[14] == 2 && h[15] == 0;
+        fclose(g);
+        return ok;
+    }
+    bool open(const std::string& p)
+    {
+        path = p;
+        f = fopen(p.c_str(), "rb");
+        threads = (int)std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
+        return f != nullptr;
+    }
+    bool fail(const std::string& why) { err = path + ": " + why; return false; }
+    // reads and inflates the next batch of blocks behind the unread bytes; false at the end of the file or on an error
+    bool refill()
+    {
+        struct Block { size_t in_off, in_len, out_off; uint32_t crc, isize; };
+        std::vector<Block> blocks;
+        in.clear();
+        size_t out_total = 0;
+        while (blocks.size() < kBatch) {
+            unsigned char h[12];
+            const size_t got = fread(h, 1, 12, f);
+            if (got == 0) break;
+            if (got < 12) return fail("truncated BGZF block header.");
+            if (h[0] != 31 || h[1] != 139 || h[2] != 8 || !(h[3] & 4)) return fail("not a BGZF block header.");
+            const size_t xlen = h[10] | (size_t)h[11] << 8;
+            std::vector<unsigned char> x(xlen);
+            if (fread(x.data(), 1, xlen, f) != xlen) return fail("truncated BGZF block header.");
+            long bsize = -1;
+            for (size_t q = 0; q + 4 <= xlen;) {
+                const size_t slen = x[q + 2] | (size_t)x[q + 3] << 8;
+                if (x[q] == 'B' && x[q + 1] == 'C' && slen == 2 && q + 6 <= xlen) bsize = x[q + 4] | (long)x[q + 5] << 8;
+                q += 4 + slen;
+            }
+            if (bsize < 0) return fail("a gzip member without the BGZF block size (BC subfield).");
+            const long rest = bsize + 1 - 12 - (long)xlen;
+            if (rest < 8) return fail("BGZF block size smaller than its header.");
+            const size_t base = in.size();
+            in.resize(base + rest);
+            if (fread(in.data() + base, 1, rest, f) != (size_t)rest) return fail("truncated BGZF block.");
+            const unsigned char* t = in.data() + base + rest - 8;
+            const uint32_t crc = t[0] | t[1] << 8 | t[2] << 16 | (uint32_t)t[3] << 24;
+            const uint32_t isize = t[4] | t[5] << 8 | t[6] << 16 | (uint32_t)t[7] << 24;
+            if (isize > 65536) return fail("BGZF block with ISIZE above 64 KiB.");
+            blocks.push_back({base, (size_t)rest - 8, out_total, crc, isize});
+            out_total += isize;
+        }
+        if (blocks.empty()) return false;
+        if (pos > 0) { memmove(buf.data(), buf.data() + pos, end - pos); end -= pos; pos = 0; }
+        if (buf.size() < end + out_total) buf.resize(end + out_total);
+        std::vector<char> bad(blocks.size(), 0);
+        auto work = [&](int id) {
+            for (size_t k = id; k < blocks.size(); k += threads) {
+                const Block& b = blocks[k];
+                char dummy;
+                Bytef* dst = b.isize ? (Bytef*)buf.data() + end + b.out_off : (Bytef*)&dummy;
+                z_stream zs;
+                memset(&zs, 0, sizeof(zs));
+                if (inflateInit2(&zs, -15) != Z_OK) { bad[k] = 1; continue; }
+                zs.next_in = in.data() + b.in_off;
+                zs.avail_in = (uInt)b.in_len;
+                zs.next_out = dst;
+                zs.avail_out = b.isize ? b.isize : 1;
+                const int rc = inflate(&zs, Z_FINISH);
+                if (rc != Z_STREAM_END || zs.total_out != b.isize) bad[k] = 1;
+                else if (crc32(0L, dst, b.isize) != b.crc) bad[k] = 2;
+                inflateEnd(&zs);
+            }
+        };
+        const int nt = (int)std::min<size_t>(threads, blocks.size());
+        std::vector<std::thread> pool;
+        for (int id = 1; id < nt; ++id) pool.emplace_back(work, id);
+        work(0);
+        for (auto& th : pool) th.join();
+        for (size_t k = 0; k < blocks.size(); ++k)
+            if (bad[k]) return fail(bad[k] == 2 ? "CRC32 mismatch in a BGZF block." : "corrupt BGZF block (inflate failed or ISIZE mismatch).");
+        end += out_total;
+        return true;
+    }
+    bool next_view(const char*& p, size_t& n)
+    {
+        for (;;) {
+            const char* nl = end > pos ? (const char*)memchr(buf.data() + pos, '\n', end - pos) : nullptr;
+            if (nl || (eof && end > pos)) {
+                const size_t stop = nl ? (size_t)(nl - buf.data()) : end;
+                p = buf.data() + pos;
+                n = stop - pos;
+                pos = nl ? stop + 1 : end;
+                if (n && p[n - 1] == '\r') --n;
+                return true;
+            }
+            if (eof) return false;
+            if (!refill()) eof = true;
+            if (!err.empty()) return false;
+        }
+    }
+    ~BgzfLines() { if (f) fclose(f); }
+};
+
+std::string read_error(const GzLines&) { return ""; }
+std::string read_error(const BgzfLines& b) { return b.err; }
 
 inline const char* skip_ws(const char* p) { while (*p == ' ' || *p == '\t') ++p; return p; }
 inline const char* skip_tok(const char* p) { while (*p && *p != ' ' && *p != '\t') ++p; return p; }
@@ -151,6 +277,117 @@ bool load_tped(const std::string& path, char missing, Tped& t, bool host_tokeniz
     t.chr_names.push_back(prev_chr);
     t.chr_off.push_back(t.n_loci);
     return true;
+}
+
+// VCF: '##' meta lines, the '#CHROM' header (its columns after FORMAT are the samples), then one record per line with
+// 9 tab-separated fixed columns and the sample columns.  CHROM / ID / POS take the places of the tped's columns 1 / 2 / 4;
+// the sample text is kept raw, as load_tped keeps its genotype columns, and parsed on the GPU (vcf.cu).
+template <class Lines>
+bool parse_vcf(Lines& in, const std::string& path, Tped& t, Vcf& v)
+{
+    t = Tped();
+    v = Vcf();
+    t.chr_off.push_back(0);
+    t.text_off.push_back(0);
+    const char* p;
+    size_t n;
+    int64_t line_no = 0, cur = 0;
+    std::string prev_chr;
+    bool header = false;
+    while (in.next_view(p, n)) {
+        ++line_no;
+        const char* e = p + n;
+        auto bad = [&](const std::string& where, const std::string& why) {
+            LOG.error("ERROR: " + path + " line " + std::to_string(line_no) + where + ": " + why);
+            return false;
+        };
+        if (!header) {
+            if (n >= 2 && p[0] == '#' && p[1] == '#') continue;
+            if (n < 6 || memcmp(p, "#CHROM", 6) != 0) return bad("", "no #CHROM header line before the first record.");
+            std::vector<std::string> cols;
+            for (const char* q = p;;) {
+                const char* tab = (const char*)memchr(q, '\t', e - q);
+                cols.emplace_back(q, tab ? tab : e);
+                if (!tab) break;
+                q = tab + 1;
+            }
+            if (cols.size() < 9 || cols[8] != "FORMAT") return bad("", "the #CHROM header has no FORMAT column.");
+            if (cols.size() == 9) return bad("", "the #CHROM header names no samples.");
+            std::set<std::string> seen;
+            for (size_t k = 9; k < cols.size(); ++k) {
+                if (!seen.insert(cols[k]).second) return bad("", "duplicate sample ID ( " + cols[k] + " ).");
+                v.samples.push_back(cols[k]);
+            }
+            t.n_ind = (int)v.samples.size();
+            header = true;
+            continue;
+        }
+        if (n == 0) continue;
+        const char* f[9];
+        size_t fl[9];
+        const char* q = p;
+        int k = 0;
+        while (k < 9 && q) {
+            const char* tab = (const char*)memchr(q, '\t', e - q);
+            f[k] = q;
+            fl[k] = (size_t)((tab ? tab : e) - q);
+            q = tab ? tab + 1 : nullptr;
+            ++k;
+        }
+        const std::string chr(f[0], fl[0]);
+        const std::string pos_text = k > 1 ? std::string(f[1], fl[1]) : std::string();
+        const std::string where = " (" + chr + ":" + pos_text + ")";
+        if (k < 9) return bad(where, "fewer than 9 fixed columns (CHROM POS ID REF ALT QUAL FILTER INFO FORMAT).");
+        bool num = !pos_text.empty() && pos_text.size() <= 10;
+        for (char c : pos_text) num = num && c >= '0' && c <= '9';
+        if (!num || strtoll(pos_text.c_str(), nullptr, 10) > INT32_MAX) return bad(where, "POS is not an integer.");
+        if (!(fl[8] == 2 || (fl[8] > 2 && f[8][2] == ':')) || f[8][0] != 'G' || f[8][1] != 'T')
+            return bad(where, "FORMAT does not start with GT (" + std::string(f[8], fl[8]) + ").");
+        if (t.n_loci == 0) prev_chr = chr;
+        if (chr != prev_chr) {
+            LOG.line("Chromosome " + chr_label(prev_chr) + ": " + std::to_string(cur) + " sites.");
+            t.chr_names.push_back(prev_chr);
+            t.chr_off.push_back(t.n_loci);
+            prev_chr = chr;
+            cur = 0;
+        }
+        ++cur;
+        t.snp_id.emplace_back(f[2], fl[2]);
+        t.pos.push_back((int32_t)strtod(pos_text.c_str(), nullptr));
+        v.ref.emplace_back(f[3], fl[3]);
+        v.alts.emplace_back();
+        if (!(fl[4] == 1 && f[4][0] == '.'))
+            for (const char *a = f[4], *ae = f[4] + fl[4];;) {
+                const char* c = (const char*)memchr(a, ',', ae - a);
+                v.alts.back().emplace_back(a, c ? c : ae);
+                if (!c) break;
+                a = c + 1;
+            }
+        v.line.push_back(line_no);
+        if (q) t.text.insert(t.text.end(), q, e);      // the sample columns: parsed on the GPU
+        t.text_off.push_back((int64_t)t.text.size());
+        ++t.n_loci;
+    }
+    const std::string rerr = read_error(in);
+    if (!rerr.empty()) { LOG.error("ERROR: " + rerr); return false; }
+    if (!header) { LOG.error("ERROR: " + path + " has no #CHROM header line."); return false; }
+    if (t.n_loci == 0) { LOG.error("ERROR: " + path + " has no records."); return false; }
+    LOG.line("Chromosome " + chr_label(prev_chr) + ": " + std::to_string(cur) + " sites.");
+    t.chr_names.push_back(prev_chr);
+    t.chr_off.push_back(t.n_loci);
+    return true;
+}
+
+bool load_vcf(const std::string& path, Tped& t, Vcf& v)
+{
+    if (BgzfLines::sniff(path)) {
+        BgzfLines in;
+        if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
+        return parse_vcf(in, path, t, v);
+    }
+    GzLines in;
+    if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
+    return parse_vcf(in, path, t, v);
 }
 
 // scanIndData3 / readIndData3 (garlic-data.cpp:1893-2014): single population, unique IDs.

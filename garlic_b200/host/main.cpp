@@ -292,8 +292,13 @@ int main(int argc, char** argv)
     LOG.line("Output file basename: " + o.out);
 
     // ---- validation and parameter log, in the reference's order (garlic-main.cpp:39-183) ----
-    const bool bed = o.bfile != "none";
-    if (bed) {
+    const bool bed = o.bfile != "none", vcf = o.vcf != "none";
+    if (vcf) {
+        if (o.tped != "none" || bed) { LOG.error("ERROR: Provide exactly one input: --tped/--tfam, --bfile or --vcf."); return -1; }
+        if (o.host_tokenize) { LOG.error("ERROR: --host-tokenize applies to tped input only, not to --vcf."); return -1; }
+        LOG.line("VCF file: " + o.vcf);
+        if (o.tfam != "none") LOG.line("TFAM file: " + o.tfam);
+    } else if (bed) {
         if (o.tped != "none" || o.tfam != "none") { LOG.error("ERROR: Provide either --bfile or --tped and --tfam, not both."); return -1; }
         if (o.phased) { LOG.error("ERROR: --phased cannot be used with --bfile: a PLINK .bed stores unphased genotypes."); return -1; }
         LOG.line("PLINK binary fileset: " + o.bfile);
@@ -396,10 +401,25 @@ int main(int argc, char** argv)
     // ---- inputs ----
     if (!load_centromeres(o.build, o.centromere, c.cen)) return -1;
     std::vector<std::string> a1, a2;                   // .bim allele names (--bfile)
-    if (bed ? !load_bim(o.bfile + ".bim", c.tped, a1, a2) : !load_tped(o.tped, o.tped_missing, c.tped, o.host_tokenize)) return 1;
+    Vcf vc;                                            // VCF samples and allele names (--vcf)
+    if (vcf ? !load_vcf(o.vcf, c.tped, vc)
+            : bed ? !load_bim(o.bfile + ".bim", c.tped, a1, a2) : !load_tped(o.tped, o.tped_missing, c.tped, o.host_tokenize)) return 1;
     Tped& t = c.tped;
     LOG.line("Total loci: " + std::to_string(t.n_loci));
-    if (!load_tfam(bed ? o.bfile + ".fam" : o.tfam, c.tfam)) return 1;
+    if (vcf) {
+        // the samples are the individuals; a --tfam must list the same IDs in the same order and names the population
+        if (o.tfam == "none") { c.tfam.pop = "VCF"; c.tfam.ids = vc.samples; }
+        else {
+            if (!load_tfam(o.tfam, c.tfam)) return 1;
+            for (size_t i = 0; i < std::max(c.tfam.ids.size(), vc.samples.size()); ++i)
+                if (i >= c.tfam.ids.size() || i >= vc.samples.size() || c.tfam.ids[i] != vc.samples[i]) {
+                    LOG.error("ERROR: " + o.tfam + " and " + o.vcf + " differ at individual " + std::to_string(i + 1) + ": " +
+                              (i < c.tfam.ids.size() ? c.tfam.ids[i] : std::string("(none)")) + " in the tfam, " +
+                              (i < vc.samples.size() ? vc.samples[i] : std::string("(none)")) + " in the VCF header.");
+                    return 1;
+                }
+        }
+    } else if (!load_tfam(bed ? o.bfile + ".fam" : o.tfam, c.tfam)) return 1;
     if (bed) t.n_ind = (int)c.tfam.ids.size();
     else if ((int)c.tfam.ids.size() != t.n_ind) { LOG.error("ERROR: tfam and tped disagree on the number of individuals."); return 1; }
     FILE* bed_in = nullptr;
@@ -447,7 +467,36 @@ int main(int argc, char** argv)
             if (!rank_ok(R, garlic_gpu_set_shape(R.g, n, R.lo, t.n_loci, C, t.chr_off.data(), t.pos.data()), "set_shape")) return false;
             std::vector<uint8_t> slice;
             std::vector<int32_t> nb;
-            for (int64_t s0 = 0; s0 < t.n_loci && !bed && !o.host_tokenize; s0 += blk) {
+            std::vector<int32_t> nc, mx, bc;
+            for (int64_t s0 = 0; s0 < t.n_loci && vcf; s0 += blk) {
+                // the VCF sample columns go to every rank, which keeps its own individuals' allele indices; every rank
+                // parses every column, so each finds the same malformed records
+                const int ns = (int)std::min(blk, t.n_loci - s0);
+                nc.resize(ns); mx.resize(ns); bc.resize(ns);
+                if (!rank_ok(R, garlic_gpu_put_vcf_text(R.g, t.text.data(), t.text_off.data() + s0, s0, ns, nc.data(), mx.data(), bc.data()),
+                             "put_vcf_text")) return false;
+                for (int k = 0; k < ns; ++k) {
+                    const int64_t s = s0 + k;
+                    auto rec = [&]() {                   // names the record: file line and CHROM:POS
+                        const int ch = (int)(std::upper_bound(t.chr_off.begin(), t.chr_off.end(), s) - t.chr_off.begin()) - 1;
+                        return o.vcf + " line " + std::to_string(vc.line[s]) + " (" + t.chr_names[ch] + ":" + std::to_string(t.pos[s]) + "): ";
+                    };
+                    if (nc[k] != t.n_ind) {
+                        R.err = rec() + std::to_string(nc[k]) + " sample columns, but the #CHROM header names " + std::to_string(t.n_ind) + " samples.";
+                        return false;
+                    }
+                    if (bc[k] >= 0) {
+                        R.err = rec() + "the GT of sample " + vc.samples[bc[k]] + " is not two allele indices 0..254 (or '.') separated by / or |, "
+                                "nor a lone '.'. Haploid calls (chrX in males, chrY, chrM) are not supported: restrict the input to the autosomes.";
+                        return false;
+                    }
+                    if (mx[k] > (int)vc.alts[s].size()) {
+                        R.err = rec() + "allele index " + std::to_string(mx[k]) + " but only " + std::to_string(vc.alts[s].size()) + " ALT allele(s).";
+                        return false;
+                    }
+                }
+            }
+            for (int64_t s0 = 0; s0 < t.n_loci && !bed && !vcf && !o.host_tokenize; s0 += blk) {
                 // K0: the raw genotype columns go to every rank, which keeps its own individuals' characters
                 const int ns = (int)std::min(blk, t.n_loci - s0);
                 nb.resize(ns);
@@ -538,14 +587,16 @@ int main(int argc, char** argv)
         }
     std::vector<double> freq0(t.n_loci);
     std::vector<uint8_t> one(t.n_loci);
-    if (!gpu_ok(c, garlic_gpu_get_one_allele(c.g, one.data(), o.tped_missing), "get_one_allele")) return 1;
+    const uint8_t no_one = vcf ? 255 : (uint8_t)o.tped_missing;     // get_one_allele's value for "no allele present"
+    if (!gpu_ok(c, garlic_gpu_get_one_allele(c.g, one.data(), (char)no_one), "get_one_allele")) return 1;
     std::vector<std::string> one_name(t.n_loci);       // what .freq.gz prints and --freq-file is compared with
     for (int64_t s = 0; s < t.n_loci; ++s)
-        one_name[s] = !bed ? std::string(1, (char)one[s]) : one[s] == 1 ? a1[s] : one[s] == 2 ? a2[s] : std::string("0");
+        one_name[s] = vcf ? (one[s] == 255 ? std::string("0") : one[s] == 0 ? vc.ref[s] : vc.alts[s][one[s] - 1])
+                    : !bed ? std::string(1, (char)one[s]) : one[s] == 1 ? a1[s] : one[s] == 2 ? a2[s] : std::string("0");
     std::vector<double> panel;
     if (!auto_freq) {   // readFreqData (garlic-data.cpp:1345-1440): panel frequencies, flipped where the row names the other allele
         printf("Loading user provided allele frequencies from %s\n", o.freq_file.c_str());
-        if (!load_freq_file(o.freq_file, t, one_name, bed, panel)) { team.stop(); return -1; }
+        if (!load_freq_file(o.freq_file, t, one_name, bed || vcf, panel)) { team.stop(); return -1; }
     }
     if (!team.all([&](Rank& R) {                               // SUM all-reduce of the per-SNP counters inside
             int64_t L = 0;
@@ -560,7 +611,7 @@ int main(int argc, char** argv)
         // the filter, tables and everything downstream then use the resampled frequencies
         for (int64_t s = 0; s < t.n_loci; ++s) {
             // total != 0 (garlic-data.cpp:142) <=> some non-missing allele <=> the line has a "1" allele
-            if (one[s] == (uint8_t)o.tped_missing) continue;
+            if (one[s] == no_one) continue;
             int count = 0;
             for (int i = 0; i < o.resample; ++i) count += (c.rng() / 4294967296.0) <= freq0[s];
             freq0[s] = double(count) / double(o.resample);

@@ -75,14 +75,23 @@ class HotPath:
         self.g.close()
 
     def load(self, ds, weighted=False, cm=False, error=None, max_gap=200000, packed_rows=None,
-             nalleles_corr=None, total_corr=None, mu=1e-9, M=7, bed=None):
-        """bed: uint8[L0, ceil(N/4)] SNP-major .bed rows (plink.Fileset.rows) in place of ds.alleles."""
+             nalleles_corr=None, total_corr=None, mu=1e-9, M=7, bed=None, vcf=None):
+        """bed: uint8[L0, ceil(N/4)] SNP-major .bed rows (plink.Fileset.rows) in place of ds.alleles.
+        vcf: (text, offsets) of the VCF sample columns (vcf.sample_text) in place of ds.alleles."""
         g = self.g
         N = ds.n_ind if packed_rows is None else packed_rows.shape[0]
         g.set_shape(N, len(ds.pos), ds.chr_offsets, ds.pos)
         if bed is not None:
             for s0 in range(0, len(ds.pos), 4096):
                 g.put_bed(bed[s0:s0 + 4096], s0)
+            g.code_alleles()
+        elif vcf is not None:
+            text, off = vcf
+            for s0 in range(0, len(ds.pos), 4096):
+                o = off[s0:s0 + 4097]
+                nc, mx, bad = g.put_vcf_text(text, o, s0)
+                if (nc != N).any() or (bad >= 0).any():
+                    raise ValueError("malformed VCF records in block %d" % s0)
             g.code_alleles()
         elif packed_rows is None:
             step = 1 << 16

@@ -91,6 +91,21 @@ int garlic_gpu_put_tped_text(garlic_gpu_t *h, const char *text, const int64_t *l
  * a handle (a .bed stores no phase).  _dev: rows on this GPU, complete before the call. */
 int garlic_gpu_put_bed(garlic_gpu_t *h, const uint8_t *rows, int64_t snp_stride_bytes, int64_t snp0, int n_snp);
 int garlic_gpu_put_bed_dev(garlic_gpu_t *h, const void *rows_dev, int64_t snp_stride_bytes, int64_t snp0, int n_snp);
+/* VCF genotypes: text = per record the characters after the FORMAT column's tab (the sample columns, separated by
+ * '\t'), record l of the block = text[line_off[l], line_off[l+1]), SNPs [snp0, snp0+n_snp), snp0 % 32 == 0.  Each GT
+ * (the start of a sample column, up to ':', '\t' or the end) must be two alleles separated by '/' or '|', each '.' or
+ * an allele index 0..254, or a lone '.'; this handle's individuals [ind_offset, ind_offset+n_ind) are stored as allele
+ * index bytes, 255 = missing.  A record means exactly the tped line that writes each sample's two alleles in GT order
+ * by name (REF for index 0, the k-th ALT for index k, the missing code for '.'), so the "1" allele is the first
+ * present allele in file order, half-missing calls count their present allele, and a multi-allelic record is coded
+ * "1" allele against the rest.  Phase ('|' or '/') is not checked; --phased reads the alleles in GT order.  The block
+ * is pre-filled with 255 and every call synchronises (the caller may reuse text).  Every handle parses every column,
+ * so the diagnostics are the same on all ranks; per record (each may be NULL): n_cols = sample columns,
+ * max_allele = largest allele index (-1 if none), bad_col = first column whose GT is malformed (-1 if none).  The
+ * caller checks them against the header's sample count and the record's ALT count.  Fails on a handle that holds
+ * tped or .bed input.  garlic_gpu_code_alleles then codes the block with missing = 255. */
+int garlic_gpu_put_vcf_text(garlic_gpu_t *h, const char *text, const int64_t *line_off, int64_t snp0, int n_snp,
+                            int32_t *n_cols, int32_t *max_allele, int32_t *bad_col);
 int garlic_gpu_code_alleles(garlic_gpu_t *h);
 
 /* ---- pre-coded input: packed 2-bit rows (codes 0/1/2, 3 = missing) -------------------------
@@ -109,7 +124,8 @@ int garlic_gpu_count_packed(garlic_gpu_t *h, const int32_t *nalleles_corr, const
 void *garlic_gpu_counts_dev(garlic_gpu_t *h);
 int garlic_gpu_get_counts(garlic_gpu_t *h, int32_t *nalleles, int32_t *total, int32_t *hom, int32_t *nonmiss);
 /* the "1" allele per SNP after code_alleles (missing char if all calls missing).  After put_bed: 1 = the .bim's A1
- * (5th column), 2 = its A2 (6th column), missing if no call is present */
+ * (5th column), 2 = its A2 (6th column), missing if no call is present.  After put_vcf_text: the allele index
+ * (0 = REF, k = the k-th ALT), or 255 if no allele is present (pass missing = (char)0xFF) */
 int garlic_gpu_get_one_allele(garlic_gpu_t *h, uint8_t *allele, char missing);
 
 /* ---- optional per-genotype likelihoods (readTGLSData, src/garlic-data.cpp:1516-1586) -------
