@@ -28,7 +28,7 @@ EXPORTS = [
     "garlic_gpu_windows_dev", "garlic_gpu_windows_gather", "garlic_gpu_comm_id", "garlic_gpu_comm_init",
     "garlic_gpu_call_roh", "garlic_gpu_last_stats", "garlic_gpu_n_kept", "garlic_gpu_get_kept_index",
     "garlic_gpu_get_genotypes", "garlic_gpu_get_piece_bounds", "garlic_gpu_set_prune", "garlic_gpu_kde", "garlic_gpu_put_tgls_text", "garlic_gpu_get_gl",
-    "garlic_gpu_put_bed", "garlic_gpu_put_bed_dev", "garlic_gpu_put_vcf_text",
+    "garlic_gpu_put_bed", "garlic_gpu_put_bed_dev", "garlic_gpu_put_vcf_text", "garlic_gpu_put_bcf_gt",
 ]
 
 
@@ -145,6 +145,21 @@ class GarlicGPU:
         self._ck(self.lib.garlic_gpu_put_vcf_text(self.h, _p(buf), _p(off), C.c_int64(snp0), C.c_int(n), _p(nc), _p(mx),
                                                   _p(bad)))
         return nc, mx, bad
+
+    def put_bcf_gt(self, gt, rec_off, gt_type, n_samples, snp0=0):
+        """BCF GT vectors (bcf.gt_payload: payload bytes, rec_off[n+1] at multiples of 4, the GT descriptor per record) →
+        allele index bytes on the device (255 = missing).  Returns per record (largest allele index or -1, first
+        malformed sample or -1)."""
+        off = np.ascontiguousarray(rec_off, np.int64)
+        n = len(off) - 1
+        types = np.ascontiguousarray(gt_type, np.uint8)
+        mx, bad = np.empty(n, np.int32), np.empty(n, np.int32)
+        buf = np.frombuffer(gt, np.uint8) if isinstance(gt, (bytes, bytearray)) else np.ascontiguousarray(gt, np.uint8)
+        if not buf.size:
+            buf = np.zeros(1, np.uint8)
+        self._ck(self.lib.garlic_gpu_put_bcf_gt(self.h, _p(buf), _p(off), _p(types), C.c_int(n_samples), C.c_int64(snp0),
+                                                C.c_int(n), _p(mx), _p(bad)))
+        return mx, bad
 
     def put_bed(self, rows, snp0=0):
         """rows: uint8[n_snp, ceil(N_total/4)] SNP-major .bed rows of the whole fileset (no magic bytes); this handle keeps

@@ -1,0 +1,136 @@
+// bcf.cu — BCF GT decoder (sm_100a): the GT vectors of BCF records → allele index bytes in the [n_snp][n_ind][2] block
+// that K1 (kernels.cu: first_allele_kernel, code_alleles_kernel) codes with missing = 255.
+//
+// A BCF states every field's width, so there is nothing to tokenise: record l's n_samples × count values of `width`
+// bytes start at gt + off[l] (a multiple of 4).  One CTA per record, grid-stride over records.  The common case, int8
+// with count 2, is read as 32-bit words of two samples each, four words per thread in flight, coalesced across the
+// warp; a word whose four bytes are all non-negative is a valid pair of calls and is decoded with byte-SIMD
+// ((v >> 1) - 1 per byte, which is also 255 for a missing 0 or 1).  Any other word, and the int16 / int32 / count-1
+// layouts, go through bcf_gt.cuh:decode_gt one sample per thread.  Every rank decodes every sample so that the
+// per-record diagnostics are the same on all ranks; it stores only its own individuals [ind_lo, ind_lo + n_ind).  The
+// diagnostics are reduced per warp and folded in with global atomics on arrays pre-set to -1 (atomicMax for the
+// largest allele index, an unsigned atomicMin for the first malformed sample), so a CTA never waits on a barrier.
+#include <cstdint>
+
+#include "bcf_gt.cuh"
+#include "kernels.h"
+
+namespace garlic {
+
+namespace {
+
+constexpr int kBcfThreads = 256;
+constexpr int kBcfWords = 4;      // 32-bit words per thread in flight (int8, count 2)
+
+__device__ __forceinline__ int32_t load_value(const uint8_t* p, long long k, int width)
+{
+    if (width == 1) return (int8_t)__ldg(p + k);
+    if (width == 2) return __ldg((const int16_t*)p + k);
+    return __ldg((const int32_t*)p + k);
+}
+
+__device__ __forceinline__ void store_call(uint8_t* dst, long long i, long long lo, long long hi, uint32_t ab)
+{
+    if (i >= lo && i < hi) *(uint16_t*)(dst + 2 * (i - lo)) = (uint16_t)ab;
+}
+
+__global__ void __launch_bounds__(kBcfThreads)
+decode_bcf_gt_kernel(const uint8_t* __restrict__ gt, const long long* __restrict__ off, const uint8_t* __restrict__ type,
+                     int n_snp, int n_samples, int n_ind, int ind_lo, uint8_t* __restrict__ alleles,
+                     int* __restrict__ max_allele, unsigned* __restrict__ bad_sample)
+{
+    const long long lo = ind_lo, hi = (long long)ind_lo + n_ind;
+    for (int l = blockIdx.x; l < n_snp; l += gridDim.x) {
+        const uint8_t* p = gt + off[l];
+        uint8_t* dst = alleles + (size_t)l * n_ind * 2;
+        const int count = type[l] >> 4, t = type[l] & 15, width = t == 1 ? 1 : t == 2 ? 2 : 4;
+        int my_max = -1;
+        unsigned my_bad = 0xffffffffu;
+        if (width == 1 && count == 2) {
+            const uint32_t* w = (const uint32_t*)p;
+            const int n_words = (n_samples + 1) / 2;
+            uint32_t hmax = 0;                                   // per byte: the largest (v >> 1) of a fast word
+            for (int k0 = 0; k0 < n_words; k0 += kBcfWords * kBcfThreads) {
+                uint32_t x[kBcfWords];
+#pragma unroll
+                for (int u = 0; u < kBcfWords; ++u) {
+                    const int k = k0 + u * kBcfThreads + threadIdx.x;
+                    x[u] = k < n_words ? __ldg(w + k) : 0u;
+                }
+#pragma unroll
+                for (int u = 0; u < kBcfWords; ++u) {
+                    const int k = k0 + u * kBcfThreads + threadIdx.x;
+                    if (k >= n_words) continue;
+                    const long long i = 2LL * k;                 // the word's first sample
+                    uint32_t v = x[u];
+                    if (i + 1 >= n_samples) v &= 0xffffu;         // an odd sample count: the pad is not a sample
+                    uint32_t out;
+                    if (!(v & 0x80808080u)) {                    // four non-negative values: two valid calls
+                        const uint32_t h = (v >> 1) & 0x7f7f7f7fu;
+                        hmax = __vmaxu4(hmax, h);
+                        out = __vsub4(h, 0x01010101u);
+                    } else {
+                        out = 0xffffffffu;
+#pragma unroll
+                        for (int j = 0; j < 2; ++j) {
+                            if (i + j >= n_samples) break;
+                            int a, b;
+                            if (decode_gt((int8_t)(v >> (16 * j)), (int8_t)(v >> (16 * j + 8)), 2, 1, &a, &b)) {
+                                out = (out & ~(0xffffu << (16 * j))) | (uint32_t)(a | b << 8) << (16 * j);
+                                if (a != kBcfMissing) my_max = max(my_max, a);
+                                if (b != kBcfMissing) my_max = max(my_max, b);
+                            } else if ((unsigned)(i + j) < my_bad) {
+                                my_bad = (unsigned)(i + j);
+                            }
+                        }
+                    }
+                    store_call(dst, i, lo, hi, out);
+                    store_call(dst, i + 1, lo, hi, out >> 16);
+                }
+            }
+            const uint32_t m = max(max(hmax & 0xff, (hmax >> 8) & 0xff), max((hmax >> 16) & 0xff, hmax >> 24));
+            my_max = max(my_max, (int)m - 1);
+        } else {
+            for (int i = threadIdx.x; i < n_samples; i += kBcfThreads) {
+                int a = kBcfMissing, b = kBcfMissing, ok = 0;
+                if (count >= 1 && count <= 2) {
+                    const long long k = (long long)i * count;
+                    ok = decode_gt(load_value(p, k, width), count == 2 ? load_value(p, k + 1, width) : 0, count, width, &a, &b);
+                }
+                if (ok) {
+                    if (a != kBcfMissing) my_max = max(my_max, a);
+                    if (b != kBcfMissing) my_max = max(my_max, b);
+                } else if ((unsigned)i < my_bad) {
+                    my_bad = (unsigned)i;
+                }
+                store_call(dst, i, lo, hi, ok ? (uint32_t)(a | b << 8) : 0xffffu);
+            }
+        }
+        for (int o = 16; o; o >>= 1) {
+            my_max = max(my_max, __shfl_xor_sync(0xffffffffu, my_max, o));
+            my_bad = min(my_bad, __shfl_xor_sync(0xffffffffu, my_bad, o));
+        }
+        if ((threadIdx.x & 31) == 0) {
+            if (my_max >= 0) atomicMax(max_allele + l, my_max);
+            if (my_bad != 0xffffffffu) atomicMin(bad_sample + l, my_bad);
+        }
+    }
+}
+
+}  // namespace
+
+cudaError_t launch_decode_bcf_gt(const uint8_t* gt, const long long* off, const uint8_t* type, int n_snp, int n_samples,
+                                 int n_ind, int ind_lo, uint8_t* alleles, int* max_allele, int* bad_sample,
+                                 cudaStream_t st)
+{
+    if (!n_snp) return cudaSuccess;
+    // -1 in both: "no allele" for atomicMax, and as unsigned the identity of atomicMin ("no malformed sample")
+    cudaError_t e = cudaMemsetAsync(max_allele, 0xff, (size_t)n_snp * sizeof(int), st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(bad_sample, 0xff, (size_t)n_snp * sizeof(int), st);
+    if (e != cudaSuccess) return e;
+    decode_bcf_gt_kernel<<<n_snp < 148 * 8 ? n_snp : 148 * 8, kBcfThreads, 0, st>>>(
+        gt, off, type, n_snp, n_samples, n_ind, ind_lo, alleles, max_allele, (unsigned*)bad_sample);
+    return cudaGetLastError();
+}
+
+}  // namespace garlic

@@ -71,6 +71,7 @@ struct garlic_gpu {
     char* d_text = nullptr;           // K0 staging: raw tped line tails, their offsets, non-blank counts
     long long* d_textoff = nullptr;
     int* d_nonblank = nullptr;
+    uint8_t* d_gt_type = nullptr;     // BCF: per record the GT's typed descriptor (put_bcf_gt; payloads staged in d_text)
     int2* d_hard = nullptr;           // K0-GL: tokens the device conversion leaves to strtod
     StitchScratch stitch_scratch;     // host buffers of call_roh kept between calls
     std::vector<RohRec> recs_buf, ambs_buf, merged_buf, tmp_buf;
@@ -502,7 +503,7 @@ void garlic_gpu_destroy(garlic_gpu_t* h)
     dev_free(h->d_alleles); dev_free(h->d_key); dev_free(h->d_bed); dev_free(h->d_bed_rows); dev_free(h->d_a1); dev_free(h->d_geno0); dev_free(h->d_geno);
     free_counts(h);
     dev_free(h->d_gl0); dev_free(h->d_gl); dev_free(h->d_freq0); dev_free(h->d_freq); dev_free(h->d_lut);
-    dev_free(h->d_ldplanes); dev_free(h->d_ldpairs); dev_free(h->d_text); dev_free(h->d_textoff); dev_free(h->d_nonblank);
+    dev_free(h->d_ldplanes); dev_free(h->d_ldpairs); dev_free(h->d_text); dev_free(h->d_textoff); dev_free(h->d_nonblank); dev_free(h->d_gt_type);
     dev_free(h->d_gpos); dev_free(h->d_nomut); dev_free(h->d_norec); dev_free(h->d_wlut); dev_free(h->d_invld);
     dev_free(h->d_homf); dev_free(h->d_keep); dev_free(h->d_src); dev_free(h->d_pos0); dev_free(h->d_chr_of0);
     dev_free(h->d_pos); dev_free(h->d_chr_of); dev_free(h->d_chr_start); dev_free(h->d_chr_param);
@@ -693,6 +694,55 @@ int garlic_gpu_put_vcf_text(garlic_gpu_t* h, const char* text, const int64_t* li
     for (int k = 0; k < 3; ++k)
         if (out[k]) CK(cudaMemcpyAsync(out[k], diag + (size_t)k * n_snp, (size_t)n_snp * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));   // the caller may reuse its text buffer
+    return 0;
+}
+
+int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec_off, const uint8_t* gt_type,
+                          int n_samples, int64_t snp0, int n_snp, int32_t* max_allele, int32_t* bad_sample)
+{
+    CK(cudaSetDevice(h->device));
+    if (!h->L0) FAIL("put_bcf_gt: call set_shape first");
+    if (snp0 % 32 != 0 || snp0 < 0 || snp0 + n_snp > h->L0) FAIL("put_bcf_gt: bad SNP range (snp0 must be a multiple of 32)");
+    if (n_snp <= 0) return 0;
+    if (h->bed_input) FAIL("put_bcf_gt: this handle holds .bed input");
+    if (h->d_alleles && !h->vcf_input) FAIL("put_bcf_gt: this handle holds tped input");
+    if (n_samples < h->ind_offset + h->n_ind) FAIL("put_bcf_gt: n_samples does not cover this handle's individuals");
+    for (int l = 0; l < n_snp; ++l) {
+        const int count = gt_type[l] >> 4, t = gt_type[l] & 15;
+        if (count == 0 || t < 1 || t > 3)
+            FAIL("put_bcf_gt: record " + std::to_string(l) + ": GT descriptor " + std::to_string(gt_type[l]) +
+                 " is not an int8, int16 or int32 vector with a count of 1 or more");
+        if (rec_off[l] % 4 != 0) FAIL("put_bcf_gt: record " + std::to_string(l) + ": offset is not a multiple of 4");
+        const int64_t need = (int64_t)n_samples * count * (t == 3 ? 4 : t);
+        if (rec_off[l + 1] - rec_off[l] < need)
+            FAIL("put_bcf_gt: record " + std::to_string(l) + ": payload shorter than its descriptor needs");
+    }
+    if (!h->d_alleles) {
+        if (dev_alloc(h, &h->d_alleles, (size_t)h->L0 * h->n_ind * 2)) return 1;
+        if (dev_alloc(h, &h->d_key, (size_t)h->L0)) return 1;
+        h->vcf_input = true;
+    }
+    const int64_t bytes = rec_off[n_snp] - rec_off[0];
+    if (dev_alloc(h, &h->d_text, (size_t)bytes + 16)) return 1;
+    if (dev_alloc(h, &h->d_textoff, (size_t)n_snp + 1)) return 1;
+    if (dev_alloc(h, &h->d_gt_type, (size_t)n_snp)) return 1;
+    if (dev_alloc(h, &h->d_nonblank, (size_t)2 * n_snp)) return 1;     // largest index, first bad sample
+    std::vector<long long> rel(n_snp + 1);
+    for (int i = 0; i <= n_snp; ++i) rel[i] = (long long)(rec_off[i] - rec_off[0]);
+    CK(cudaMemcpyAsync(h->d_text, gt + rec_off[0], (size_t)bytes, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->d_textoff, rel.data(), rel.size() * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->d_gt_type, gt_type, (size_t)n_snp, cudaMemcpyHostToDevice, h->stream));
+    uint8_t* dst = h->d_alleles + (size_t)snp0 * h->n_ind * 2;
+    int* diag = h->d_nonblank;
+    // every sample of this handle is stored (a malformed one as 255), so no pre-fill is needed
+    LAUNCH(launch_decode_bcf_gt((const uint8_t*)h->d_text, h->d_textoff, h->d_gt_type, n_snp, n_samples, h->n_ind,
+                                h->ind_offset, dst, diag, diag + n_snp, h->stream));
+    LAUNCH(launch_first_allele(dst, n_snp, h->n_ind, h->ind_offset, 255, h->d_key + snp0, h->stream));
+    h->missing_char = 255;
+    int32_t* out[2] = {max_allele, bad_sample};
+    for (int k = 0; k < 2; ++k)
+        if (out[k]) CK(cudaMemcpyAsync(out[k], diag + (size_t)k * n_snp, (size_t)n_snp * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));   // the caller may reuse its buffers
     return 0;
 }
 

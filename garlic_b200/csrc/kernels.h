@@ -79,6 +79,12 @@ cudaError_t launch_tokenize_tped(const char* text, const long long* off, int n_s
 // index (-1 if none) and the first column whose GT is malformed (-1 if none)
 cudaError_t launch_tokenize_vcf(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, uint8_t* alleles,
                                 int* n_cols, int* max_allele, int* bad_col, cudaStream_t st);
+// bcf.cu: BCF GT vectors (record l: n_samples x count values at gt + off[l], type[l] = the GT's typed descriptor) →
+// allele index bytes (255 = missing) and per record the largest allele index (-1 if none) and the first malformed
+// sample (-1 if none)
+cudaError_t launch_decode_bcf_gt(const uint8_t* gt, const long long* off, const uint8_t* type, int n_snp, int n_samples,
+                                 int n_ind, int ind_lo, uint8_t* alleles, int* max_allele, int* bad_sample,
+                                 cudaStream_t st);
 cudaError_t launch_first_allele(const uint8_t* alleles, int n_snp, int n_ind, int ind_offset, int missing,
                                 unsigned long long* key, cudaStream_t st);
 cudaError_t launch_code_alleles(const uint8_t* alleles, int n_snp, int n_ind, int missing,

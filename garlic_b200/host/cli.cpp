@@ -77,8 +77,9 @@ static const char* kHelp =
     "  --max-gap --lod-cutoff --size-bounds --kde-subsample --ld-subsample --no-kde-thinning --nclust --M --mu\n"
     "  --build --centromere --tped-missing --threads --resample --out --raw-lod\n"
     "Extensions: --bfile <prefix> (PLINK 1 binary fileset prefix.bed/.bim/.fam in place of --tped/--tfam; not with --phased),\n"
-    "  --vcf <file> (VCF, plain, gzip or BGZF, in place of --tped; FORMAT must start with GT and every GT must be diploid, so\n"
-    "  restrict the input to the autosomes; QUAL, FILTER and INFO are ignored and no filter is applied; --tfam is optional:\n"
+    "  --vcf <file> (VCF, plain, gzip or BGZF, or BCF 2.2, uncompressed or BGZF, in place of --tped; FORMAT must start\n"
+    "  with GT and every GT must be diploid, so restrict the input to the autosomes; QUAL, FILTER and INFO are ignored and\n"
+    "  no filter is applied; --tfam is optional:\n"
     "  its IDs must equal the VCF samples in order and it names the population, which is VCF without it; not with\n"
     "  --host-tokenize),\n"
     "  --gpus <n> (shard individuals over n GPUs), --exact (whole-segment chains), --device <n>, --seed <n> (subsample RNG seed), --device-lut, --kde-direct, --kde-gpu (the KDE itself on the GPU: exact Gauss transform of the thinned windows still in HBM), --host-tokenize (tped allele columns extracted on the host instead of the GPU tokeniser)\n";

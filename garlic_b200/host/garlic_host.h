@@ -79,11 +79,16 @@ bool open_bed(const std::string& path, int n_ind, int64_t n_loci, FILE*& f);
 // individuals; per record CHROM / ID / POS fill the tped's columns 1 / 2 / 4 (same chromosome log lines as load_tped),
 // and the sample columns (the text after FORMAT's tab) go to Tped::text / text_off for the GPU (garlic_gpu_put_vcf_text).
 // FORMAT must be GT or start with GT:.  QUAL, FILTER and INFO are ignored.
+// BCF 2.2 (uncompressed or BGZF, told from a VCF by its first inflated bytes "BCF\2\2") fills the same records, with
+// each record's GT vector in Tped::text (at a multiple of 4 bytes) and its descriptor in gt_type, for
+// garlic_gpu_put_bcf_gt.
 struct Vcf {
     std::vector<std::string> samples;
     std::vector<std::string> ref;                 // per record
     std::vector<std::vector<std::string>> alts;   // per record, ALT split on ',' ('.' = none)
-    std::vector<int64_t> line;                    // per record, its line number in the file (for messages)
+    std::vector<int64_t> line;                    // per record, its line number in the file, or its record number
+                                                  // (1-based) in a BCF (for messages)
+    std::vector<uint8_t> gt_type;                 // BCF: per record the GT's typed descriptor; empty for VCF text
 };
 bool load_vcf(const std::string& path, Tped& t, Vcf& v);
 struct Scaffold { std::string chr; std::vector<int32_t> pos; std::vector<double> gen; };

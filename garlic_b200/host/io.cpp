@@ -48,11 +48,29 @@ struct GzLines {
                 return true;
             }
             if (eof) return false;
-            if (pos > 0) { memmove(buf.data(), buf.data() + pos, end - pos); end -= pos; pos = 0; }
-            if (end == buf.size()) buf.resize(buf.size() * 2);          // a line longer than the buffer
-            const int got = gzread(f, buf.data() + end, (unsigned)std::min<size_t>(buf.size() - end, (size_t)1 << 30));
-            if (got <= 0) eof = true; else end += (size_t)got;
+            refill();
         }
+    }
+    // reads more bytes behind the unread ones, growing the buffer when it is full (a line longer than the buffer);
+    // false, and eof set, at the end of the file
+    bool refill()
+    {
+        if (pos > 0) { memmove(buf.data(), buf.data() + pos, end - pos); end -= pos; pos = 0; }
+        if (end == buf.size()) buf.resize(buf.size() * 2);
+        const int got = gzread(f, buf.data() + end, (unsigned)std::min<size_t>(buf.size() - end, (size_t)1 << 30));
+        if (got <= 0) { eof = true; return false; }
+        end += (size_t)got;
+        return true;
+    }
+    // the next n bytes as [p, p+n), valid until the following call; false if the file ends first (got = bytes left)
+    bool next_bytes(size_t n, const char*& p, size_t& got)
+    {
+        while (end - pos < n && !eof) refill();
+        got = std::min(n, end - pos);
+        if (got < n) return false;
+        p = buf.data() + pos;
+        pos += n;
+        return true;
     }
     // reads one line (without the newline) of any length; false at EOF
     bool next(std::string& line)
@@ -183,6 +201,17 @@ struct BgzfLines {
             if (!err.empty()) return false;
         }
     }
+    // as GzLines::next_bytes (records of a BCF cross block and batch boundaries); also false on a damaged block
+    bool next_bytes(size_t n, const char*& p, size_t& got)
+    {
+        while (end - pos < n && !eof && err.empty())
+            if (!refill()) eof = true;
+        got = std::min(n, end - pos);
+        if (got < n || !err.empty()) return false;
+        p = buf.data() + pos;
+        pos += n;
+        return true;
+    }
     ~BgzfLines() { if (f) fclose(f); }
 };
 
@@ -279,6 +308,54 @@ bool load_tped(const std::string& path, char missing, Tped& t, bool host_tokeniz
     return true;
 }
 
+namespace {
+
+// The '#CHROM' line of a VCF, or of a BCF's header text: its columns after FORMAT are the samples.  Returns "" and the
+// samples, or why the line is rejected.
+std::string vcf_samples(const char* p, const char* e, std::vector<std::string>& samples)
+{
+    std::vector<std::string> cols;
+    for (const char* q = p;;) {
+        const char* tab = (const char*)memchr(q, '\t', e - q);
+        cols.emplace_back(q, tab ? tab : e);
+        if (!tab) break;
+        q = tab + 1;
+    }
+    if (cols.size() < 9 || cols[8] != "FORMAT") return "the #CHROM header has no FORMAT column.";
+    if (cols.size() == 9) return "the #CHROM header names no samples.";
+    std::set<std::string> seen;
+    samples.clear();
+    for (size_t k = 9; k < cols.size(); ++k) {
+        if (!seen.insert(cols[k]).second) return "duplicate sample ID ( " + cols[k] + " ).";
+        samples.push_back(cols[k]);
+    }
+    return "";
+}
+
+// The chromosome runs of a VCF or BCF, as load_tped records them: a log line per run, names and offsets in Tped.
+struct ChrRuns {
+    std::string prev;
+    int64_t cur = 0;
+    void add(Tped& t, const std::string& chr)
+    {
+        if (t.n_loci == 0) prev = chr;
+        if (chr != prev) {
+            LOG.line("Chromosome " + chr_label(prev) + ": " + std::to_string(cur) + " sites.");
+            t.chr_names.push_back(prev);
+            t.chr_off.push_back(t.n_loci);
+            prev = chr;
+            cur = 0;
+        }
+        ++cur;
+    }
+    void finish(Tped& t)
+    {
+        LOG.line("Chromosome " + chr_label(prev) + ": " + std::to_string(cur) + " sites.");
+        t.chr_names.push_back(prev);
+        t.chr_off.push_back(t.n_loci);
+    }
+};
+
 // VCF: '##' meta lines, the '#CHROM' header (its columns after FORMAT are the samples), then one record per line with
 // 9 tab-separated fixed columns and the sample columns.  CHROM / ID / POS take the places of the tped's columns 1 / 2 / 4;
 // the sample text is kept raw, as load_tped keeps its genotype columns, and parsed on the GPU (vcf.cu).
@@ -291,8 +368,8 @@ bool parse_vcf(Lines& in, const std::string& path, Tped& t, Vcf& v)
     t.text_off.push_back(0);
     const char* p;
     size_t n;
-    int64_t line_no = 0, cur = 0;
-    std::string prev_chr;
+    int64_t line_no = 0;
+    ChrRuns runs;
     bool header = false;
     while (in.next_view(p, n)) {
         ++line_no;
@@ -304,20 +381,8 @@ bool parse_vcf(Lines& in, const std::string& path, Tped& t, Vcf& v)
         if (!header) {
             if (n >= 2 && p[0] == '#' && p[1] == '#') continue;
             if (n < 6 || memcmp(p, "#CHROM", 6) != 0) return bad("", "no #CHROM header line before the first record.");
-            std::vector<std::string> cols;
-            for (const char* q = p;;) {
-                const char* tab = (const char*)memchr(q, '\t', e - q);
-                cols.emplace_back(q, tab ? tab : e);
-                if (!tab) break;
-                q = tab + 1;
-            }
-            if (cols.size() < 9 || cols[8] != "FORMAT") return bad("", "the #CHROM header has no FORMAT column.");
-            if (cols.size() == 9) return bad("", "the #CHROM header names no samples.");
-            std::set<std::string> seen;
-            for (size_t k = 9; k < cols.size(); ++k) {
-                if (!seen.insert(cols[k]).second) return bad("", "duplicate sample ID ( " + cols[k] + " ).");
-                v.samples.push_back(cols[k]);
-            }
+            const std::string why = vcf_samples(p, e, v.samples);
+            if (!why.empty()) return bad("", why);
             t.n_ind = (int)v.samples.size();
             header = true;
             continue;
@@ -343,15 +408,7 @@ bool parse_vcf(Lines& in, const std::string& path, Tped& t, Vcf& v)
         if (!num || strtoll(pos_text.c_str(), nullptr, 10) > INT32_MAX) return bad(where, "POS is not an integer.");
         if (!(fl[8] == 2 || (fl[8] > 2 && f[8][2] == ':')) || f[8][0] != 'G' || f[8][1] != 'T')
             return bad(where, "FORMAT does not start with GT (" + std::string(f[8], fl[8]) + ").");
-        if (t.n_loci == 0) prev_chr = chr;
-        if (chr != prev_chr) {
-            LOG.line("Chromosome " + chr_label(prev_chr) + ": " + std::to_string(cur) + " sites.");
-            t.chr_names.push_back(prev_chr);
-            t.chr_off.push_back(t.n_loci);
-            prev_chr = chr;
-            cur = 0;
-        }
-        ++cur;
+        runs.add(t, chr);
         t.snp_id.emplace_back(f[2], fl[2]);
         t.pos.push_back((int32_t)strtod(pos_text.c_str(), nullptr));
         v.ref.emplace_back(f[3], fl[3]);
@@ -372,22 +429,266 @@ bool parse_vcf(Lines& in, const std::string& path, Tped& t, Vcf& v)
     if (!rerr.empty()) { LOG.error("ERROR: " + rerr); return false; }
     if (!header) { LOG.error("ERROR: " + path + " has no #CHROM header line."); return false; }
     if (t.n_loci == 0) { LOG.error("ERROR: " + path + " has no records."); return false; }
-    LOG.line("Chromosome " + chr_label(prev_chr) + ": " + std::to_string(cur) + " sites.");
-    t.chr_names.push_back(prev_chr);
-    t.chr_off.push_back(t.n_loci);
+    runs.finish(t);
     return true;
 }
 
+uint32_t le32(const char* p)
+{
+    const unsigned char* u = (const unsigned char*)p;
+    return u[0] | u[1] << 8 | u[2] << 16 | (uint32_t)u[3] << 24;
+}
+
+// A BCF header dictionary (BCF 2.2): the IDs of its header lines, indexed by their IDX= values when every line has one,
+// else in order of first appearance (an ID on several lines — INFO and FORMAT — has one index).
+struct BcfDict {
+    std::vector<std::string> ids;
+    std::map<std::string, int> seen;
+    int with_idx = 0, without_idx = 0;
+    void add(const std::string& id, long idx)
+    {
+        if (idx >= 0) {
+            ++with_idx;
+            if ((size_t)idx >= ids.size()) ids.resize(idx + 1);
+            ids[idx] = id;
+        } else {
+            ++without_idx;
+            if (seen.emplace(id, (int)ids.size()).second) ids.push_back(id);
+        }
+    }
+    // the ID of index k, or "" if k names no header line
+    std::string at(int64_t k) const { return k >= 0 && (size_t)k < ids.size() ? ids[k] : std::string(); }
+};
+
+// ID= and IDX= of a structured meta line "##KEY=<k=v,...>" (values may be quoted); idx = -1 without IDX=
+void meta_id(const char* p, const char* e, std::string& id, long& idx)
+{
+    id.clear();
+    idx = -1;
+    const char* q = (const char*)memchr(p, '<', e - p);
+    if (!q) return;
+    ++q;
+    while (q < e && *q != '>') {
+        const char* k = q;
+        while (q < e && *q != '=' && *q != ',' && *q != '>') ++q;
+        const std::string key(k, q);
+        std::string val;
+        if (q < e && *q == '=') {
+            ++q;
+            if (q < e && *q == '"') {
+                for (++q; q < e && *q != '"'; ++q) {
+                    if (*q == '\\' && q + 1 < e) ++q;
+                    val += *q;
+                }
+                if (q < e) ++q;
+            } else {
+                const char* v0 = q;
+                while (q < e && *q != ',' && *q != '>') ++q;
+                val.assign(v0, q);
+            }
+        }
+        if (key == "ID") id = val;
+        else if (key == "IDX") idx = strtol(val.c_str(), nullptr, 10);
+        if (q < e && *q == ',') ++q;
+    }
+}
+
+// Reads the typed values of a BCF record part [p, p+n) (BCF 2.2): a descriptor byte (count << 4 | type, count 15 =
+// a typed int with the count follows), then count values.
+struct Typed {
+    const unsigned char* p;
+    size_t n, i = 0;
+    static int width(int type) { return type == 1 ? 1 : type == 2 ? 2 : (type == 3 || type == 5) ? 4 : type == 7 ? 1 : 0; }
+    bool int_value(int type, int64_t& v)
+    {
+        const int w = width(type);
+        if (type < 1 || type > 3 || i + w > n) return false;
+        v = w == 1 ? (int64_t)(int8_t)p[i] : w == 2 ? (int64_t)(int16_t)(p[i] | p[i + 1] << 8) : (int64_t)(int32_t)le32((const char*)p + i);
+        i += w;
+        return true;
+    }
+    bool desc(int& type, int64_t& count)
+    {
+        if (i >= n) return false;
+        type = p[i] & 15;
+        count = p[i] >> 4;
+        ++i;
+        if (count == 15) {
+            int ct;
+            int64_t c1;
+            if (!desc(ct, c1) || c1 != 1 || !int_value(ct, count) || count < 0) return false;
+        }
+        return true;
+    }
+    bool typed_int(int64_t& v)
+    {
+        int type;
+        int64_t count;
+        return desc(type, count) && count == 1 && int_value(type, v);
+    }
+    // a typed string (type char, or any type with count 0); the value ends at its first NUL
+    bool str(std::string& s)
+    {
+        int type;
+        int64_t count;
+        if (!desc(type, count) || (count && type != 7) || (uint64_t)count > n - i) return false;
+        const char* a = (const char*)p + i;
+        s.assign(a, strnlen(a, (size_t)count));
+        i += (size_t)count;
+        return true;
+    }
+};
+
+// BCF 2.2: magic "BCF\2\2", uint32 l_text, the header text (a VCF header, NUL-terminated), then records of uint32
+// l_shared, uint32 l_indiv, the shared part (CHROM, POS, rlen, QUAL, n_allele / n_info, n_sample / n_fmt, ID, the
+// alleles, FILTER and INFO) and the indiv part (n_fmt FORMAT fields: key, descriptor, n_sample x count values).  The
+// same records as parse_vcf fills, with the record number in Vcf::line; FILTER, INFO and QUAL are skipped through
+// l_shared.  The first FORMAT field must be GT, whose values are appended to Tped::text with each record's payload at
+// a multiple of 4 bytes, and its descriptor to Vcf::gt_type: decoded on the GPU (bcf.cu).
+template <class Reader>
+bool parse_bcf(Reader& in, const std::string& path, Tped& t, Vcf& v)
+{
+    t = Tped();
+    v = Vcf();
+    t.chr_off.push_back(0);
+    t.text_off.push_back(0);
+    const char* p;
+    size_t got;
+    auto head_bad = [&](const std::string& why) {
+        const std::string rerr = read_error(in);
+        LOG.error("ERROR: " + (rerr.empty() ? path + " (BCF header): " + why : rerr));
+        return false;
+    };
+    if (!in.next_bytes(9, p, got)) return head_bad("truncated header.");
+    const uint32_t l_text = le32(p + 5);
+    if (!in.next_bytes(l_text, p, got)) return head_bad("truncated header.");
+    const char* he = p + strnlen(p, l_text);
+    BcfDict strings, contigs;
+    strings.ids.push_back("PASS");
+    strings.seen["PASS"] = 0;
+    bool header = false;
+    for (const char* q = p; q < he && !header;) {
+        const char* nl = (const char*)memchr(q, '\n', he - q);
+        const char* e = nl ? nl : he;
+        const size_t n = e - q - (e > q && e[-1] == '\r');
+        std::string id;
+        long idx;
+        auto starts = [&](const char* key) { return n >= strlen(key) && memcmp(q, key, strlen(key)) == 0; };
+        if (starts("##FILTER=<") || starts("##INFO=<") || starts("##FORMAT=<")) {
+            meta_id(q, q + n, id, idx);
+            if (!(id == "PASS" && idx < 0)) strings.add(id, idx);
+        } else if (starts("##contig=<")) {
+            meta_id(q, q + n, id, idx);
+            contigs.add(id, idx);
+        } else if (starts("#CHROM")) {
+            const std::string why = vcf_samples(q, q + n, v.samples);
+            if (!why.empty()) return head_bad(why);
+            header = true;
+        }
+        q = nl ? nl + 1 : he;
+    }
+    if (!header) return head_bad("no #CHROM header line.");
+    if (strings.with_idx && strings.without_idx) return head_bad("the FILTER / INFO / FORMAT lines mix lines with and without IDX=.");
+    if (contigs.with_idx && contigs.without_idx) return head_bad("the contig lines mix lines with and without IDX=.");
+    if (strings.ids[0].empty()) strings.ids[0] = "PASS";
+    t.n_ind = (int)v.samples.size();
+    ChrRuns runs;
+    for (int64_t rec = 1;; ++rec) {
+        std::string where;
+        auto bad = [&](const std::string& why) {
+            const std::string rerr = read_error(in);
+            LOG.error("ERROR: " + (rerr.empty() ? path + " record " + std::to_string(rec) + where + ": " + why : rerr));
+            return false;
+        };
+        if (!in.next_bytes(8, p, got)) {
+            if (got == 0 && read_error(in).empty()) break;
+            return bad("truncated record.");
+        }
+        const uint32_t l_shared = le32(p), l_indiv = le32(p + 4);
+        if (!in.next_bytes((size_t)l_shared + l_indiv, p, got))
+            return bad("truncated record: its lengths (l_shared " + std::to_string(l_shared) + ", l_indiv " +
+                       std::to_string(l_indiv) + ") run past the end of the file.");
+        const std::string chr = l_shared >= 8 ? contigs.at((int32_t)le32(p)) : std::string();
+        const int64_t pos = l_shared >= 8 ? (int64_t)(int32_t)le32(p + 4) + 1 : 0;
+        if (!chr.empty()) where = " (" + chr + ":" + std::to_string(pos) + ")";
+        if (l_shared < 24) return bad("l_shared (" + std::to_string(l_shared) + ") is too small for its fields.");
+        if (chr.empty()) return bad("CHROM index " + std::to_string((int32_t)le32(p)) + " is not in the header's contig dictionary.");
+        if (pos < 0 || pos > INT32_MAX) return bad("POS is out of range.");
+        const uint32_t n_allele = le32(p + 16) & 0xffff, n_sample = le32(p + 20) & 0xffffff, n_fmt = le32(p + 20) >> 24;
+        Typed sh{(const unsigned char*)p, l_shared, 24};
+        std::string id;
+        std::vector<std::string> alleles(n_allele);
+        bool ok = sh.str(id);
+        for (uint32_t k = 0; k < n_allele && ok; ++k) ok = sh.str(alleles[k]);
+        if (!ok) return bad("l_shared (" + std::to_string(l_shared) + ") is too small for its fields (ID and alleles).");
+        if ((int)n_sample != t.n_ind)
+            return bad(std::to_string(n_sample) + " samples, but the #CHROM header names " + std::to_string(t.n_ind) + " samples.");
+        if (n_fmt == 0) return bad("FORMAT does not start with GT (no FORMAT fields).");
+        Typed ind{(const unsigned char*)p + l_shared, l_indiv};
+        int64_t key, count;
+        int type;
+        if (!ind.typed_int(key) || !ind.desc(type, count)) return bad("l_indiv (" + std::to_string(l_indiv) + ") is too small for the GT field.");
+        const std::string fmt = strings.at(key);
+        if (fmt.empty()) return bad("FORMAT key " + std::to_string(key) + " is not in the header's dictionary of strings.");
+        if (fmt != "GT") return bad("FORMAT does not start with GT (" + fmt + ").");
+        if (type < 1 || type > 3) return bad("the GT field is of type " + std::to_string(type) + ", not int8, int16 or int32.");
+        if (count == 0) return bad("the GT field has a count of 0.");
+        const uint64_t bytes = (uint64_t)n_sample * (uint64_t)count * Typed::width(type);
+        if (bytes > ind.n - ind.i)
+            return bad("the GT vector (" + std::to_string(bytes) + " bytes) is longer than l_indiv (" + std::to_string(l_indiv) + ").");
+        runs.add(t, chr);
+        t.snp_id.push_back(id.empty() ? "." : id);
+        t.pos.push_back((int32_t)pos);
+        v.ref.push_back(n_allele ? alleles[0] : ".");
+        v.alts.emplace_back(alleles.begin() + (n_allele ? 1 : 0), alleles.end());
+        v.line.push_back(rec);
+        v.gt_type.push_back((uint8_t)(std::min<int64_t>(count, 15) << 4 | type));
+        t.text.insert(t.text.end(), p + l_shared + ind.i, p + l_shared + ind.i + bytes);   // the GT vector: decoded on the GPU
+        t.text.resize((t.text.size() + 3) & ~(size_t)3, 0);
+        t.text_off.push_back((int64_t)t.text.size());
+        ++t.n_loci;
+    }
+    if (t.n_loci == 0) { LOG.error("ERROR: " + path + " has no records."); return false; }
+    runs.finish(t);
+    return true;
+}
+
+// the first 5 inflated bytes of a file (gzip, BGZF or plain), or fewer
+std::string head_bytes(const std::string& path)
+{
+    gzFile g = gzopen(path.c_str(), "rb");
+    if (!g) return "";
+    char m[5];
+    const int n = gzread(g, m, 5);
+    gzclose(g);
+    return n > 0 ? std::string(m, n) : std::string();
+}
+
+template <class Reader>
+bool parse_vcf_or_bcf(Reader& in, const std::string& path, Tped& t, Vcf& v, bool bcf)
+{
+    return bcf ? parse_bcf(in, path, t, v) : parse_vcf(in, path, t, v);
+}
+
+}  // namespace
+
 bool load_vcf(const std::string& path, Tped& t, Vcf& v)
 {
+    const std::string magic = head_bytes(path);
+    const bool bcf = magic.size() >= 3 && magic.compare(0, 3, "BCF") == 0;
+    if (bcf && magic != std::string("BCF\2\2", 5)) {
+        const std::string ver = magic.size() == 5 ? std::to_string((unsigned char)magic[3]) + "." + std::to_string((unsigned char)magic[4]) : "?";
+        LOG.error("ERROR: " + path + " is BCF version " + ver + "; only BCF 2.2 is supported.");
+        return false;
+    }
     if (BgzfLines::sniff(path)) {
         BgzfLines in;
         if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
-        return parse_vcf(in, path, t, v);
+        return parse_vcf_or_bcf(in, path, t, v, bcf);
     }
     GzLines in;
     if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
-    return parse_vcf(in, path, t, v);
+    return parse_vcf_or_bcf(in, path, t, v, bcf);
 }
 
 // scanIndData3 / readIndData3 (garlic-data.cpp:1893-2014): single population, unique IDs.

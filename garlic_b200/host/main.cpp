@@ -18,6 +18,7 @@
 
 #include "../../include/garlic_b200.h"
 #include "garlic_host.h"
+#include "../csrc/bcf_gt.cuh"
 
 using namespace gh;
 
@@ -98,6 +99,25 @@ struct Team {
         return "unknown error";
     }
 };
+
+// BCF: the first sample of record s whose GT names an allele index above n_alt (bcf_gt.cuh:decode_gt, the rule the GPU
+// applies), -1 if none
+int bcf_sample_above(const Tped& t, const Vcf& v, int64_t s, int n_alt)
+{
+    const int count = v.gt_type[s] >> 4, type = v.gt_type[s] & 15, w = type == 3 ? 4 : type;
+    const unsigned char* p = (const unsigned char*)t.text.data() + t.text_off[s];
+    auto value = [&](int64_t k) -> int32_t {
+        const unsigned char* q = p + k * w;
+        return w == 1 ? (int8_t)q[0] : w == 2 ? (int16_t)(q[0] | q[1] << 8) : (int32_t)(q[0] | q[1] << 8 | q[2] << 16 | (uint32_t)q[3] << 24);
+    };
+    for (int i = 0; i < t.n_ind && count <= 2; ++i) {
+        int a, b;
+        if (garlic::decode_gt(value((int64_t)i * count), count == 2 ? value((int64_t)i * count + 1) : 0, count, w, &a, &b) &&
+            ((a != garlic::kBcfMissing && a > n_alt) || (b != garlic::kBcfMissing && b > n_alt)))
+            return i;
+    }
+    return -1;
+}
 
 bool rank_ok(Rank& r, int rc, const char* what)
 {
@@ -460,6 +480,27 @@ int main(int argc, char** argv)
     for (int r = 0; r < G; ++r) { team.ranks[r].rank = r; team.ranks[r].lo = std::min(t.n_ind, r * per); team.ranks[r].hi = std::min(t.n_ind, (r + 1) * per); }
     auto fail = [&](int code) { LOG.error("ERROR: " + team.first_error()); team.stop(); return code; };
     const int64_t blk = 1 << 12;                       // tped lines per upload (multiple of 32)
+    const bool bcf = !vc.gt_type.empty();
+    auto vcf_record = [&](int64_t s) {                 // names a VCF / BCF record: file, line or record, CHROM:POS
+        const int ch = (int)(std::upper_bound(t.chr_off.begin(), t.chr_off.end(), s) - t.chr_off.begin()) - 1;
+        return o.vcf + (bcf ? " record " : " line ") + std::to_string(vc.line[s]) + " (" + t.chr_names[ch] + ":" + std::to_string(t.pos[s]) + "): ";
+    };
+    // the checks of a record's GT diagnostics (first malformed sample, largest allele index) against its ALT count
+    auto vcf_record_error = [&](int64_t s, int bad, int max_allele) -> std::string {
+        if (bad >= 0)
+            return vcf_record(s) + "the GT of sample " + vc.samples[bad] +
+                   (bcf ? " is not two allele indices 0..254 (or missing), nor a lone missing value."
+                        : " is not two allele indices 0..254 (or '.') separated by / or |, nor a lone '.'.") +
+                   " Haploid calls (chrX in males, chrY, chrM) are not supported: restrict the input to the autosomes.";
+        const int n_alt = (int)vc.alts[s].size();
+        if (max_allele > n_alt) {
+            std::string e = vcf_record(s) + "allele index " + std::to_string(max_allele) + " but only " + std::to_string(n_alt) + " ALT allele(s).";
+            const int i = bcf ? bcf_sample_above(t, vc, s, n_alt) : -1;
+            if (i >= 0) e += " First in sample " + vc.samples[i] + ".";
+            return e;
+        }
+        return "";
+    };
     if (!team.all([&](Rank& R) {
             if (garlic_gpu_create(o.device + R.rank, &R.g)) { R.err = "no usable CUDA device " + std::to_string(o.device + R.rank) + "; garlic_b200 has no CPU path"; return false; }
             if (G > 1 && !rank_ok(R, garlic_gpu_comm_init(R.g, comm_id, R.rank, G), "comm_init")) return false;
@@ -469,31 +510,21 @@ int main(int argc, char** argv)
             std::vector<int32_t> nb;
             std::vector<int32_t> nc, mx, bc;
             for (int64_t s0 = 0; s0 < t.n_loci && vcf; s0 += blk) {
-                // the VCF sample columns go to every rank, which keeps its own individuals' allele indices; every rank
-                // parses every column, so each finds the same malformed records
+                // the VCF sample columns (or the BCF GT vectors) go to every rank, which keeps its own individuals'
+                // allele indices; every rank parses every sample, so each finds the same malformed records
                 const int ns = (int)std::min(blk, t.n_loci - s0);
                 nc.resize(ns); mx.resize(ns); bc.resize(ns);
-                if (!rank_ok(R, garlic_gpu_put_vcf_text(R.g, t.text.data(), t.text_off.data() + s0, s0, ns, nc.data(), mx.data(), bc.data()),
-                             "put_vcf_text")) return false;
+                if (bcf ? !rank_ok(R, garlic_gpu_put_bcf_gt(R.g, (const uint8_t*)t.text.data(), t.text_off.data() + s0, vc.gt_type.data() + s0,
+                                                            t.n_ind, s0, ns, mx.data(), bc.data()), "put_bcf_gt")
+                        : !rank_ok(R, garlic_gpu_put_vcf_text(R.g, t.text.data(), t.text_off.data() + s0, s0, ns, nc.data(), mx.data(), bc.data()),
+                                   "put_vcf_text")) return false;
                 for (int k = 0; k < ns; ++k) {
-                    const int64_t s = s0 + k;
-                    auto rec = [&]() {                   // names the record: file line and CHROM:POS
-                        const int ch = (int)(std::upper_bound(t.chr_off.begin(), t.chr_off.end(), s) - t.chr_off.begin()) - 1;
-                        return o.vcf + " line " + std::to_string(vc.line[s]) + " (" + t.chr_names[ch] + ":" + std::to_string(t.pos[s]) + "): ";
-                    };
-                    if (nc[k] != t.n_ind) {
-                        R.err = rec() + std::to_string(nc[k]) + " sample columns, but the #CHROM header names " + std::to_string(t.n_ind) + " samples.";
+                    if (!bcf && nc[k] != t.n_ind) {
+                        R.err = vcf_record(s0 + k) + std::to_string(nc[k]) + " sample columns, but the #CHROM header names " + std::to_string(t.n_ind) + " samples.";
                         return false;
                     }
-                    if (bc[k] >= 0) {
-                        R.err = rec() + "the GT of sample " + vc.samples[bc[k]] + " is not two allele indices 0..254 (or '.') separated by / or |, "
-                                "nor a lone '.'. Haploid calls (chrX in males, chrY, chrM) are not supported: restrict the input to the autosomes.";
-                        return false;
-                    }
-                    if (mx[k] > (int)vc.alts[s].size()) {
-                        R.err = rec() + "allele index " + std::to_string(mx[k]) + " but only " + std::to_string(vc.alts[s].size()) + " ALT allele(s).";
-                        return false;
-                    }
+                    R.err = vcf_record_error(s0 + k, bc[k], mx[k]);
+                    if (!R.err.empty()) return false;
                 }
             }
             for (int64_t s0 = 0; s0 < t.n_loci && !bed && !vcf && !o.host_tokenize; s0 += blk) {

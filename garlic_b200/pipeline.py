@@ -75,9 +75,10 @@ class HotPath:
         self.g.close()
 
     def load(self, ds, weighted=False, cm=False, error=None, max_gap=200000, packed_rows=None,
-             nalleles_corr=None, total_corr=None, mu=1e-9, M=7, bed=None, vcf=None):
+             nalleles_corr=None, total_corr=None, mu=1e-9, M=7, bed=None, vcf=None, bcf=None):
         """bed: uint8[L0, ceil(N/4)] SNP-major .bed rows (plink.Fileset.rows) in place of ds.alleles.
-        vcf: (text, offsets) of the VCF sample columns (vcf.sample_text) in place of ds.alleles."""
+        vcf: (text, offsets) of the VCF sample columns (vcf.sample_text) in place of ds.alleles.
+        bcf: (payload, offsets, descriptors) of the BCF GT vectors (bcf.gt_payload) in place of ds.alleles."""
         g = self.g
         N = ds.n_ind if packed_rows is None else packed_rows.shape[0]
         g.set_shape(N, len(ds.pos), ds.chr_offsets, ds.pos)
@@ -92,6 +93,13 @@ class HotPath:
                 nc, mx, bad = g.put_vcf_text(text, o, s0)
                 if (nc != N).any() or (bad >= 0).any():
                     raise ValueError("malformed VCF records in block %d" % s0)
+            g.code_alleles()
+        elif bcf is not None:
+            gt, off, types = bcf
+            for s0 in range(0, len(ds.pos), 4096):
+                _, bad = g.put_bcf_gt(gt, off[s0:s0 + 4097], types[s0:s0 + 4096], N, s0)
+                if (bad >= 0).any():
+                    raise ValueError("malformed BCF records in block %d" % s0)
             g.code_alleles()
         elif packed_rows is None:
             step = 1 << 16

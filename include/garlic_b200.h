@@ -106,6 +106,22 @@ int garlic_gpu_put_bed_dev(garlic_gpu_t *h, const void *rows_dev, int64_t snp_st
  * tped or .bed input.  garlic_gpu_code_alleles then codes the block with missing = 255. */
 int garlic_gpu_put_vcf_text(garlic_gpu_t *h, const char *text, const int64_t *line_off, int64_t snp0, int n_snp,
                             int32_t *n_cols, int32_t *max_allele, int32_t *bad_col);
+/* BCF 2.2 genotypes: per record the GT field's values (n_samples x count values of the width its typed descriptor
+ * names), record l of the block at gt + rec_off[l] (rec_off: n_snp + 1 entries, rec_off[l] % 4 == 0, the payloads in
+ * ascending order), gt_type[l] = the GT's descriptor byte (count << 4 | type, type 1/2/3 = int8/int16/int32; count 15
+ * = 15 or more), SNPs [snp0, snp0+n_snp), snp0 % 32 == 0.  Each value is (allele + 1) << 1 | phased; a call must be two
+ * values, each a missing allele (0 or 1) or an allele index 0..254, or a missing allele then end-of-vector (a lone '.'),
+ * or a count-1 field whose value is a missing allele.  Phase bits are ignored.  n_samples is the file's sample count:
+ * this handle's individuals [ind_offset, ind_offset+n_ind) are stored as allele index bytes, 255 = missing, and a
+ * record means exactly the VCF text record with the same GTs (garlic_gpu_put_vcf_text), so the coding, the "1" allele
+ * and --phased are the same.  Every handle decodes every sample, so the diagnostics are the same on all ranks; per
+ * record (each may be NULL): max_allele = largest allele index (-1 if none), bad_sample = first sample whose GT is
+ * malformed (-1 if none).  The caller checks max_allele against the record's ALT count.  Fails on a descriptor of
+ * another type or of count 0, a payload shorter than its descriptor needs, an offset that is not a multiple of 4, and
+ * a handle that holds tped or .bed input; BCF and VCF text blocks may be mixed on one handle.  Every call
+ * synchronises (the caller may reuse its buffers).  garlic_gpu_code_alleles then codes the block with missing = 255. */
+int garlic_gpu_put_bcf_gt(garlic_gpu_t *h, const uint8_t *gt, const int64_t *rec_off, const uint8_t *gt_type,
+                          int n_samples, int64_t snp0, int n_snp, int32_t *max_allele, int32_t *bad_sample);
 int garlic_gpu_code_alleles(garlic_gpu_t *h);
 
 /* ---- pre-coded input: packed 2-bit rows (codes 0/1/2, 3 = missing) -------------------------
@@ -125,7 +141,7 @@ void *garlic_gpu_counts_dev(garlic_gpu_t *h);
 int garlic_gpu_get_counts(garlic_gpu_t *h, int32_t *nalleles, int32_t *total, int32_t *hom, int32_t *nonmiss);
 /* the "1" allele per SNP after code_alleles (missing char if all calls missing).  After put_bed: 1 = the .bim's A1
  * (5th column), 2 = its A2 (6th column), missing if no call is present.  After put_vcf_text: the allele index
- * (0 = REF, k = the k-th ALT), or 255 if no allele is present (pass missing = (char)0xFF) */
+ * (0 = REF, k = the k-th ALT), or 255 if no allele is present (pass missing = (char)0xFF); the same after put_bcf_gt */
 int garlic_gpu_get_one_allele(garlic_gpu_t *h, uint8_t *allele, char missing);
 
 /* ---- optional per-genotype likelihoods (readTGLSData, src/garlic-data.cpp:1516-1586) -------
