@@ -28,7 +28,7 @@ EXPORTS = [
     "garlic_gpu_windows_dev", "garlic_gpu_windows_gather", "garlic_gpu_comm_id", "garlic_gpu_comm_init",
     "garlic_gpu_call_roh", "garlic_gpu_last_stats", "garlic_gpu_n_kept", "garlic_gpu_get_kept_index",
     "garlic_gpu_get_genotypes", "garlic_gpu_get_piece_bounds", "garlic_gpu_set_prune", "garlic_gpu_kde", "garlic_gpu_put_tgls_text", "garlic_gpu_get_gl",
-    "garlic_gpu_put_bed", "garlic_gpu_put_bed_dev", "garlic_gpu_put_vcf_text", "garlic_gpu_put_bcf_gt",
+    "garlic_gpu_put_bed", "garlic_gpu_put_bed_dev", "garlic_gpu_put_vcf_text", "garlic_gpu_put_bcf_gt", "garlic_gpu_select_columns",
 ]
 
 
@@ -119,6 +119,20 @@ class GarlicGPU:
         self.n_ind, self.L0, self.n_chr = int(n_ind), int(n_loci), len(co) - 1
         self._ck(self.lib.garlic_gpu_set_shape(self.h, C.c_int(n_ind), C.c_int(ind_offset), C.c_int64(n_loci),
                                                C.c_int(self.n_chr), _p(co), _p(po)))
+
+    def select_columns(self, columns, n_input):
+        """The input columns (individuals of the whole input, from 0) this handle holds: strictly ascending, below n_input,
+        one per individual of set_shape.  put_tped_text / put_vcf_text / put_bcf_gt / put_tgls_text / put_bed[_dev] then
+        store these columns; call after set_shape and before the first put_*."""
+        cols = np.ascontiguousarray(columns, np.int32)
+        if cols.ndim != 1 or len(cols) != self.n_ind:
+            raise GarlicError("select_columns: %d columns for a handle of %d individuals" % (cols.size, self.n_ind))
+        if (np.diff(cols) <= 0).any():
+            raise GarlicError("select_columns: the columns must be strictly ascending")
+        bad = cols[(cols < 0) | (cols >= n_input)]
+        if bad.size:
+            raise GarlicError("select_columns: column %d is outside [0, %d)" % (bad[0], n_input))
+        self._ck(self.lib.garlic_gpu_select_columns(self.h, _p(cols), C.c_int(n_input)))
 
     def put_alleles(self, alleles, snp0=0, missing="0"):
         a = np.ascontiguousarray(alleles, np.uint8)

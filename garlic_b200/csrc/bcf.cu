@@ -7,7 +7,8 @@
 // warp; a word whose four bytes are all non-negative is a valid pair of calls and is decoded with byte-SIMD
 // ((v >> 1) - 1 per byte, which is also 255 for a missing 0 or 1).  Any other word, and the int16 / int32 / count-1
 // layouts, go through bcf_gt.cuh:decode_gt one sample per thread.  Every rank decodes every sample so that the
-// per-record diagnostics are the same on all ranks; it stores only its own individuals [ind_lo, ind_lo + n_ind).  The
+// per-record diagnostics are the same on all ranks; it stores only its own individuals [ind_lo, ind_lo + n_ind), or with
+// SEL the samples listed in local[n_input] (common.cuh:select_local; the loads stay as they are, only the stores move).  The
 // diagnostics are reduced per warp and folded in with global atomics on arrays pre-set to -1 (atomicMax for the
 // largest allele index, an unsigned atomicMin for the first malformed sample), so a CTA never waits on a barrier.
 #include <cstdint>
@@ -29,14 +30,21 @@ __device__ __forceinline__ int32_t load_value(const uint8_t* p, long long k, int
     return __ldg((const int32_t*)p + k);
 }
 
-__device__ __forceinline__ void store_call(uint8_t* dst, long long i, long long lo, long long hi, uint32_t ab)
+template <bool SEL>
+__device__ __forceinline__ void store_call(uint8_t* dst, long long i, long long lo, long long hi, const int* local, int n_input,
+                                           uint32_t ab)
 {
-    if (i >= lo && i < hi) *(uint16_t*)(dst + 2 * (i - lo)) = (uint16_t)ab;
+    if (SEL) {
+        const int j = select_local(local, n_input, i);
+        if (j >= 0) *(uint16_t*)(dst + 2 * j) = (uint16_t)ab;
+    } else if (i >= lo && i < hi) *(uint16_t*)(dst + 2 * (i - lo)) = (uint16_t)ab;
 }
 
+template <bool SEL>
 __global__ void __launch_bounds__(kBcfThreads)
 decode_bcf_gt_kernel(const uint8_t* __restrict__ gt, const long long* __restrict__ off, const uint8_t* __restrict__ type,
-                     int n_snp, int n_samples, int n_ind, int ind_lo, uint8_t* __restrict__ alleles,
+                     int n_snp, int n_samples, int n_ind, int ind_lo, const int* __restrict__ local, int n_input,
+                     uint8_t* __restrict__ alleles,
                      int* __restrict__ max_allele, unsigned* __restrict__ bad_sample)
 {
     const long long lo = ind_lo, hi = (long long)ind_lo + n_ind;
@@ -84,8 +92,8 @@ decode_bcf_gt_kernel(const uint8_t* __restrict__ gt, const long long* __restrict
                             }
                         }
                     }
-                    store_call(dst, i, lo, hi, out);
-                    store_call(dst, i + 1, lo, hi, out >> 16);
+                    store_call<SEL>(dst, i, lo, hi, local, n_input, out);
+                    store_call<SEL>(dst, i + 1, lo, hi, local, n_input, out >> 16);
                 }
             }
             const uint32_t m = max(max(hmax & 0xff, (hmax >> 8) & 0xff), max((hmax >> 16) & 0xff, hmax >> 24));
@@ -103,7 +111,7 @@ decode_bcf_gt_kernel(const uint8_t* __restrict__ gt, const long long* __restrict
                 } else if ((unsigned)i < my_bad) {
                     my_bad = (unsigned)i;
                 }
-                store_call(dst, i, lo, hi, ok ? (uint32_t)(a | b << 8) : 0xffffu);
+                store_call<SEL>(dst, i, lo, hi, local, n_input, ok ? (uint32_t)(a | b << 8) : 0xffffu);
             }
         }
         for (int o = 16; o; o >>= 1) {
@@ -120,16 +128,21 @@ decode_bcf_gt_kernel(const uint8_t* __restrict__ gt, const long long* __restrict
 }  // namespace
 
 cudaError_t launch_decode_bcf_gt(const uint8_t* gt, const long long* off, const uint8_t* type, int n_snp, int n_samples,
-                                 int n_ind, int ind_lo, uint8_t* alleles, int* max_allele, int* bad_sample,
-                                 cudaStream_t st)
+                                 int n_ind, int ind_lo, const int* local, int n_input, uint8_t* alleles, int* max_allele,
+                                 int* bad_sample, cudaStream_t st)
 {
     if (!n_snp) return cudaSuccess;
     // -1 in both: "no allele" for atomicMax, and as unsigned the identity of atomicMin ("no malformed sample")
     cudaError_t e = cudaMemsetAsync(max_allele, 0xff, (size_t)n_snp * sizeof(int), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(bad_sample, 0xff, (size_t)n_snp * sizeof(int), st);
     if (e != cudaSuccess) return e;
-    decode_bcf_gt_kernel<<<n_snp < 148 * 8 ? n_snp : 148 * 8, kBcfThreads, 0, st>>>(
-        gt, off, type, n_snp, n_samples, n_ind, ind_lo, alleles, max_allele, (unsigned*)bad_sample);
+    const unsigned blocks = n_snp < 148 * 8 ? n_snp : 148 * 8;
+    if (local)
+        decode_bcf_gt_kernel<true><<<blocks, kBcfThreads, 0, st>>>(gt, off, type, n_snp, n_samples, n_ind, ind_lo, local, n_input,
+                                                                   alleles, max_allele, (unsigned*)bad_sample);
+    else
+        decode_bcf_gt_kernel<false><<<blocks, kBcfThreads, 0, st>>>(gt, off, type, n_snp, n_samples, n_ind, ind_lo, nullptr, 0,
+                                                                    alleles, max_allele, (unsigned*)bad_sample);
     return cudaGetLastError();
 }
 

@@ -5,13 +5,15 @@
 // 3 = hom A2.  The equivalent tped writes hom A1 as "A1 A1", het as "A1 A2", hom A2 as "A2 A2", missing as "0 0", so the
 // "1" allele (the first non-missing character, garlic-data.cpp:112-113) is A2 iff the first present call is hom A2.
 // The caller stages, per SNP, the byte columns that hold its own individuals: field sh + i of a staged row is this
-// rank's individual i (sh = ind_offset % 4), the fields around them belong to other ranks and are ignored.
+// rank's individual i (sh = ind_offset % 4), the fields around them belong to other ranks and are ignored.  With a column
+// selection the whole rows are staged by bed_select_kernel, which gathers the listed columns to fields 0 .. n_ind (sh = 0).
 //   phase a (bed_count_kernel, per uploaded block): first-allele key ((2·global_ind) << 8 | id, id 1 = A1, 2 = A2 —
 //            the key format of first_allele_kernel) and the four counters, nalleles counting copies of A2;
 //   phase b (bed_code): nalleles of the SNPs whose "1" allele is A1 become total - nalleles, then the 2-bit transpose
 //            into the individual-major packed matrix with the per-SNP recode as whole-word bit operations.
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "bed_select.cuh"
 #include "common.cuh"
 #include "kernels.h"
 
@@ -167,7 +169,53 @@ bed_transpose_kernel(const uint8_t* __restrict__ stage, int64_t stride, long lon
     }
 }
 
+// A column selection (garlic_gpu_select_columns): one warp per SNP row.  The warp stages the row in shared memory as the
+// 16-byte aligned chunks that cover it (coalesced loads; the chunks never leave the aligned blocks that hold row bytes),
+// then each lane forms output bytes from four listed columns (bed_select.cuh:bed_gather_byte), reading the column list
+// through L1.  A row too long for shared memory (smem_row = 0) is read from global memory instead.
+constexpr int kSelWarps = 4;
+
+__global__ void __launch_bounds__(kSelWarps * 32)
+bed_select_kernel(const uint8_t* __restrict__ rows, int64_t in_stride, int n_snp, const int32_t* __restrict__ cols, int n_ind,
+                  uint8_t* __restrict__ stage, int64_t stride, int smem_row)
+{
+    extern __shared__ uint4 s_rows[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint4* my = s_rows + (size_t)warp * (smem_row / 16);
+    const long long out_bytes = (n_ind + 3) / 4;
+    for (long long s = (long long)blockIdx.x * kSelWarps + warp; s < n_snp; s += (long long)gridDim.x * kSelWarps) {
+        const uint8_t* row = rows + s * in_stride;
+        const uint8_t* src = row;
+        if (smem_row) {
+            const uintptr_t a0 = (uintptr_t)row & ~(uintptr_t)15, a1 = ((uintptr_t)row + in_stride + 15) & ~(uintptr_t)15;
+            const int n16 = (int)((a1 - a0) / 16);
+            for (int k = lane; k < n16; k += 32) my[k] = __ldg(reinterpret_cast<const uint4*>(a0) + k);
+            __syncwarp();
+            src = reinterpret_cast<const uint8_t*>(my) + ((uintptr_t)row & 15);
+        }
+        uint8_t* out = stage + s * stride;
+        for (long long ob = lane; ob < out_bytes; ob += 32) out[ob] = bed_gather_byte(src, cols, n_ind, ob);
+        __syncwarp();
+    }
+}
+
 }  // namespace
+
+cudaError_t launch_bed_select(const uint8_t* rows, int64_t in_stride, int n_snp, const int32_t* cols, int n_ind, uint8_t* stage,
+                              int64_t stride, cudaStream_t st)
+{
+    if (n_snp <= 0) return cudaSuccess;
+    const int64_t need = (in_stride + 30 + 15) / 16 * 16;               // the aligned chunks covering a row
+    const int smem_row = need * kSelWarps <= 200 * 1024 ? (int)need : 0;
+    if (smem_row * kSelWarps > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(bed_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_row * kSelWarps);
+        if (e != cudaSuccess) return e;
+    }
+    const int blocks = (n_snp + kSelWarps - 1) / kSelWarps < 148 * 16 ? (n_snp + kSelWarps - 1) / kSelWarps : 148 * 16;
+    bed_select_kernel<<<blocks, kSelWarps * 32, (size_t)smem_row * kSelWarps, st>>>(rows, in_stride, n_snp, cols, n_ind, stage,
+                                                                                    stride, smem_row);
+    return cudaGetLastError();
+}
 
 cudaError_t launch_bed_count(const uint8_t* stage, int64_t stride, int n_snp, int sh, int n_ind, int ind_offset,
                              int* counts, long long L0, unsigned long long* key, cudaStream_t st)

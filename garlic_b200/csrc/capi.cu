@@ -73,6 +73,12 @@ struct garlic_gpu {
     int* d_nonblank = nullptr;
     uint8_t* d_gt_type = nullptr;     // BCF: per record the GT's typed descriptor (put_bcf_gt; payloads staged in d_text)
     int2* d_hard = nullptr;           // K0-GL: tokens the device conversion leaves to strtod
+    // select_columns: the handle holds input columns sel_cols (ascending) of n_input instead of [ind_offset, +n_ind);
+    // d_local[col] = the handle's individual of input column col, or -1
+    std::vector<int32_t> sel_cols;
+    int n_input = 0;
+    int* d_local = nullptr;
+    int32_t* d_sel_cols = nullptr;
     StitchScratch stitch_scratch;     // host buffers of call_roh kept between calls
     std::vector<RohRec> recs_buf, ambs_buf, merged_buf, tmp_buf;
     uint64_t* d_ldplanes = nullptr;   // LD scratch: bit-planes and the ordered pair matrix (kept between calls)
@@ -504,6 +510,7 @@ void garlic_gpu_destroy(garlic_gpu_t* h)
     free_counts(h);
     dev_free(h->d_gl0); dev_free(h->d_gl); dev_free(h->d_freq0); dev_free(h->d_freq); dev_free(h->d_lut);
     dev_free(h->d_ldplanes); dev_free(h->d_ldpairs); dev_free(h->d_text); dev_free(h->d_textoff); dev_free(h->d_nonblank); dev_free(h->d_gt_type);
+    dev_free(h->d_local); dev_free(h->d_sel_cols);
     dev_free(h->d_gpos); dev_free(h->d_nomut); dev_free(h->d_norec); dev_free(h->d_wlut); dev_free(h->d_invld);
     dev_free(h->d_homf); dev_free(h->d_keep); dev_free(h->d_src); dev_free(h->d_pos0); dev_free(h->d_chr_of0);
     dev_free(h->d_pos); dev_free(h->d_chr_of); dev_free(h->d_chr_start); dev_free(h->d_chr_param);
@@ -603,6 +610,31 @@ int garlic_gpu_set_shape(garlic_gpu_t* h, int n_ind, int ind_offset, int64_t n_l
     h->have_geno0 = false; h->filtered = false; h->tables = false; h->have_gl = false; h->have_ld = false;
     dev_free(h->d_alleles); dev_free(h->d_key); dev_free(h->d_bed);
     h->bed_input = false; h->vcf_input = false;
+    h->sel_cols.clear(); h->n_input = 0;
+    return 0;
+}
+
+int garlic_gpu_select_columns(garlic_gpu_t* h, const int32_t* columns, int n_input)
+{
+    if (!h) return 1;
+    if (!h->L0) FAIL("select_columns: call set_shape first");
+    if (h->d_alleles || h->d_bed || h->have_geno0 || h->have_gl) FAIL("select_columns: call it before the first put_*");
+    if (n_input < h->n_ind) FAIL("select_columns: n_input is smaller than the handle's number of individuals");
+    for (int i = 0; i < h->n_ind; ++i) {
+        if (columns[i] < 0 || columns[i] >= n_input)
+            FAIL("select_columns: column " + std::to_string(columns[i]) + " is outside [0, " + std::to_string(n_input) + ")");
+        if (i && columns[i] <= columns[i - 1]) FAIL("select_columns: the columns must be strictly ascending");
+    }
+    CK(cudaSetDevice(h->device));
+    std::vector<int32_t> local(n_input, -1);
+    for (int i = 0; i < h->n_ind; ++i) local[columns[i]] = i;
+    if (dev_alloc(h, &h->d_local, (size_t)n_input)) return 1;
+    if (dev_alloc(h, &h->d_sel_cols, (size_t)h->n_ind)) return 1;
+    CK(cudaMemcpyAsync(h->d_local, local.data(), (size_t)n_input * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->d_sel_cols, columns, (size_t)h->n_ind * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    h->sel_cols.assign(columns, columns + h->n_ind);
+    h->n_input = n_input;
     return 0;
 }
 
@@ -651,7 +683,8 @@ int garlic_gpu_put_tped_text(garlic_gpu_t* h, const char* text, const int64_t* l
     uint8_t* dst = h->d_alleles + (size_t)snp0 * h->n_ind * 2;
     // a short line leaves its tail untouched: pre-fill with the missing character so that nothing undefined is coded
     CK(cudaMemsetAsync(dst, (unsigned char)missing, (size_t)n_snp * h->n_ind * 2, h->stream));
-    LAUNCH(launch_tokenize_tped(h->d_text, h->d_textoff, n_snp, h->n_ind, h->ind_offset, dst, h->d_nonblank, h->stream));
+    LAUNCH(launch_tokenize_tped(h->d_text, h->d_textoff, n_snp, h->n_ind, h->ind_offset, h->n_input ? h->d_local : nullptr,
+                                h->n_input, dst, h->d_nonblank, h->stream));
     LAUNCH(launch_first_allele(dst, n_snp, h->n_ind, h->ind_offset, (unsigned char)missing, h->d_key + snp0, h->stream));
     h->missing_char = (unsigned char)missing;
     if (nonblank) CK(cudaMemcpyAsync(nonblank, h->d_nonblank, (size_t)n_snp * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
@@ -686,8 +719,8 @@ int garlic_gpu_put_vcf_text(garlic_gpu_t* h, const char* text, const int64_t* li
     // a short record leaves its tail untouched: pre-fill with the missing code so that nothing undefined is coded
     CK(cudaMemsetAsync(dst, 255, (size_t)n_snp * h->n_ind * 2, h->stream));
     int* diag = h->d_nonblank;
-    LAUNCH(launch_tokenize_vcf(h->d_text, h->d_textoff, n_snp, h->n_ind, h->ind_offset, dst, diag, diag + n_snp,
-                               diag + 2 * n_snp, h->stream));
+    LAUNCH(launch_tokenize_vcf(h->d_text, h->d_textoff, n_snp, h->n_ind, h->ind_offset, h->n_input ? h->d_local : nullptr,
+                               h->n_input, dst, diag, diag + n_snp, diag + 2 * n_snp, h->stream));
     LAUNCH(launch_first_allele(dst, n_snp, h->n_ind, h->ind_offset, 255, h->d_key + snp0, h->stream));
     h->missing_char = 255;
     int32_t* out[3] = {n_cols, max_allele, bad_col};
@@ -706,7 +739,8 @@ int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec
     if (n_snp <= 0) return 0;
     if (h->bed_input) FAIL("put_bcf_gt: this handle holds .bed input");
     if (h->d_alleles && !h->vcf_input) FAIL("put_bcf_gt: this handle holds tped input");
-    if (n_samples < h->ind_offset + h->n_ind) FAIL("put_bcf_gt: n_samples does not cover this handle's individuals");
+    if (h->n_input ? n_samples <= h->sel_cols.back() : n_samples < h->ind_offset + h->n_ind)
+        FAIL("put_bcf_gt: n_samples does not cover this handle's individuals");
     for (int l = 0; l < n_snp; ++l) {
         const int count = gt_type[l] >> 4, t = gt_type[l] & 15;
         if (count == 0 || t < 1 || t > 3)
@@ -736,7 +770,7 @@ int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec
     int* diag = h->d_nonblank;
     // every sample of this handle is stored (a malformed one as 255), so no pre-fill is needed
     LAUNCH(launch_decode_bcf_gt((const uint8_t*)h->d_text, h->d_textoff, h->d_gt_type, n_snp, n_samples, h->n_ind,
-                                h->ind_offset, dst, diag, diag + n_snp, h->stream));
+                                h->ind_offset, h->n_input ? h->d_local : nullptr, h->n_input, dst, diag, diag + n_snp, h->stream));
     LAUNCH(launch_first_allele(dst, n_snp, h->n_ind, h->ind_offset, 255, h->d_key + snp0, h->stream));
     h->missing_char = 255;
     int32_t* out[2] = {max_allele, bad_sample};
@@ -748,15 +782,18 @@ int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec
 
 void* garlic_gpu_first_allele_keys_dev(garlic_gpu_t* h) { return h ? (void*)h->d_key : nullptr; }
 
-// .bed rows of the whole file → this handle's byte columns of SNPs [snp0, snp0 + n_snp), then phase a (bed.cu)
+// .bed rows of the whole file → this handle's byte columns of SNPs [snp0, snp0 + n_snp), then phase a (bed.cu).  With a
+// column selection the whole rows go to the device and bed_select_kernel gathers the listed fields to bit offset 0.
 static int put_bed_common(garlic_gpu* h, const void* rows, int64_t stride, int64_t snp0, int n_snp, cudaMemcpyKind kind)
 {
     CK(cudaSetDevice(h->device));
     if (!h->L0) FAIL("put_bed: call set_shape first");
     if (snp0 % 32 != 0 || snp0 < 0 || n_snp < 0 || snp0 + n_snp > h->L0) FAIL("put_bed: bad SNP range (snp0 must be a multiple of 32)");
     if (h->d_alleles) FAIL("put_bed: this handle holds allele input");
-    const int64_t byte0 = h->ind_offset / 4, sh = h->ind_offset % 4;
+    const bool sel = h->n_input > 0;
+    const int64_t byte0 = sel ? 0 : h->ind_offset / 4, sh = sel ? 0 : h->ind_offset % 4;
     const int64_t width = (sh + h->n_ind + 3) / 4;
+    if (sel && stride < (h->n_input + 3) / 4) FAIL("put_bed: SNP row stride smaller than ceil(n_input/4)");
     if (stride < byte0 + width) FAIL("put_bed: SNP row stride smaller than the bytes of this handle's individuals");
     if (!h->d_bed) {
         h->bed_stride = (width + 31) / 32 * 32;               // whole 32-byte sectors per row (bed_transpose_kernel)
@@ -766,7 +803,16 @@ static int put_bed_common(garlic_gpu* h, const void* rows, int64_t stride, int64
     }
     if (n_snp == 0) return 0;
     uint8_t* dst = h->d_bed + (size_t)snp0 * h->bed_stride;
-    if (kind == cudaMemcpyHostToDevice && width == stride) {
+    if (sel) {
+        if (kind == cudaMemcpyHostToDevice) {
+            if (dev_alloc(h, &h->d_bed_rows, (size_t)n_snp * stride)) return 1;
+            CK(cudaMemcpyAsync(h->d_bed_rows, rows, (size_t)n_snp * stride, kind, h->stream));
+            CK(cudaEventRecord(h->ev_copy, h->stream));
+            rows = h->d_bed_rows;
+        }
+        LAUNCH(launch_bed_select((const uint8_t*)rows, stride, n_snp, h->d_sel_cols, h->n_ind, dst, h->bed_stride, h->stream));
+        if (kind == cudaMemcpyDeviceToDevice) CK(cudaEventRecord(h->ev_copy, h->stream));   // the kernel read the caller's rows
+    } else if (kind == cudaMemcpyHostToDevice && width == stride) {
         // a pitched host-to-device copy costs about 0.13 us per row (76 ms for the 600 k rows of a 2,000-individual file
         // on a B200 box): a handle that keeps every column takes the rows in one piece and re-pitches them on the device
         if (dev_alloc(h, &h->d_bed_rows, (size_t)n_snp * stride)) return 1;
@@ -774,9 +820,11 @@ static int put_bed_common(garlic_gpu* h, const void* rows, int64_t stride, int64
         rows = h->d_bed_rows;
         kind = cudaMemcpyDeviceToDevice;
     }
-    CK(cudaMemcpy2DAsync(dst, (size_t)h->bed_stride, (const uint8_t*)rows + byte0, (size_t)stride, (size_t)width, (size_t)n_snp,
-                         kind, h->stream));
-    CK(cudaEventRecord(h->ev_copy, h->stream));
+    if (!sel) {
+        CK(cudaMemcpy2DAsync(dst, (size_t)h->bed_stride, (const uint8_t*)rows + byte0, (size_t)stride, (size_t)width, (size_t)n_snp,
+                             kind, h->stream));
+        CK(cudaEventRecord(h->ev_copy, h->stream));
+    }
     LAUNCH(launch_bed_count(dst, h->bed_stride, n_snp, (int)sh, h->n_ind, h->ind_offset, h->d_counts + snp0, h->L0,
                             h->d_key + snp0, h->stream));
     h->counts_reduced = false; h->counts_hi_reduced = false;
@@ -804,7 +852,7 @@ int garlic_gpu_code_alleles(garlic_gpu_t* h)
     if (h->d_bed) {
         // put_bed's phase a left the counters of every SNP; nothing reads the staged rows after the transpose
         if (dev_alloc(h, &h->d_a1, (size_t)(h->L0 + 31) / 32)) return 1;
-        LAUNCH(launch_bed_code(h->d_bed, h->bed_stride, h->L0, h->ind_offset % 4, h->n_ind, h->d_key, h->d_counts, h->d_a1,
+        LAUNCH(launch_bed_code(h->d_bed, h->bed_stride, h->L0, h->n_input ? 0 : h->ind_offset % 4, h->n_ind, h->d_key, h->d_counts, h->d_a1,
                                h->d_geno0, h->row_words0, h->stream));
         h->launches++;                     // (two kernels)
         CK(cudaStreamSynchronize(h->stream));
@@ -964,8 +1012,8 @@ int garlic_gpu_put_tgls_text(garlic_gpu_t* h, const char* text, const int64_t* l
     CK(cudaMemcpyAsync(h->d_text, base, (size_t)bytes, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(h->d_textoff, rel.data(), rel.size() * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemsetAsync(d_hard_n, 0, sizeof(unsigned), h->stream));
-    LAUNCH(launch_tokenize_tgls(h->d_text, h->d_textoff, n_snp, h->n_ind, h->ind_offset, h->d_gl0, h->L0, snp0, h->d_nonblank,
-                                h->d_hard, d_hard_n, hard_cap, h->stream));
+    LAUNCH(launch_tokenize_tgls(h->d_text, h->d_textoff, n_snp, h->n_ind, h->ind_offset, h->n_input ? h->d_local : nullptr,
+                                h->n_input, h->d_gl0, h->L0, snp0, h->d_nonblank, h->d_hard, d_hard_n, hard_cap, h->stream));
     std::vector<int32_t> ntok_local;
     if (!n_tokens) { ntok_local.resize(n_snp); n_tokens = ntok_local.data(); }
     unsigned n_hard = 0;
@@ -998,14 +1046,16 @@ int garlic_gpu_put_tgls_text(garlic_gpu_t* h, const char* text, const int64_t* l
             CK(cudaMemcpy(list.data(), h->d_hard, n_hard * sizeof(int2), cudaMemcpyDeviceToHost));
         } else {
             for (int l = 0; l < n_snp; ++l)
-                for (int k = h->ind_offset; k < h->ind_offset + h->n_ind; ++k) list.push_back(make_int2(l, k));
+                for (int i = 0; i < h->n_ind; ++i) list.push_back(make_int2(l, h->n_input ? h->sel_cols[i] : h->ind_offset + i));
         }
         std::sort(list.begin(), list.end(), [](const int2& a, const int2& b) { return a.x != b.x ? a.x < b.x : a.y < b.y; });
         for (const int2& t : list) {
             const char* p = token_at(t.x, t.y);
             if (!p) continue;
             const double v = convert(p, t.x);
-            CK(cudaMemcpyAsync(h->d_gl0 + (size_t)(t.y - h->ind_offset) * h->L0 + snp0 + t.x, &v, sizeof(double), cudaMemcpyHostToDevice, h->stream));
+            const int64_t i = h->n_input ? std::lower_bound(h->sel_cols.begin(), h->sel_cols.end(), t.y) - h->sel_cols.begin()
+                                         : t.y - h->ind_offset;
+            CK(cudaMemcpyAsync(h->d_gl0 + (size_t)i * h->L0 + snp0 + t.x, &v, sizeof(double), cudaMemcpyHostToDevice, h->stream));
             CK(cudaStreamSynchronize(h->stream));                          // v lives on this stack frame
         }
     }

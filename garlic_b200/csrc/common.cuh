@@ -68,6 +68,13 @@ struct WalkParams {
 // next to each other for every SNP, so a warp walking 32 consecutive individuals reads 256 contiguous bytes per SNP
 // and a group's SNP range is one contiguous slab (what gl_walk_kernel copies with cp.async.bulk).
 constexpr int kGlLanes = 32;
+// Column selection of the ingest kernels (garlic_gpu_select_columns): local[col] is the handle's individual that input
+// column col holds, or -1.  Columns at or beyond n_input (the extra columns of a malformed line) are never stored.
+GHD int select_local(const int* local, int n_input, long long col)
+{
+    return col < n_input ? local[col] : -1;
+}
+
 GHD const double* gl_lane(const WalkParams& P, int ind)
 {
     return P.gl + ((int64_t)(ind >> 5) * P.gl_stride) * kGlLanes + (ind & 31);

@@ -2,7 +2,8 @@
 // `ss >> gl` loop, garlic-data.cpp:1538-1554; SURVEY §8f.1).  The host hands over, per line, the raw text that follows
 // the 4th field; token k of a line (blank-separated) is individual k's value.  One CTA per line: every thread scans 16
 // characters, a block scan ranks the token starts, and the thread that owns a start converts its token to fp64 and
-// stores it into the individual-major matrix garlic_gpu_put_gl fills (this rank keeps its own individuals' tokens).
+// stores it into the individual-major matrix garlic_gpu_put_gl fills (this rank keeps its own individuals' tokens, or
+// with SEL the columns listed in local[n_input], common.cuh:select_local).
 // Consecutive lines are handled by neighbouring CTAs, so the 8-byte stores of one individual's row merge into whole
 // sectors in L2 before they reach HBM.
 //
@@ -67,10 +68,11 @@ __device__ double parse_decimal(const char* p, long long n, bool* hard)
     return neg ? -v : v;
 }
 
+template <bool SEL>
 __global__ void __launch_bounds__(256)
 tokenize_tgls_kernel(const char* __restrict__ text, const long long* __restrict__ off, int n_snp, int n_ind, int ind_lo,
-                     double* __restrict__ out, int64_t out_stride, long long snp0, int* __restrict__ n_tokens,
-                     int2* __restrict__ hard_list, unsigned* __restrict__ hard_count, unsigned hard_cap)
+                     const int* __restrict__ local, int n_input, double* __restrict__ out, int64_t out_stride, long long snp0,
+                     int* __restrict__ n_tokens, int2* __restrict__ hard_list, unsigned* __restrict__ hard_count, unsigned hard_cap)
 {
     __shared__ int s_warp[8];
     __shared__ int s_base;
@@ -102,11 +104,13 @@ tokenize_tgls_kernel(const char* __restrict__ text, const long long* __restrict_
             for (int w = 0; w < 8; ++w) if (w < warp) wbase += s_warp[w];
             int k = s_base + wbase + incl - n;                           // rank of this thread's first token
             for (; starts; starts &= starts - 1u, ++k) {
-                if (k < ind_lo || k >= ind_lo + n_ind) continue;
+                int j;
+                if (SEL) { j = select_local(local, n_input, k); if (j < 0) continue; }
+                else { if (k < ind_lo || k >= ind_lo + n_ind) continue; j = k - ind_lo; }
                 const long long at = i0 + (__ffs((int)starts) - 1);
                 bool hard = false;
                 const double v = parse_decimal(line + at, len - at, &hard);
-                out[(int64_t)(k - ind_lo) * out_stride + snp0 + l] = v;
+                out[(int64_t)j * out_stride + snp0 + l] = v;
                 if (hard) {
                     const unsigned slot = atomicAdd(hard_count, 1u);
                     if (slot < hard_cap) hard_list[slot] = make_int2(l, k);
@@ -123,13 +127,18 @@ tokenize_tgls_kernel(const char* __restrict__ text, const long long* __restrict_
 
 }  // namespace
 
-cudaError_t launch_tokenize_tgls(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, double* out,
-                                 int64_t out_stride, long long snp0, int* n_tokens, int2* hard_list, unsigned* hard_count,
-                                 unsigned hard_cap, cudaStream_t st)
+cudaError_t launch_tokenize_tgls(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
+                                 int n_input, double* out, int64_t out_stride, long long snp0, int* n_tokens, int2* hard_list,
+                                 unsigned* hard_count, unsigned hard_cap, cudaStream_t st)
 {
     if (!n_snp) return cudaSuccess;
-    tokenize_tgls_kernel<<<n_snp < 148 * 8 ? n_snp : 148 * 8, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, out, out_stride, snp0,
-                                                                          n_tokens, hard_list, hard_count, hard_cap);
+    const unsigned blocks = n_snp < 148 * 8 ? n_snp : 148 * 8;
+    if (local)
+        tokenize_tgls_kernel<true><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, local, n_input, out, out_stride, snp0,
+                                                           n_tokens, hard_list, hard_count, hard_cap);
+    else
+        tokenize_tgls_kernel<false><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, nullptr, 0, out, out_stride, snp0,
+                                                            n_tokens, hard_list, hard_count, hard_cap);
     return cudaGetLastError();
 }
 

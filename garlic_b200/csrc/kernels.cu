@@ -920,11 +920,13 @@ __global__ void first_allele_kernel(const uint8_t* __restrict__ alleles, int n_s
 // raw text; here one CTA per line ranks the non-blank characters (per-thread count, block scan) and scatters the ones
 // belonging to this GPU's individuals [ind_lo, ind_lo + n_ind) into the [n_snp][n_ind][2] allele block K1 works on.
 // nonblank[l] = number of non-blank characters of line l (the host checks it against 2 x individuals).
+// SEL: the handle holds the columns listed in local[n_input] (common.cuh:select_local) instead of the range.
 // ------------------------------------------------------------------------------------------
 constexpr int kTokChars = 16;   // characters per thread per tile
+template <bool SEL>
 __global__ void __launch_bounds__(256)
 tokenize_tped_kernel(const char* __restrict__ text, const long long* __restrict__ off, int n_snp, int n_ind, int ind_lo,
-                     uint8_t* __restrict__ alleles, int* __restrict__ nonblank)
+                     const int* __restrict__ local, int n_input, uint8_t* __restrict__ alleles, int* __restrict__ nonblank)
 {
     __shared__ int s_warp[8];
     __shared__ int s_base;
@@ -958,7 +960,10 @@ tokenize_tped_kernel(const char* __restrict__ text, const long long* __restrict_
 #pragma unroll
             for (int q = 0; q < kTokChars; ++q)
                 if (c[q] != ' ' && c[q] != '\t' && c[q] != '\r' && c[q] != '\n') {
-                    if (k >= k_lo && k < k_hi) dst[k - k_lo] = (uint8_t)c[q];
+                    if (SEL) {
+                        const int j = select_local(local, n_input, k >> 1);
+                        if (j >= 0) dst[2 * j + (k & 1)] = (uint8_t)c[q];
+                    } else if (k >= k_lo && k < k_hi) dst[k - k_lo] = (uint8_t)c[q];
                     ++k;
                 }
             __syncthreads();
@@ -970,11 +975,13 @@ tokenize_tped_kernel(const char* __restrict__ text, const long long* __restrict_
     }
 }
 
-cudaError_t launch_tokenize_tped(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, uint8_t* alleles,
-                                 int* nonblank, cudaStream_t st)
+cudaError_t launch_tokenize_tped(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
+                                 int n_input, uint8_t* alleles, int* nonblank, cudaStream_t st)
 {
     if (!n_snp) return cudaSuccess;
-    tokenize_tped_kernel<<<n_snp < 148 * 8 ? n_snp : 148 * 8, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, alleles, nonblank);
+    const unsigned blocks = n_snp < 148 * 8 ? n_snp : 148 * 8;
+    if (local) tokenize_tped_kernel<true><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, local, n_input, alleles, nonblank);
+    else tokenize_tped_kernel<false><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, nullptr, 0, alleles, nonblank);
     return cudaGetLastError();
 }
 

@@ -73,18 +73,20 @@ cudaError_t launch_thin_windows(const uint64_t* geno, int64_t row_words, const d
 cudaError_t launch_fill_f64(double* p, size_t n, double v, cudaStream_t st);
 cudaError_t launch_bucket_by_individual(RohRec* in, const unsigned* count, unsigned cap, unsigned* hist, int n_ind,
                                         RohRec* out, int thr, unsigned* kept, unsigned* total, cudaStream_t st);
-cudaError_t launch_tokenize_tped(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, uint8_t* alleles,
-                                 int* nonblank, cudaStream_t st);
+// The ingest kernels store the input columns [ind_lo, ind_lo + n_ind), or with local != nullptr the columns that
+// local[n_input] maps to an individual (garlic_gpu_select_columns, common.cuh:select_local)
+cudaError_t launch_tokenize_tped(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
+                                 int n_input, uint8_t* alleles, int* nonblank, cudaStream_t st);
 // vcf.cu: VCF sample columns → allele index bytes (255 = missing) and per record the column count, the largest allele
 // index (-1 if none) and the first column whose GT is malformed (-1 if none)
-cudaError_t launch_tokenize_vcf(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, uint8_t* alleles,
-                                int* n_cols, int* max_allele, int* bad_col, cudaStream_t st);
+cudaError_t launch_tokenize_vcf(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
+                                int n_input, uint8_t* alleles, int* n_cols, int* max_allele, int* bad_col, cudaStream_t st);
 // bcf.cu: BCF GT vectors (record l: n_samples x count values at gt + off[l], type[l] = the GT's typed descriptor) →
 // allele index bytes (255 = missing) and per record the largest allele index (-1 if none) and the first malformed
 // sample (-1 if none)
 cudaError_t launch_decode_bcf_gt(const uint8_t* gt, const long long* off, const uint8_t* type, int n_snp, int n_samples,
-                                 int n_ind, int ind_lo, uint8_t* alleles, int* max_allele, int* bad_sample,
-                                 cudaStream_t st);
+                                 int n_ind, int ind_lo, const int* local, int n_input, uint8_t* alleles, int* max_allele,
+                                 int* bad_sample, cudaStream_t st);
 cudaError_t launch_first_allele(const uint8_t* alleles, int n_snp, int n_ind, int ind_offset, int missing,
                                 unsigned long long* key, cudaStream_t st);
 cudaError_t launch_code_alleles(const uint8_t* alleles, int n_snp, int n_ind, int missing,
@@ -93,6 +95,10 @@ cudaError_t launch_code_alleles(const uint8_t* alleles, int n_snp, int n_ind, in
 cudaError_t launch_count_packed(const uint64_t* geno, int64_t row_words, int n_ind, long long L0,
                                 int* counts, cudaStream_t st);
 // bed.cu: PLINK .bed rows staged SNP-major ([n_snp][stride] bytes, this rank's individual i at field sh + i)
+// whole .bed rows ([n_snp][in_stride] bytes) → the fields of the listed columns cols[n_ind] (ascending), dense from bit 0
+// of each staged row (bed_select.cuh:bed_gather_byte)
+cudaError_t launch_bed_select(const uint8_t* rows, int64_t in_stride, int n_snp, const int32_t* cols, int n_ind, uint8_t* stage,
+                              int64_t stride, cudaStream_t st);
 cudaError_t launch_bed_count(const uint8_t* stage, int64_t stride, int n_snp, int sh, int n_ind, int ind_offset,
                              int* counts, long long L0, unsigned long long* key, cudaStream_t st);
 cudaError_t launch_bed_code(const uint8_t* stage, int64_t stride, long long L0, int sh, int n_ind,
@@ -115,9 +121,9 @@ cudaError_t launch_wlod_weights(const int* pos, const double* gpos, const int* c
 cudaError_t launch_build_wlut(const double* lut, const double* nomut, const double* norec, long long L,
                               double* wlut, cudaStream_t st);
 // K0-GL (ingest.cu): tgls value columns from raw text into the individual-major matrix out[(k - ind_lo) * out_stride + snp0 + l]
-cudaError_t launch_tokenize_tgls(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, double* out,
-                                 int64_t out_stride, long long snp0, int* n_tokens, int2* hard_list, unsigned* hard_count,
-                                 unsigned hard_cap, cudaStream_t st);
+cudaError_t launch_tokenize_tgls(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
+                                 int n_input, double* out, int64_t out_stride, long long snp0, int* n_tokens, int2* hard_list,
+                                 unsigned* hard_count, unsigned hard_cap, cudaStream_t st);
 // the counter exchange over NVLink peer memory, fused with freq + keep (xchg.cu)
 constexpr int kXchgMaxRanks = 16, kXchgReady = 0, kXchgDone = 16;   // flag words per rank: ready[16] | done[16]
 struct XchgParams {

@@ -5,7 +5,7 @@
 // column starts (position 0 of a non-empty record and every position after a '\t'), and the thread that owns a column
 // start parses that column's GT (vcf_gt.cuh:parse_gt) from global memory.  Every rank parses every column so that the
 // per-record diagnostics are the same on all ranks; it stores only the columns of its own individuals
-// [ind_lo, ind_lo + n_ind).
+// [ind_lo, ind_lo + n_ind), or with SEL the columns listed in local[n_input] (common.cuh:select_local).
 #include <climits>
 #include <cstdint>
 
@@ -18,10 +18,11 @@ namespace {
 
 constexpr int kVcfChars = 16;   // characters per thread per tile
 
+template <bool SEL>
 __global__ void __launch_bounds__(256)
 tokenize_vcf_kernel(const char* __restrict__ text, const long long* __restrict__ off, int n_snp, int n_ind, int ind_lo,
-                    uint8_t* __restrict__ alleles, int* __restrict__ n_cols, int* __restrict__ max_allele,
-                    int* __restrict__ bad_col)
+                    const int* __restrict__ local, int n_input, uint8_t* __restrict__ alleles, int* __restrict__ n_cols,
+                    int* __restrict__ max_allele, int* __restrict__ bad_col)
 {
     __shared__ int s_warp[8];
     __shared__ int s_base, s_max, s_bad;
@@ -61,7 +62,10 @@ tokenize_vcf_kernel(const char* __restrict__ text, const long long* __restrict__
                 const long long i = i0 + k;
                 int a, b;
                 if (parse_gt(line + i, len - i, &a, &b)) {
-                    if (col >= c_lo && col < c_hi) {
+                    if (SEL) {
+                        const int j = select_local(local, n_input, col);
+                        if (j >= 0) { dst[2 * j] = (uint8_t)a; dst[2 * j + 1] = (uint8_t)b; }
+                    } else if (col >= c_lo && col < c_hi) {
                         dst[2 * (col - c_lo)] = (uint8_t)a;
                         dst[2 * (col - c_lo) + 1] = (uint8_t)b;
                     }
@@ -93,12 +97,17 @@ tokenize_vcf_kernel(const char* __restrict__ text, const long long* __restrict__
 
 }  // namespace
 
-cudaError_t launch_tokenize_vcf(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, uint8_t* alleles,
-                                int* n_cols, int* max_allele, int* bad_col, cudaStream_t st)
+cudaError_t launch_tokenize_vcf(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
+                                int n_input, uint8_t* alleles, int* n_cols, int* max_allele, int* bad_col, cudaStream_t st)
 {
     if (!n_snp) return cudaSuccess;
-    tokenize_vcf_kernel<<<n_snp < 148 * 8 ? n_snp : 148 * 8, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, alleles, n_cols,
-                                                                          max_allele, bad_col);
+    const unsigned blocks = n_snp < 148 * 8 ? n_snp : 148 * 8;
+    if (local)
+        tokenize_vcf_kernel<true><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, local, n_input, alleles, n_cols,
+                                                          max_allele, bad_col);
+    else
+        tokenize_vcf_kernel<false><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, nullptr, 0, alleles, n_cols,
+                                                           max_allele, bad_col);
     return cudaGetLastError();
 }
 

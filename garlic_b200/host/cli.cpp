@@ -32,10 +32,12 @@ void Log::close()
 }
 void Log::line(const std::string& s)
 {
+    if (hold) { held.push_back(s); return; }
     if (log) { fputs(s.c_str(), log); fputc('\n', log); fflush(log); }
 }
 void Log::error(const std::string& s)
 {
+    last = s;
     fprintf(stderr, "%s\n", s.c_str());
     if (err) { fputs(s.c_str(), err); fputc('\n', err); fflush(err); }
 }
@@ -82,7 +84,10 @@ static const char* kHelp =
     "  no filter is applied; --tfam is optional:\n"
     "  its IDs must equal the VCF samples in order and it names the population, which is VCF without it; not with\n"
     "  --host-tokenize),\n"
-    "  --gpus <n> (shard individuals over n GPUs), --exact (whole-segment chains), --device <n>, --seed <n> (subsample RNG seed), --device-lut, --kde-direct, --kde-gpu (the KDE itself on the GPU: exact Gauss transform of the thinned windows still in HBM), --host-tokenize (tped allele columns extracted on the host instead of the GPU tokeniser)\n";
+    "  --gpus <n> (shard individuals over n GPUs), --exact (whole-segment chains), --device <n>, --seed <n> (subsample RNG seed), --device-lut, --kde-direct, --kde-gpu (the KDE itself on the GPU: exact Gauss transform of the thinned windows still in HBM), --host-tokenize (tped allele columns extracted on the host instead of the GPU tokeniser)\n"
+    "  --by-pop (a tfam or .fam with several population IDs, the first column: each population, in order of first\n"
+    "  appearance, is analysed as a separate run with the same flags would analyse it, its outputs under <out>.<pop>;\n"
+    "  <out>.log lists the populations; with --gpus n each population is sharded over min(n, its size) GPUs)\n";
 
 int parse_cli(int argc, char** argv, Options& o, std::string& cmdline)
 {
@@ -90,7 +95,8 @@ int parse_cli(int argc, char** argv, Options& o, std::string& cmdline)
     for (int i = 0; i < argc; ++i) { cmdline += argv[i]; cmdline += " "; }
     std::map<std::string, bool*> fb = {{"--weighted", &o.weighted}, {"--cm", &o.cm}, {"--auto-winsize", &o.auto_winsize},
         {"--auto-overlap-frac", &o.auto_overlap}, {"--raw-lod", &o.raw_lod}, {"--freq-only", &o.freq_only},
-        {"--phased", &o.phased}, {"--no-kde-thinning", &o.no_kde_thinning}, {"--exact", &o.exact}, {"--device-lut", &o.device_lut}, {"--kde-direct", &o.kde_direct}, {"--kde-gpu", &o.kde_gpu}, {"--host-tokenize", &o.host_tokenize}};
+        {"--phased", &o.phased}, {"--no-kde-thinning", &o.no_kde_thinning}, {"--exact", &o.exact}, {"--device-lut", &o.device_lut}, {"--kde-direct", &o.kde_direct}, {"--kde-gpu", &o.kde_gpu}, {"--host-tokenize", &o.host_tokenize},
+        {"--by-pop", &o.by_pop}};
     std::map<std::string, int*> fi = {{"--winsize", &o.winsize}, {"--auto-winsize-step", &o.auto_winsize_step},
         {"--max-gap", &o.max_gap}, {"--resample", &o.resample}, {"--threads", &o.threads}, {"--M", &o.M},
         {"--nclust", &o.nclust}, {"--kde-subsample", &o.kde_subsample}, {"--ld-subsample", &o.ld_subsample},

@@ -19,6 +19,9 @@ extern const char* const kVersion;   // "1.1.6a": printed in the BED track lines
 struct Log {
     FILE* log = nullptr;
     FILE* err = nullptr;
+    bool hold = false;                       // line() appends to `held` instead (--by-pop: replayed per population)
+    std::vector<std::string> held;
+    std::string last;                        // the last error() line
     bool open(const std::string& base);
     void close();
     void line(const std::string& s);        // to .log
@@ -49,6 +52,7 @@ struct Options {
     bool host_tokenize = false;  // extension: extract the tped allele characters on the host instead of K0 (--host-tokenize)
     bool kde_direct = false;     // extension: exact (reproducible) Gauss transform for the KDE (--kde-direct)
     bool kde_gpu = false;        // extension: computeKDE on the GPU, from the thinned windows still in HBM (--kde-gpu)
+    bool by_pop = false;         // extension: analyse each population of the tfam in turn, outputs under <out>.<pop> (--by-pop)
     long seed = -1;              // extension: RNG seed for the KDE / LD subsamples (--seed; default time)
 };
 // returns 0 = run, 1 = help printed (exit 0), -1 = error
@@ -68,8 +72,9 @@ struct Tped {
 };
 // host_tokenize: extract the allele characters here (the pre-K0 path, kept for A/B timing) instead of keeping raw text
 bool load_tped(const std::string& path, char missing, Tped& t, bool host_tokenize = false);
-struct Tfam { std::string pop; std::vector<std::string> ids; };
-bool load_tfam(const std::string& path, Tfam& f);
+struct Tfam { std::string pop; std::vector<std::string> ids, pops; };
+// multi: several population IDs are allowed (pops[i] = individual i's); otherwise they are refused
+bool load_tfam(const std::string& path, Tfam& f, bool multi = false);
 // PLINK .bim: chr / id / cM / bp fill the tped's first four columns (same chromosome log lines as load_tped); a1 / a2 =
 // the allele names of columns 5 and 6
 bool load_bim(const std::string& path, Tped& t, std::vector<std::string>& a1, std::vector<std::string>& a2);

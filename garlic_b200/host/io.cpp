@@ -692,7 +692,7 @@ bool load_vcf(const std::string& path, Tped& t, Vcf& v)
 }
 
 // scanIndData3 / readIndData3 (garlic-data.cpp:1893-2014): single population, unique IDs.
-bool load_tfam(const std::string& path, Tfam& f)
+bool load_tfam(const std::string& path, Tfam& f, bool multi)
 {
     GzLines in;
     if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
@@ -713,8 +713,9 @@ bool load_tfam(const std::string& path, Tfam& f)
         if (seen.count(id)) { LOG.error("ERROR: Found duplicate individual ID (  " + id + " ) in " + path); return false; }
         seen[id] = 1;
         if (n == 1) f.pop = pop;
-        else if (pop != f.pop) { LOG.error("ERROR: Found multiple population IDs (  " + pop + ", " + f.pop + " ) in " + path); return false; }
+        else if (pop != f.pop && !multi) { LOG.error("ERROR: Found multiple population IDs (  " + pop + ", " + f.pop + " ) in " + path); return false; }
         f.ids.push_back(id);
+        f.pops.push_back(pop);
     }
     if (n < 1) { LOG.error("ERROR: Number of individuals must be positive: 0"); return false; }
     return true;

@@ -45,9 +45,8 @@ struct Team {
     int pending = 0;
     bool quit = false, failed = false;
 
-    void follower(int r)
+    void follower(int r, long seen)
     {
-        long seen = 0;
         for (;;) {
             std::function<bool(Rank&)> j;
             {
@@ -82,8 +81,9 @@ struct Team {
     }
     void start(int G)
     {
-        ranks.resize(G);
-        for (int r = 1; r < G; ++r) threads.emplace_back(&Team::follower, this, r);
+        ranks.assign(G, Rank());
+        quit = failed = false;
+        for (int r = 1; r < G; ++r) threads.emplace_back(&Team::follower, this, r, generation);
     }
     void stop()
     {
@@ -252,7 +252,7 @@ double calc_density(const Ctx& c)   // calcDensity, garlic-data.cpp:318-328
 // streamed in blocks so that the window matrix never exists as a whole
 bool write_raw_lod(Ctx& c, int W)
 {
-    const int C = (int)c.labels.size(), N = c.tped.n_ind;
+    const int C = (int)c.labels.size(), N = (int)c.tfam.ids.size();
     std::vector<gzFile> f(C);
     for (int ch = 0; ch < C; ++ch) {
         const std::string fn = c.o.out + "." + c.tfam.pop + "." + c.labels[ch] + ".raw.lod.windows.gz";
@@ -309,6 +309,7 @@ int main(int argc, char** argv)
     if (pr < 0) return -1;
     if (!LOG.open(o.out)) return -1;
     LOG.line(cmdline);
+    LOG.hold = o.by_pop;                       // --by-pop: <out>.log lists the populations; these lines go to theirs
     LOG.line("Output file basename: " + o.out);
 
     // ---- validation and parameter log, in the reference's order (garlic-main.cpp:39-183) ----
@@ -428,9 +429,9 @@ int main(int argc, char** argv)
     LOG.line("Total loci: " + std::to_string(t.n_loci));
     if (vcf) {
         // the samples are the individuals; a --tfam must list the same IDs in the same order and names the population
-        if (o.tfam == "none") { c.tfam.pop = "VCF"; c.tfam.ids = vc.samples; }
+        if (o.tfam == "none") { c.tfam.pop = "VCF"; c.tfam.ids = vc.samples; c.tfam.pops.assign(vc.samples.size(), "VCF"); }
         else {
-            if (!load_tfam(o.tfam, c.tfam)) return 1;
+            if (!load_tfam(o.tfam, c.tfam, o.by_pop)) return 1;
             for (size_t i = 0; i < std::max(c.tfam.ids.size(), vc.samples.size()); ++i)
                 if (i >= c.tfam.ids.size() || i >= vc.samples.size() || c.tfam.ids[i] != vc.samples[i]) {
                     LOG.error("ERROR: " + o.tfam + " and " + o.vcf + " differ at individual " + std::to_string(i + 1) + ": " +
@@ -439,16 +440,57 @@ int main(int argc, char** argv)
                     return 1;
                 }
         }
-    } else if (!load_tfam(bed ? o.bfile + ".fam" : o.tfam, c.tfam)) return 1;
+    } else if (!load_tfam(bed ? o.bfile + ".fam" : o.tfam, c.tfam, o.by_pop)) return 1;
     if (bed) t.n_ind = (int)c.tfam.ids.size();
     else if ((int)c.tfam.ids.size() != t.n_ind) { LOG.error("ERROR: tfam and tped disagree on the number of individuals."); return 1; }
     FILE* bed_in = nullptr;
+    if (bed) {                                          // the size check, once for the whole file
+        if (!open_bed(o.bfile + ".bed", t.n_ind, t.n_loci, bed_in)) return 1;
+        fclose(bed_in);
+    }
+    std::vector<double> gl;
+    const bool oob = o.weighted || o.cm;
+
+    // ---- populations: in order of first appearance, each the individuals (input columns) carrying its ID ----
+    std::vector<std::string> pop_ids;
+    std::vector<std::vector<int32_t>> pop_cols;
+    if (!o.by_pop) { pop_ids.push_back(c.tfam.pop); pop_cols.emplace_back(); }
+    else
+        for (int i = 0; i < t.n_ind; ++i) {
+            const std::string& p = c.tfam.pops[i];
+            const size_t k = std::find(pop_ids.begin(), pop_ids.end(), p) - pop_ids.begin();
+            if (k == pop_ids.size()) {
+                if (p == "." || p == ".." || p.find('/') != std::string::npos) {
+                    LOG.error("ERROR: Population ID " + p + " cannot be part of a file name (--by-pop writes <out>." + p + ".*).");
+                    return 1;
+                }
+                pop_ids.push_back(p);
+                pop_cols.emplace_back();
+            }
+            pop_cols[k].push_back(i);
+        }
+    const Tfam all = c.tfam;
+    const std::string out_base = o.out;
+    const int winsize0 = winsize;
+    const double cutoff0 = cutoff;
+    const std::vector<double> bounds0 = bounds;
+
+    // one population (without --by-pop: the whole input, cols empty): what a separate run does from here on
+    auto run_population = [&](const std::string& pop, const std::vector<int32_t>& cols, bool last_pop) -> int {
+    const bool sel = !cols.empty();
+    const int N = sel ? (int)cols.size() : t.n_ind;
+    int winsize = winsize0;
+    double cutoff = cutoff0;
+    std::vector<double> bounds = bounds0;
+    c.rng.seed(o.seed >= 0 ? (o.seed == 0 ? 4357u : (unsigned)o.seed) : (unsigned)time(nullptr));
+    c.tfam.pop = pop;
+    if (sel) { c.tfam.ids.clear(); for (int i : cols) c.tfam.ids.push_back(all.ids[i]); }
+    c.labels.clear(); c.cen_arr.clear(); c.scaffold.clear();
     if (bed && !open_bed(o.bfile + ".bed", t.n_ind, t.n_loci, bed_in)) return 1;
     LOG.line("Population: " + c.tfam.pop);
-    LOG.line("Total diploid individuals: " + std::to_string(t.n_ind));
-    std::vector<double> gl;
-    if (use_gl && o.host_tokenize && !load_tgls(o.tgls, t, gl)) return 1;   // (K0-GL streams the file to the GPUs below)
-    const bool oob = o.weighted || o.cm;
+    LOG.line("Total diploid individuals: " + std::to_string(N));
+    // (K0-GL streams the file to the GPUs below; --host-tokenize reads it once, for every population)
+    if (use_gl && o.host_tokenize && gl.empty() && !load_tgls(o.tgls, t, gl)) return 1;
     if (oob) {
         if (!load_map(o.map, c.scaffold)) return 1;
         if (c.scaffold.size() != t.chr_names.size()) {
@@ -470,14 +512,14 @@ int main(int argc, char** argv)
     }
 
     // ---- GPU: coding, counts, freq, filter (K1-K3), individuals sharded over --gpus ranks ----
-    const int G = o.gpus;
-    if (G < 1 || G > t.n_ind) { LOG.error("ERROR: --gpus must be between 1 and the number of individuals."); return -1; }
+    const int G = o.by_pop ? std::min(o.gpus, N) : o.gpus;
+    if (G < 1 || G > N) { LOG.error("ERROR: --gpus must be between 1 and the number of individuals."); return -1; }
     Team& team = c.team;
     team.start(G);
     uint8_t comm_id[128];
     if (G > 1 && garlic_gpu_comm_id(comm_id)) { LOG.error("ERROR: ncclGetUniqueId failed."); return 1; }
-    const int per = (t.n_ind + G - 1) / G;
-    for (int r = 0; r < G; ++r) { team.ranks[r].rank = r; team.ranks[r].lo = std::min(t.n_ind, r * per); team.ranks[r].hi = std::min(t.n_ind, (r + 1) * per); }
+    const int per = (N + G - 1) / G;
+    for (int r = 0; r < G; ++r) { team.ranks[r].rank = r; team.ranks[r].lo = std::min(N, r * per); team.ranks[r].hi = std::min(N, (r + 1) * per); }
     auto fail = [&](int code) { LOG.error("ERROR: " + team.first_error()); team.stop(); return code; };
     const int64_t blk = 1 << 12;                       // tped lines per upload (multiple of 32)
     const bool bcf = !vc.gt_type.empty();
@@ -506,6 +548,8 @@ int main(int argc, char** argv)
             if (G > 1 && !rank_ok(R, garlic_gpu_comm_init(R.g, comm_id, R.rank, G), "comm_init")) return false;
             const int n = R.hi - R.lo;
             if (!rank_ok(R, garlic_gpu_set_shape(R.g, n, R.lo, t.n_loci, C, t.chr_off.data(), t.pos.data()), "set_shape")) return false;
+            // --by-pop: every rank parses every input column and keeps its own individuals of the population
+            if (sel && !rank_ok(R, garlic_gpu_select_columns(R.g, cols.data() + R.lo, t.n_ind), "select_columns")) return false;
             std::vector<uint8_t> slice;
             std::vector<int32_t> nb;
             std::vector<int32_t> nc, mx, bc;
@@ -541,7 +585,13 @@ int main(int argc, char** argv)
             for (int64_t s0 = 0; s0 < t.n_loci && !bed && o.host_tokenize; s0 += blk) {
                 const int ns = (int)std::min(blk, t.n_loci - s0);
                 const uint8_t* src_ = t.alleles.data() + (size_t)s0 * t.n_ind * 2;
-                if (G > 1) {                                   // this rank's columns of the block
+                if (sel) {                                     // this rank's columns of the population
+                    slice.resize((size_t)ns * n * 2);
+                    for (int k = 0; k < ns; ++k)
+                        for (int i = 0; i < n; ++i)
+                            memcpy(slice.data() + ((size_t)k * n + i) * 2, src_ + ((size_t)k * t.n_ind + cols[R.lo + i]) * 2, 2);
+                    src_ = slice.data();
+                } else if (G > 1) {                            // this rank's columns of the block
                     slice.resize((size_t)ns * n * 2);
                     for (int k = 0; k < ns; ++k) memcpy(slice.data() + (size_t)k * n * 2, src_ + ((size_t)k * t.n_ind + R.lo) * 2, (size_t)n * 2);
                     src_ = slice.data();
@@ -551,7 +601,10 @@ int main(int argc, char** argv)
             if (!bed && !rank_ok(R, garlic_gpu_code_alleles(R.g), "code_alleles")) return false;     // MIN all-reduce of the first-allele keys
             if (use_gl && o.host_tokenize) {
                 const int type = o.gl_type == "GQ" ? GARLIC_GL_GQ : o.gl_type == "GL" ? GARLIC_GL_GL : GARLIC_GL_PL;
-                if (!rank_ok(R, garlic_gpu_put_gl(R.g, gl.data() + (size_t)R.lo * t.n_loci, type), "put_gl")) return false;
+                std::vector<double> rows;
+                if (sel)
+                    for (int i = R.lo; i < R.hi; ++i) rows.insert(rows.end(), gl.begin() + (size_t)cols[i] * t.n_loci, gl.begin() + (size_t)(cols[i] + 1) * t.n_loci);
+                if (!rank_ok(R, garlic_gpu_put_gl(R.g, sel ? rows.data() : gl.data() + (size_t)R.lo * t.n_loci, type), "put_gl")) return false;
             }
             return true;
         })) return fail(1);
@@ -607,9 +660,11 @@ int main(int argc, char** argv)
         }
     }
     c.g = team.ranks[0].g;
-    std::vector<uint8_t>().swap(t.alleles);
-    std::vector<char>().swap(t.text);
-    std::vector<double>().swap(gl);
+    if (last_pop) {                                    // the parsed input stays on the host until the last population
+        std::vector<uint8_t>().swap(t.alleles);
+        std::vector<char>().swap(t.text);
+        std::vector<double>().swap(gl);
+    }
     std::vector<int32_t> chr_param;
     if (oob)
         for (int ch = 0; ch < C; ++ch) {
@@ -704,8 +759,8 @@ int main(int argc, char** argv)
     if (explore || (o.auto_winsize && !o.weighted)) {
         std::vector<int32_t> sub;
         const std::vector<int32_t>* subp = nullptr;
-        if (o.kde_subsample > 0 && o.kde_subsample < t.n_ind) {   // subsetData, garlic-data.cpp:2171-2244
-            sub = choose(c, o.kde_subsample, t.n_ind);
+        if (o.kde_subsample > 0 && o.kde_subsample < N) {   // subsetData, garlic-data.cpp:2171-2244
+            sub = choose(c, o.kde_subsample, N);
             std::string s = "Individuals used for KDE: ";
             for (int i : sub) s += c.tfam.ids[i] + " ";
             LOG.line(s);
@@ -714,7 +769,7 @@ int main(int argc, char** argv)
         auto kde_for = [&](int W, Kde& k) -> bool {
             if (o.weighted) {
                 std::vector<int32_t> ld;
-                if (o.ld_subsample > 0 && o.ld_subsample < t.n_ind) ld = choose(c, o.ld_subsample, t.n_ind);
+                if (o.ld_subsample > 0 && o.ld_subsample < N) ld = choose(c, o.ld_subsample, N);
                 if (!ld_band_all(c, W, ld)) return false;
             }
             std::vector<double> data;
@@ -773,7 +828,7 @@ int main(int argc, char** argv)
     if (o.weighted) {
         fprintf(stderr, "Calculating LD matrix.\n");
         std::vector<int32_t> ld;
-        if (o.ld_subsample > 0 && o.ld_subsample < t.n_ind) ld = choose(c, o.ld_subsample, t.n_ind);
+        if (o.ld_subsample > 0 && o.ld_subsample < N) ld = choose(c, o.ld_subsample, N);
         if (!ld_band_all(c, winsize, ld)) return 1;
     }
 
@@ -786,8 +841,8 @@ int main(int argc, char** argv)
             std::vector<int32_t> sub;
             const std::vector<int32_t>* subp = nullptr;
             if (o.kde_subsample > 0) {
-                if (o.kde_subsample < t.n_ind) sub = choose(c, o.kde_subsample, t.n_ind);
-                else { sub.resize(t.n_ind); for (int i = 0; i < t.n_ind; ++i) sub[i] = i; }
+                if (o.kde_subsample < N) sub = choose(c, o.kde_subsample, N);
+                else { sub.resize(N); for (int i = 0; i < N; ++i) sub[i] = i; }
                 std::string s = "Individuals used for KDE: ";
                 for (int i : sub) s += c.tfam.ids[i] + " ";
                 LOG.line(s);
@@ -840,5 +895,32 @@ int main(int argc, char** argv)
     if (!write_bed(o.out + ".roh.bed", roh, c.tfam.ids, c.labels, bounds, c.tfam.pop, o.cm)) return 1;
     printf("Finished.\n");
     LOG.close();
+    return 0;
+    };
+
+    if (!o.by_pop) return run_population(c.tfam.pop, {}, true);
+    // --by-pop: the parameter and input lines a separate run writes before "Population:" go to each population's log
+    LOG.hold = false;
+    const std::vector<std::string> held = LOG.held;
+    Log top = LOG;
+    for (size_t k = 0; k < pop_ids.size(); ++k) {
+        const std::string prefix = out_base + "." + pop_ids[k];
+        top.line("Population " + pop_ids[k] + ": " + std::to_string(pop_cols[k].size()) + " individuals, output prefix " + prefix);
+        LOG = Log();
+        if (!LOG.open(prefix)) { top.close(); return -1; }
+        LOG.line(cmdline);
+        LOG.line("Output file basename: " + prefix);
+        for (size_t i = 1; i < held.size(); ++i) LOG.line(held[i]);
+        o.out = prefix;
+        const int rc = run_population(pop_ids[k], pop_cols[k], k + 1 == pop_ids.size());
+        const std::string msg = LOG.last;
+        LOG.close();
+        if (rc) {
+            top.error("ERROR: population " + pop_ids[k] + ": " + (msg.empty() ? std::string("failed") : msg));
+            top.close();
+            return rc;
+        }
+    }
+    top.close();
     return 0;
 }

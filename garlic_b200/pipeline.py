@@ -75,13 +75,20 @@ class HotPath:
         self.g.close()
 
     def load(self, ds, weighted=False, cm=False, error=None, max_gap=200000, packed_rows=None,
-             nalleles_corr=None, total_corr=None, mu=1e-9, M=7, bed=None, vcf=None, bcf=None):
+             nalleles_corr=None, total_corr=None, mu=1e-9, M=7, bed=None, vcf=None, bcf=None, columns=None, n_input=None):
         """bed: uint8[L0, ceil(N/4)] SNP-major .bed rows (plink.Fileset.rows) in place of ds.alleles.
         vcf: (text, offsets) of the VCF sample columns (vcf.sample_text) in place of ds.alleles.
-        bcf: (payload, offsets, descriptors) of the BCF GT vectors (bcf.gt_payload) in place of ds.alleles."""
+        bcf: (payload, offsets, descriptors) of the BCF GT vectors (bcf.gt_payload) in place of ds.alleles.
+        columns: the individuals of a bed / vcf / bcf input of n_input individuals that form the analysed sample
+        (ascending; GarlicGPU.select_columns); ds.gl, if any, holds the sample's individuals only."""
         g = self.g
         N = ds.n_ind if packed_rows is None else packed_rows.shape[0]
+        if columns is not None:
+            N = len(columns)
         g.set_shape(N, len(ds.pos), ds.chr_offsets, ds.pos)
+        if columns is not None:
+            g.select_columns(columns, n_input)
+        n_samples = N if n_input is None else n_input
         if bed is not None:
             for s0 in range(0, len(ds.pos), 4096):
                 g.put_bed(bed[s0:s0 + 4096], s0)
@@ -91,13 +98,13 @@ class HotPath:
             for s0 in range(0, len(ds.pos), 4096):
                 o = off[s0:s0 + 4097]
                 nc, mx, bad = g.put_vcf_text(text, o, s0)
-                if (nc != N).any() or (bad >= 0).any():
+                if (nc != n_samples).any() or (bad >= 0).any():
                     raise ValueError("malformed VCF records in block %d" % s0)
             g.code_alleles()
         elif bcf is not None:
             gt, off, types = bcf
             for s0 in range(0, len(ds.pos), 4096):
-                _, bad = g.put_bcf_gt(gt, off[s0:s0 + 4097], types[s0:s0 + 4096], N, s0)
+                _, bad = g.put_bcf_gt(gt, off[s0:s0 + 4097], types[s0:s0 + 4096], n_samples, s0)
                 if (bad >= 0).any():
                     raise ValueError("malformed BCF records in block %d" % s0)
             g.code_alleles()

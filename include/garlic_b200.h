@@ -68,6 +68,16 @@ int garlic_gpu_comm_init(garlic_gpu_t *h, const uint8_t *id128, int rank, int wo
  * filtering; chr_offsets[n_chr+1] into the SNP axis; pos[n_loci] physical positions. */
 int garlic_gpu_set_shape(garlic_gpu_t *h, int n_ind, int ind_offset, int64_t n_loci, int n_chr,
                          const int64_t *chr_offsets, const int32_t *pos);
+/* Column selection: columns[n_ind] lists the input columns (individuals of the input, counted from 0) that this handle
+ * holds, strictly ascending, each below n_input, the number of individuals the input holds.  put_tped_text,
+ * put_vcf_text, put_bcf_gt, put_tgls_text and put_bed / put_bed_dev then store the listed columns (individual i of
+ * the handle = input column columns[i]) instead of [ind_offset, ind_offset+n_ind); every column is still parsed, so
+ * the per-line diagnostics are those of the whole input.  ind_offset keeps its meaning: the handle's first individual
+ * within the analysed sample (the first-allele keys and the LD individual lists address that sample), so a sample of
+ * several handles lists disjoint columns.  put_alleles, put_gl, put_packed and their _dev forms receive only this
+ * handle's individuals and ignore the selection.  Call after set_shape (which resets the selection) and before the
+ * first put_*.  Fails on an unsorted or out-of-range list and after a put_*. */
+int garlic_gpu_select_columns(garlic_gpu_t *h, const int32_t *columns, int n_input);
 /* alleles: [n_snp][n_ind][2] characters for SNPs [snp0, snp0+n_snp), snp0 % 32 == 0.
  * Uploads them and records, per SNP, the first non-missing allele in file order (phase a). */
 int garlic_gpu_put_alleles(garlic_gpu_t *h, const uint8_t *alleles, int64_t snp0, int n_snp, char missing);
@@ -88,7 +98,8 @@ int garlic_gpu_put_tped_text(garlic_gpu_t *h, const char *text, const int64_t *l
  * counters (phase a).  The calls are coded as the tped that writes hom A1 "A1 A1", het "A1 A2", hom A2 "A2 A2" and
  * missing "0 0" would be: the "1" allele is A2 iff the first present call over all individuals is hom A2.
  * garlic_gpu_code_alleles then runs the transpose (phase b) and frees the staging rows.  --phased is refused on such
- * a handle (a .bed stores no phase).  _dev: rows on this GPU, complete before the call. */
+ * a handle (a .bed stores no phase).  _dev: rows on this GPU, complete before the call.  With a column selection the
+ * stride must cover ceil(n_input/4) bytes; the rows are copied whole and a kernel gathers the listed columns. */
 int garlic_gpu_put_bed(garlic_gpu_t *h, const uint8_t *rows, int64_t snp_stride_bytes, int64_t snp0, int n_snp);
 int garlic_gpu_put_bed_dev(garlic_gpu_t *h, const void *rows_dev, int64_t snp_stride_bytes, int64_t snp0, int n_snp);
 /* VCF genotypes: text = per record the characters after the FORMAT column's tab (the sample columns, separated by
