@@ -29,6 +29,8 @@ EXPORTS = [
     "garlic_gpu_call_roh", "garlic_gpu_last_stats", "garlic_gpu_n_kept", "garlic_gpu_get_kept_index",
     "garlic_gpu_get_genotypes", "garlic_gpu_get_piece_bounds", "garlic_gpu_set_prune", "garlic_gpu_kde", "garlic_gpu_put_tgls_text", "garlic_gpu_get_gl",
     "garlic_gpu_put_bed", "garlic_gpu_put_bed_dev", "garlic_gpu_put_vcf_text", "garlic_gpu_put_bcf_gt", "garlic_gpu_select_columns",
+    "garlic_gpu_set_call_filter", "garlic_gpu_put_vcf_text_filtered", "garlic_gpu_put_bcf_gt_filtered",
+    "garlic_gpu_calls_set_missing",
 ]
 
 
@@ -58,6 +60,7 @@ def load_library():
     L.garlic_gpu_counts_dev.restype = C.c_void_p
     L.garlic_gpu_window_slots.restype = C.c_int64
     L.garlic_gpu_n_kept.restype = C.c_int64
+    L.garlic_gpu_calls_set_missing.restype = C.c_uint64
     for name in EXPORTS:
         getattr(L, name)
     _LIB = L
@@ -174,6 +177,48 @@ class GarlicGPU:
         self._ck(self.lib.garlic_gpu_put_bcf_gt(self.h, _p(buf), _p(off), _p(types), C.c_int(n_samples), C.c_int64(snp0),
                                                 C.c_int(n), _p(mx), _p(bad)))
         return mx, bad
+
+    def set_call_filter(self, min_gq=0, min_dp=0):
+        """--vcf-min-gq / --vcf-min-dp (0 = off): put_vcf_text_filtered / put_bcf_gt_filtered then store a call whose GQ or
+        DP is below its threshold as two missing alleles.  Call after set_shape (and select_columns), before any put_*."""
+        self._ck(self.lib.garlic_gpu_set_call_filter(self.h, C.c_int(min_gq), C.c_int(min_dp)))
+
+    def calls_set_missing(self):
+        """Calls of this handle with a present allele that the call filter set missing."""
+        return int(self.lib.garlic_gpu_calls_set_missing(self.h))
+
+    def put_vcf_text_filtered(self, text: bytes, line_off, fmt_index, snp0=0):
+        """put_vcf_text with the call filter; fmt_index int32[n, 2] = the FORMAT index of GQ and DP per record (-1 if
+        absent, vcf.format_index).  Returns (n_cols, max_allele, bad_col, bad_value) per record."""
+        off = np.ascontiguousarray(line_off, np.int64)
+        n = len(off) - 1
+        fk = np.ascontiguousarray(fmt_index, np.int32).reshape(n, 2)
+        nc, mx, bad, badv = (np.empty(n, np.int32) for _ in range(4))
+        buf = np.frombuffer(text, np.uint8) if len(text) else np.zeros(1, np.uint8)
+        self._ck(self.lib.garlic_gpu_put_vcf_text_filtered(self.h, _p(buf), _p(off), C.c_int64(snp0), C.c_int(n), _p(fk),
+                                                           _p(nc), _p(mx), _p(bad), _p(badv)))
+        return nc, mx, bad, badv
+
+    def put_bcf_gt_filtered(self, gt, rec_off, gt_type, n_samples, fv, fv_off, fv_pos, fv_type, snp0=0):
+        """put_bcf_gt with the call filter; (fv, fv_off[n+1], fv_pos int32[n, 2], fv_type uint8[n, 2]) as
+        bcf.call_values returns them.  Returns (max_allele, bad_sample, bad_value) per record."""
+        off = np.ascontiguousarray(rec_off, np.int64)
+        n = len(off) - 1
+        types = np.ascontiguousarray(gt_type, np.uint8)
+        mx, bad, badv = (np.empty(n, np.int32) for _ in range(3))
+        buf = np.frombuffer(gt, np.uint8) if isinstance(gt, (bytes, bytearray)) else np.ascontiguousarray(gt, np.uint8)
+        if not buf.size:
+            buf = np.zeros(1, np.uint8)
+        fbuf = np.frombuffer(fv, np.uint8) if isinstance(fv, (bytes, bytearray)) else np.ascontiguousarray(fv, np.uint8)
+        if not fbuf.size:
+            fbuf = None                                            # no GQ / DP vector in the block: the library takes NULL
+        foff = np.ascontiguousarray(fv_off, np.int64)
+        fpos = np.ascontiguousarray(fv_pos, np.int32).reshape(n, 2)
+        ftype = np.ascontiguousarray(fv_type, np.uint8).reshape(n, 2)
+        self._ck(self.lib.garlic_gpu_put_bcf_gt_filtered(self.h, _p(buf), _p(off), _p(types), C.c_int(n_samples),
+                                                         C.c_int64(snp0), C.c_int(n), _p(fbuf), _p(foff), _p(fpos), _p(ftype),
+                                                         _p(mx), _p(bad), _p(badv)))
+        return mx, bad, badv
 
     def put_bed(self, rows, snp0=0):
         """rows: uint8[n_snp, ceil(N_total/4)] SNP-major .bed rows of the whole fileset (no magic bytes); this handle keeps

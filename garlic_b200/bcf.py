@@ -7,6 +7,9 @@ bytes, each (allele + 1) << 1 | phased, 0 or 1 for a missing allele, end-of-vect
 `02 04`, `0|1` is `02 05`, `./.` is `00 00` and a lone `.` is `00 81`; a record whose every sample is a lone `.` has
 count 1 and value `00`.  csrc/bcf.cu decodes the GT vectors on the GPU by the rule of decode_gt
 (csrc/bcf_gt.cuh:decode_gt).
+
+GQ and DP (the call filter, --vcf-min-gq / --vcf-min-dp) are count-1 vectors of int8, int16, int32 or float; value_rule
+restates csrc/bcf_gt.cuh:bcf_value, and call_values returns the vectors as the driver's loader copies them out.
 """
 from __future__ import annotations
 
@@ -22,6 +25,8 @@ INT8, INT16, INT32, FLOAT, CHAR = 1, 2, 3, 5, 7
 WIDTH = {INT8: 1, INT16: 2, INT32: 4, FLOAT: 4, CHAR: 1}
 TYPE_OF_WIDTH = {1: INT8, 2: INT16, 4: INT32}
 EOV = {1: -127, 2: -32767, 4: -2147483647}          # end-of-vector, sign-extended
+INT_MISSING = {1: -128, 2: -32768, 4: -2147483648}   # missing value, sign-extended
+FLOAT_MISSING, FLOAT_EOV = 0x7F800001, 0x7F800002     # the float sentinels' bits
 _DT = {INT8: "<i1", INT16: "<i2", INT32: "<i4", FLOAT: "<f4", CHAR: "u1"}
 _QUAL_MISSING = struct.pack("<I", 0x7F800001)
 _FORMAT_LINES = {"GT": 'Number=1,Type=String,Description="Genotype"',
@@ -42,6 +47,48 @@ def decode_gt(v0, v1, count, width):
     if v1 < 0 or (v1 >> 1) - 1 > vcf.MAX_ALLELE:
         return None
     return ((v0 >> 1) - 1 if v0 > 1 else M, (v1 >> 1) - 1 if v1 > 1 else M)
+
+
+def value_rule(raw, typ, thr):
+    """The rule of csrc/bcf_gt.cuh:bcf_value: raw = an int8/16/32 value sign-extended, or a float's bits (as uint32 or
+    int32) → 1 passes (>= thr, or a missing / end-of-vector sentinel), 0 is below thr, -1 is malformed (a float NaN that
+    is not a sentinel, or an infinity)."""
+    if typ == FLOAT:
+        bits = int(raw) & 0xFFFFFFFF
+        if bits in (FLOAT_MISSING, FLOAT_EOV):
+            return 1
+        f = float(np.array([bits], np.uint32).view(np.float32)[0])
+        if not np.isfinite(f):
+            return -1
+        return int(f >= thr)
+    w = WIDTH[typ]
+    if raw in (INT_MISSING[w], EOV[w]):
+        return 1
+    return int(raw >= thr)
+
+
+def value_array(values, typ):
+    """float64 values (NaN = missing) → the vector of type typ (missing → the type's missing value)."""
+    values = np.asarray(values, float)
+    if typ == FLOAT:
+        out = values.astype(np.float32).view(np.uint32).copy()
+        out[np.isnan(values)] = FLOAT_MISSING
+        return out.view("<f4")
+    w = WIDTH[typ]
+    return np.where(np.isnan(values), INT_MISSING[w], np.nan_to_num(values)).astype(_DT[typ])
+
+
+def values_float(arr, typ):
+    """A GQ / DP vector as read → float64, NaN for the sentinels."""
+    if typ == FLOAT:
+        bits = np.asarray(arr).view(np.uint32)
+        with np.errstate(invalid="ignore"):                  # the sentinels are signalling NaNs
+            out = np.asarray(arr, np.float32).astype(float)
+        out[(bits == FLOAT_MISSING) | (bits == FLOAT_EOV)] = np.nan
+        return out
+    a = np.asarray(arr).astype(np.int64)
+    w = WIDTH[typ]
+    return np.where((a == INT_MISSING[w]) | (a == EOV[w]), np.nan, a.astype(float))
 
 
 # ------------------------------------------------------------------------------------------------ typed values
@@ -148,13 +195,16 @@ def _gt_field(idx_s, lone_missing, width):
     return 2, np.stack([va, vb], 1)
 
 
-def bcf_bytes(v: vcf.Vcf, fmt="GT", lone_missing=False, width=None, idx=True) -> bytes:
+def bcf_bytes(v: vcf.Vcf, fmt="GT", lone_missing=False, width=None, idx=True, call_type=None) -> bytes:
     """The uncompressed BCF of v: fmt "GT" or "GT:AD:DP:GQ:PL" (the filler values of vcf.vcf_text), lone_missing writes
     a call with both alleles missing as a lone '.', width the GT value width (1, 2 or 4; None: gt_width), idx writes
-    IDX= on every dictionary line (else the dictionaries are in order of appearance)."""
-    if fmt not in vcf.FORMATS:
-        raise ValueError("fmt must be one of %s" % (vcf.FORMATS,))
+    IDX= on every dictionary line (else the dictionaries are in order of appearance).  With v.gq / v.dp, fmt may be any
+    ':'-list of GT (first), AD, DP, GQ and PL, and DP / GQ hold their values (NaN: missing) as call_type (INT8, INT16,
+    INT32 or FLOAT; None: the narrowest integer type)."""
     keys = fmt.split(":")
+    custom = v.gq is not None or v.dp is not None
+    if fmt not in vcf.FORMATS and not (custom and keys[0] == "GT" and set(keys) <= set(vcf.FORMAT_KEYS)):
+        raise ValueError("fmt must be one of %s" % (vcf.FORMATS,))
     contigs = list(dict.fromkeys(v.chrom))
     cidx = {c: i for i, c in enumerate(contigs)}
     idx_arr = np.asarray(v.idx, np.uint8)
@@ -172,9 +222,15 @@ def bcf_bytes(v: vcf.Vcf, fmt="GT", lone_missing=False, width=None, idx=True) ->
         shared += typed_ints([0])                                  # FILTER: PASS
         indiv = []
         for k, key in enumerate(keys):
+            val = v.gq if key == "GQ" else v.dp if key == "DP" else None
             if key == "GT":
                 count, vals = _gt_field(idx_arr[s], lone_missing, width)
                 body = typed_desc(count, TYPE_OF_WIDTH[width]) + vals.astype(_DT[TYPE_OF_WIDTH[width]]).tobytes()
+            elif val is not None:
+                row = np.asarray(val[s], float)
+                present = row[~np.isnan(row)]
+                t = call_type or (int_type(int(present.min()), int(present.max())) if present.size else INT8)
+                body = typed_desc(1, t) + value_array(row, t).tobytes()
             else:
                 per = {"AD": [3] * n_allele, "DP": [3 * n_allele], "GQ": [30],
                        "PL": [0] + [20] * (n_allele * (n_allele + 1) // 2 - 1)}[key]
@@ -186,9 +242,10 @@ def bcf_bytes(v: vcf.Vcf, fmt="GT", lone_missing=False, width=None, idx=True) ->
     return b"".join(out)
 
 
-def write_bcf(path, v: vcf.Vcf, fmt="GT", lone_missing=False, width=None, compress="bgzf", idx=True, block_size=65280):
+def write_bcf(path, v: vcf.Vcf, fmt="GT", lone_missing=False, width=None, compress="bgzf", idx=True, block_size=65280,
+              call_type=None):
     """compress: "bgzf" (vcf.bgzf_compress, blocks of block_size input bytes), "gz" (one gzip member) or None."""
-    data = bcf_bytes(v, fmt, lone_missing, width, idx)
+    data = bcf_bytes(v, fmt, lone_missing, width, idx, call_type)
     if compress == "bgzf":
         data = vcf.bgzf_compress(data, block_size)
     elif compress == "gz":
@@ -327,6 +384,7 @@ def _parse(path):
                     raise vcf.VcfError(where + ": the GT field has a count of 0")
                 rec["gt_type"] = min(count, 15) << 4 | typ
                 rec["gt_raw"] = bytes(data[ind.i:ind.i + N * count * WIDTH[typ]])
+            rec.setdefault("ftype", {}).setdefault(sdict[key], (count, typ, k))
             rec["format"][sdict[key]] = ind.values(N * count, typ).reshape(N, count)
         if n_fmt == 0:
             raise vcf.VcfError(where + ": FORMAT does not start with GT (no FORMAT fields)")
@@ -352,8 +410,47 @@ def read_bcf(path) -> vcf.Vcf:
             if max((x for x in g if x != vcf.MISSING), default=-1) > len(r["alts"]):
                 raise vcf.VcfError(r["where"] + ": allele index above the ALT count")
             idx[s, i] = g
+    vals, bad = {}, None
+    for j, key in enumerate(("GQ", "DP")):
+        if any(key in r["format"] for r in recs):
+            vals[key] = np.full((len(recs), N), np.nan)
+            bad = np.zeros((len(recs), N, 2), bool) if bad is None else bad
+            for s, r in enumerate(recs):
+                if key in r["format"]:
+                    count, typ, _ = r["ftype"][key]
+                    if count != 1 or typ not in (INT8, INT16, INT32, FLOAT):     # refused only where filtered
+                        bad[s, :, j] = True
+                        continue
+                    raw = r["format"][key][:, 0]
+                    vals[key][s] = values_float(raw, typ)
+                    if typ == FLOAT:                                  # a NaN that is not a sentinel, or an infinity
+                        bad[s, :, j] = [value_rule(int(b), FLOAT, 1) < 0 for b in np.ascontiguousarray(raw).view(np.uint32)]
+                        vals[key][s][bad[s, :, j]] = np.nan
     return vcf.Vcf(samples=samples, chrom=[r["chrom"] for r in recs], pos=np.array([r["pos"] for r in recs], np.int64),
-                   ids=[r["id"] for r in recs], ref=[r["ref"] for r in recs], alts=[r["alts"] for r in recs], idx=idx)
+                   ids=[r["id"] for r in recs], ref=[r["ref"] for r in recs], alts=[r["alts"] for r in recs], idx=idx,
+                   gq=vals.get("GQ"), dp=vals.get("DP"), bad=bad)
+
+
+def call_values(path, keys=("GQ", "DP")):
+    """(bytes fv, int64 fv_off[L0+1], int32 fv_pos[L0, 2], uint8 fv_type[L0, 2], int32 fmt_index[L0, 2]): the GQ / DP
+    vectors as the driver's loader copies them out (per record the present ones in FORMAT order, each at a multiple of
+    4 bytes; -1 / 0 where absent) and their FORMAT indices."""
+    _, recs = _parse(path)
+    parts, off = [], [0]
+    pos = np.full((len(recs), 2), -1, np.int32)
+    types = np.zeros((len(recs), 2), np.uint8)
+    fidx = np.full((len(recs), 2), -1, np.int32)
+    for s, r in enumerate(recs):
+        span = b""
+        present = sorted((r["ftype"][k][2], j, k) for j, k in enumerate(("GQ", "DP")) if k in r["ftype"] and k in keys)
+        for order, j, k in present:
+            count, typ, _ = r["ftype"][k]
+            pos[s, j], types[s, j], fidx[s, j] = len(span), 1 << 4 | typ, order
+            raw = r["format"][k].tobytes()
+            span += raw + b"\0" * (-len(raw) % 4)
+        parts.append(span)
+        off.append(off[-1] + len(span))
+    return b"".join(parts), np.array(off, np.int64), pos, types, fidx
 
 
 def gt_payload(path):

@@ -11,6 +11,13 @@
 // SEL the samples listed in local[n_input] (common.cuh:select_local; the loads stay as they are, only the stores move).  The
 // diagnostics are reduced per warp and folded in with global atomics on arrays pre-set to -1 (atomicMax for the
 // largest allele index, an unsigned atomicMin for the first malformed sample), so a CTA never waits on a barrier.
+//
+// With FILTER (--vcf-min-gq / --vcf-min-dp) the record's GQ and DP vectors (count 1, one value per sample, staged in
+// their own buffer, kernels.h:CallFilter) are read alongside GT, coalesced the same way: in the int8 count-2 path an
+// int8 GQ / DP is one 16-bit load per word of two samples.  bcf_gt.cuh:bcf_value decides each value; a call that fails
+// a threshold is stored as two missing alleles.  The GT rule and the largest allele index apply to the calls as
+// written.  The first sample with a malformed value goes to bad_val (unsigned atomicMin on an array pre-set to -1), and
+// the stored calls with a present allele set missing are counted per thread and added once per warp at the end.
 #include <cstdint>
 
 #include "bcf_gt.cuh"
@@ -30,30 +37,83 @@ __device__ __forceinline__ int32_t load_value(const uint8_t* p, long long k, int
     return __ldg((const int32_t*)p + k);
 }
 
+// returns whether sample i is one of this handle's individuals (and was stored)
 template <bool SEL>
-__device__ __forceinline__ void store_call(uint8_t* dst, long long i, long long lo, long long hi, const int* local, int n_input,
+__device__ __forceinline__ bool store_call(uint8_t* dst, long long i, long long lo, long long hi, const int* local, int n_input,
                                            uint32_t ab)
 {
     if (SEL) {
         const int j = select_local(local, n_input, i);
         if (j >= 0) *(uint16_t*)(dst + 2 * j) = (uint16_t)ab;
-    } else if (i >= lo && i < hi) *(uint16_t*)(dst + 2 * (i - lo)) = (uint16_t)ab;
+        return j >= 0;
+    }
+    if (i >= lo && i < hi) { *(uint16_t*)(dst + 2 * (i - lo)) = (uint16_t)ab; return true; }
+    return false;
 }
 
-template <bool SEL>
+// The GQ or DP values of samples i and, if two, i + 1 of a count-1 vector of `type` at p (raw bits, sign-extended):
+// an int8 pair is one 16-bit load (i is even and p a multiple of 4 in the int8 count-2 path)
+__device__ __forceinline__ void load_values(const uint8_t* p, int type, long long i, bool two, int32_t* v)
+{
+    if (type == 1 && two) {
+        const uint16_t w = __ldg((const uint16_t*)(p + i));
+        v[0] = (int8_t)w;
+        v[1] = (int8_t)(w >> 8);
+    } else {
+        const int width = type == 1 ? 1 : type == 2 ? 2 : 4;
+        v[0] = load_value(p, i, width);
+        if (two) v[1] = load_value(p, i + 1, width);
+    }
+}
+
+// the filtered values of one record (kernels.h:CallFilter); a null pointer: absent or that filter off
+struct RecFilter {
+    const uint8_t *gq = nullptr, *dp = nullptr;
+    int gq_t = 0, dp_t = 0;
+};
+
+// the call filter on samples i (and i + 1 if two): bit j of the result set = call j fails a threshold; a malformed
+// value lowers *bad to its sample
+__device__ __forceinline__ unsigned filter_calls(const RecFilter& f, const CallFilter& cf, long long i, bool two, unsigned* bad)
+{
+    int32_t g[2] = {0, 0}, d[2] = {0, 0};
+    if (f.gq) load_values(f.gq, f.gq_t, i, two, g);
+    if (f.dp) load_values(f.dp, f.dp_t, i, two, d);
+    unsigned fail = 0;
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {
+        if (j && !two) break;
+        const int rg = f.gq ? bcf_value(g[j], f.gq_t, cf.min_gq) : 1;
+        const int rd = f.dp ? bcf_value(d[j], f.dp_t, cf.min_dp) : 1;
+        if (rg < 0 || rd < 0) { if ((unsigned)(i + j) < *bad) *bad = (unsigned)(i + j); }
+        else if (!rg || !rd) fail |= 1u << j;
+    }
+    return fail;
+}
+
+template <bool SEL, bool FILTER>
 __global__ void __launch_bounds__(kBcfThreads)
 decode_bcf_gt_kernel(const uint8_t* __restrict__ gt, const long long* __restrict__ off, const uint8_t* __restrict__ type,
                      int n_snp, int n_samples, int n_ind, int ind_lo, const int* __restrict__ local, int n_input,
                      uint8_t* __restrict__ alleles,
-                     int* __restrict__ max_allele, unsigned* __restrict__ bad_sample)
+                     int* __restrict__ max_allele, unsigned* __restrict__ bad_sample, CallFilter cf)
 {
     const long long lo = ind_lo, hi = (long long)ind_lo + n_ind;
+    unsigned long long my_set = 0;                 // FILTER: stored calls set missing, over every record of this thread
     for (int l = blockIdx.x; l < n_snp; l += gridDim.x) {
         const uint8_t* p = gt + off[l];
         uint8_t* dst = alleles + (size_t)l * n_ind * 2;
         const int count = type[l] >> 4, t = type[l] & 15, width = t == 1 ? 1 : t == 2 ? 2 : 4;
         int my_max = -1;
-        unsigned my_bad = 0xffffffffu;
+        unsigned my_bad = 0xffffffffu, my_badv = 0xffffffffu;
+        RecFilter f;
+        if (FILTER) {
+            const int2 ps = cf.fv_pos[l];
+            const uint8_t* base = cf.fv + cf.fv_off[l];
+            if (cf.min_gq && ps.x >= 0) { f.gq = base + ps.x; f.gq_t = cf.fv_type[2 * l] & 15; }
+            if (cf.min_dp && ps.y >= 0) { f.dp = base + ps.y; f.dp_t = cf.fv_type[2 * l + 1] & 15; }
+        }
+        const bool filt = FILTER && (f.gq || f.dp);
         if (width == 1 && count == 2) {
             const uint32_t* w = (const uint32_t*)p;
             const int n_words = (n_samples + 1) / 2;
@@ -92,8 +152,16 @@ decode_bcf_gt_kernel(const uint8_t* __restrict__ gt, const long long* __restrict
                             }
                         }
                     }
-                    store_call<SEL>(dst, i, lo, hi, local, n_input, out);
-                    store_call<SEL>(dst, i + 1, lo, hi, local, n_input, out >> 16);
+                    unsigned drop = 0;
+                    if (filt) {
+                        drop = filter_calls(f, cf, i, i + 1 < n_samples, &my_badv);
+                        if ((out & 0xffffu) == 0xffffu) drop &= ~1u;      // already two missing alleles: not counted
+                        if ((out >> 16) == 0xffffu) drop &= ~2u;
+                        out |= (drop & 1 ? 0xffffu : 0u) | (drop & 2 ? 0xffff0000u : 0u);
+                    }
+                    const bool s0 = store_call<SEL>(dst, i, lo, hi, local, n_input, out);
+                    const bool s1 = store_call<SEL>(dst, i + 1, lo, hi, local, n_input, out >> 16);
+                    if (FILTER) my_set += (s0 && (drop & 1)) + (s1 && (drop & 2));
                 }
             }
             const uint32_t m = max(max(hmax & 0xff, (hmax >> 8) & 0xff), max((hmax >> 16) & 0xff, hmax >> 24));
@@ -111,38 +179,59 @@ decode_bcf_gt_kernel(const uint8_t* __restrict__ gt, const long long* __restrict
                 } else if ((unsigned)i < my_bad) {
                     my_bad = (unsigned)i;
                 }
-                store_call<SEL>(dst, i, lo, hi, local, n_input, ok ? (uint32_t)(a | b << 8) : 0xffffu);
+                bool drop = false;
+                if (filt) drop = filter_calls(f, cf, i, false, &my_badv) && ok && (a != kBcfMissing || b != kBcfMissing);
+                const bool s = store_call<SEL>(dst, i, lo, hi, local, n_input, ok && !drop ? (uint32_t)(a | b << 8) : 0xffffu);
+                if (FILTER) my_set += s && drop;
             }
         }
         for (int o = 16; o; o >>= 1) {
             my_max = max(my_max, __shfl_xor_sync(0xffffffffu, my_max, o));
             my_bad = min(my_bad, __shfl_xor_sync(0xffffffffu, my_bad, o));
+            if (FILTER) my_badv = min(my_badv, __shfl_xor_sync(0xffffffffu, my_badv, o));
         }
         if ((threadIdx.x & 31) == 0) {
             if (my_max >= 0) atomicMax(max_allele + l, my_max);
             if (my_bad != 0xffffffffu) atomicMin(bad_sample + l, my_bad);
+            if (FILTER && my_badv != 0xffffffffu) atomicMin((unsigned*)cf.bad_val + l, my_badv);
         }
     }
+    if (FILTER) {
+        for (int o = 16; o; o >>= 1) my_set += __shfl_xor_sync(0xffffffffu, my_set, o);
+        if ((threadIdx.x & 31) == 0 && my_set) atomicAdd(cf.n_set_missing, my_set);
+    }
+}
+
+template <bool SEL>
+void launch_bcf(unsigned blocks, const uint8_t* gt, const long long* off, const uint8_t* type, int n_snp, int n_samples,
+                int n_ind, int ind_lo, const int* local, int n_input, uint8_t* alleles, int* max_allele, int* bad_sample,
+                const CallFilter& cf, cudaStream_t st)
+{
+    if (cf.fv)
+        decode_bcf_gt_kernel<SEL, true><<<blocks, kBcfThreads, 0, st>>>(gt, off, type, n_snp, n_samples, n_ind, ind_lo, local,
+                                                                        n_input, alleles, max_allele, (unsigned*)bad_sample, cf);
+    else
+        decode_bcf_gt_kernel<SEL, false><<<blocks, kBcfThreads, 0, st>>>(gt, off, type, n_snp, n_samples, n_ind, ind_lo, local,
+                                                                         n_input, alleles, max_allele, (unsigned*)bad_sample, cf);
 }
 
 }  // namespace
 
 cudaError_t launch_decode_bcf_gt(const uint8_t* gt, const long long* off, const uint8_t* type, int n_snp, int n_samples,
                                  int n_ind, int ind_lo, const int* local, int n_input, uint8_t* alleles, int* max_allele,
-                                 int* bad_sample, cudaStream_t st)
+                                 int* bad_sample, const CallFilter& cf, cudaStream_t st)
 {
     if (!n_snp) return cudaSuccess;
-    // -1 in both: "no allele" for atomicMax, and as unsigned the identity of atomicMin ("no malformed sample")
+    // -1 in each: "no allele" for atomicMax, and as unsigned the identity of atomicMin ("no malformed sample")
     cudaError_t e = cudaMemsetAsync(max_allele, 0xff, (size_t)n_snp * sizeof(int), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(bad_sample, 0xff, (size_t)n_snp * sizeof(int), st);
+    if (e == cudaSuccess && cf.fv) e = cudaMemsetAsync(cf.bad_val, 0xff, (size_t)n_snp * sizeof(int), st);
     if (e != cudaSuccess) return e;
     const unsigned blocks = n_snp < 148 * 8 ? n_snp : 148 * 8;
     if (local)
-        decode_bcf_gt_kernel<true><<<blocks, kBcfThreads, 0, st>>>(gt, off, type, n_snp, n_samples, n_ind, ind_lo, local, n_input,
-                                                                   alleles, max_allele, (unsigned*)bad_sample);
+        launch_bcf<true>(blocks, gt, off, type, n_snp, n_samples, n_ind, ind_lo, local, n_input, alleles, max_allele, bad_sample, cf, st);
     else
-        decode_bcf_gt_kernel<false><<<blocks, kBcfThreads, 0, st>>>(gt, off, type, n_snp, n_samples, n_ind, ind_lo, nullptr, 0,
-                                                                    alleles, max_allele, (unsigned*)bad_sample);
+        launch_bcf<false>(blocks, gt, off, type, n_snp, n_samples, n_ind, ind_lo, nullptr, 0, alleles, max_allele, bad_sample, cf, st);
     return cudaGetLastError();
 }
 

@@ -35,4 +35,28 @@ GHD int decode_gt(int32_t v0, int32_t v1, int count, int width, int* a, int* b)
     return 1;
 }
 
+// One GQ or DP value of a count-1 field of `type` (1/2/3 = int8/int16/int32, 5 = float) against an integer threshold
+// thr >= 1.  raw: the integer sign-extended from its width, or the float's bits.  Returns 1 if the call passes (value
+// >= thr, or the missing or end-of-vector sentinel of its type), 0 if it is below thr, -1 if it is malformed (a float
+// NaN other than the two sentinels 0x7F800001 / 0x7F800002, or an infinity).  Other integers compare as integers.
+GHD int bcf_value(int32_t raw, int type, int thr)
+{
+    if (type == 5) {
+        if (raw == 0x7F800001 || raw == 0x7F800002) return 1;
+        if ((raw & 0x7F800000) == 0x7F800000) return -1;
+        // a finite float passes iff its integer part (toward -inf) reaches thr; exact without a float compare
+        const int e = ((raw >> 23) & 0xff) - 127;
+        if (raw < 0 && (raw & 0x7fffffff)) return 0;   // negative (not -0)
+        if (e < 0) return 0 >= thr;
+        if (e >= 31) return 1;
+        const uint32_t m = (uint32_t)(raw & 0x7fffff) | 0x800000u;
+        const uint32_t ip = e >= 23 ? m << (e - 23) : m >> (23 - e);
+        return ip >= (uint32_t)thr;
+    }
+    const int width = type == 1 ? 1 : type == 2 ? 2 : 4;
+    const int32_t miss = width == 1 ? -128 : width == 2 ? -32768 : (int32_t)0x80000000u;
+    if (raw == miss || raw == bcf_eov(width)) return 1;
+    return raw >= thr;
+}
+
 }  // namespace garlic

@@ -79,6 +79,16 @@ struct garlic_gpu {
     int n_input = 0;
     int* d_local = nullptr;
     int32_t* d_sel_cols = nullptr;
+    // set_call_filter (--vcf-min-gq / --vcf-min-dp): thresholds (0 = off), the staged per-record FORMAT indices (VCF) or
+    // GQ / DP vectors (BCF), and the count of stored calls the filter set missing (device, and its copy after each put)
+    int min_gq = 0, min_dp = 0;
+    int2* d_fk = nullptr;
+    uint8_t* d_fv = nullptr;
+    long long* d_fv_off = nullptr;
+    int2* d_fv_pos = nullptr;
+    uint8_t* d_fv_type = nullptr;
+    unsigned long long* d_n_set = nullptr;
+    unsigned long long n_set_missing = 0;
     StitchScratch stitch_scratch;     // host buffers of call_roh kept between calls
     std::vector<RohRec> recs_buf, ambs_buf, merged_buf, tmp_buf;
     uint64_t* d_ldplanes = nullptr;   // LD scratch: bit-planes and the ordered pair matrix (kept between calls)
@@ -511,6 +521,7 @@ void garlic_gpu_destroy(garlic_gpu_t* h)
     dev_free(h->d_gl0); dev_free(h->d_gl); dev_free(h->d_freq0); dev_free(h->d_freq); dev_free(h->d_lut);
     dev_free(h->d_ldplanes); dev_free(h->d_ldpairs); dev_free(h->d_text); dev_free(h->d_textoff); dev_free(h->d_nonblank); dev_free(h->d_gt_type);
     dev_free(h->d_local); dev_free(h->d_sel_cols);
+    dev_free(h->d_fk); dev_free(h->d_fv); dev_free(h->d_fv_off); dev_free(h->d_fv_pos); dev_free(h->d_fv_type); dev_free(h->d_n_set);
     dev_free(h->d_gpos); dev_free(h->d_nomut); dev_free(h->d_norec); dev_free(h->d_wlut); dev_free(h->d_invld);
     dev_free(h->d_homf); dev_free(h->d_keep); dev_free(h->d_src); dev_free(h->d_pos0); dev_free(h->d_chr_of0);
     dev_free(h->d_pos); dev_free(h->d_chr_of); dev_free(h->d_chr_start); dev_free(h->d_chr_param);
@@ -611,8 +622,25 @@ int garlic_gpu_set_shape(garlic_gpu_t* h, int n_ind, int ind_offset, int64_t n_l
     dev_free(h->d_alleles); dev_free(h->d_key); dev_free(h->d_bed);
     h->bed_input = false; h->vcf_input = false;
     h->sel_cols.clear(); h->n_input = 0;
+    h->min_gq = h->min_dp = 0; h->n_set_missing = 0;
     return 0;
 }
+
+int garlic_gpu_set_call_filter(garlic_gpu_t* h, int min_gq, int min_dp)
+{
+    if (!h) return 1;
+    if (!h->L0) FAIL("set_call_filter: call set_shape first");
+    if (h->d_alleles || h->d_bed || h->have_geno0 || h->have_gl) FAIL("set_call_filter: call it before the first put_*");
+    if (min_gq < 0 || min_dp < 0) FAIL("set_call_filter: thresholds must be 0 (off) or positive");
+    CK(cudaSetDevice(h->device));
+    if (dev_alloc(h, &h->d_n_set, 1)) return 1;
+    CK(cudaMemsetAsync(h->d_n_set, 0, sizeof(unsigned long long), h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    h->min_gq = min_gq; h->min_dp = min_dp; h->n_set_missing = 0;
+    return 0;
+}
+
+uint64_t garlic_gpu_calls_set_missing(const garlic_gpu_t* h) { return h ? h->n_set_missing : 0; }
 
 int garlic_gpu_select_columns(garlic_gpu_t* h, const int32_t* columns, int n_input)
 {
@@ -692,8 +720,9 @@ int garlic_gpu_put_tped_text(garlic_gpu_t* h, const char* text, const int64_t* l
     return 0;
 }
 
-int garlic_gpu_put_vcf_text(garlic_gpu_t* h, const char* text, const int64_t* line_off, int64_t snp0, int n_snp,
-                            int32_t* n_cols, int32_t* max_allele, int32_t* bad_col)
+// put_vcf_text and put_vcf_text_filtered: fmt_index = nullptr runs the tokeniser without the call filter
+static int put_vcf_common(garlic_gpu* h, const char* text, const int64_t* line_off, int64_t snp0, int n_snp,
+                          const int32_t* fmt_index, int32_t* n_cols, int32_t* max_allele, int32_t* bad_col, int32_t* bad_value)
 {
     CK(cudaSetDevice(h->device));
     if (!h->L0) FAIL("put_vcf_text: call set_shape first");
@@ -710,28 +739,61 @@ int garlic_gpu_put_vcf_text(garlic_gpu_t* h, const char* text, const int64_t* li
     if (bytes < 0) FAIL("put_vcf_text: line offsets must ascend");
     if (dev_alloc(h, &h->d_text, (size_t)bytes + 16)) return 1;
     if (dev_alloc(h, &h->d_textoff, (size_t)n_snp + 1)) return 1;
-    if (dev_alloc(h, &h->d_nonblank, (size_t)3 * n_snp)) return 1;     // column count, largest index, first bad column
+    const bool filter = fmt_index && (h->min_gq || h->min_dp);
+    // column count, largest index, first bad column (and with the filter, first malformed value)
+    if (dev_alloc(h, &h->d_nonblank, (size_t)(filter ? 4 : 3) * n_snp)) return 1;
     std::vector<long long> rel(n_snp + 1);
     for (int i = 0; i <= n_snp; ++i) rel[i] = (long long)(line_off[i] - line_off[0]);
     CK(cudaMemcpyAsync(h->d_text, text + line_off[0], (size_t)bytes, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(h->d_textoff, rel.data(), rel.size() * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+    int* diag = h->d_nonblank;
+    CallFilter cf;
+    if (filter) {
+        if (dev_alloc(h, &h->d_fk, (size_t)n_snp)) return 1;
+        CK(cudaMemcpyAsync(h->d_fk, fmt_index, (size_t)n_snp * sizeof(int2), cudaMemcpyHostToDevice, h->stream));
+        cf.min_gq = h->min_gq; cf.min_dp = h->min_dp;
+        cf.fk = h->d_fk; cf.bad_val = diag + 3 * n_snp; cf.n_set_missing = h->d_n_set;
+    }
     uint8_t* dst = h->d_alleles + (size_t)snp0 * h->n_ind * 2;
     // a short record leaves its tail untouched: pre-fill with the missing code so that nothing undefined is coded
     CK(cudaMemsetAsync(dst, 255, (size_t)n_snp * h->n_ind * 2, h->stream));
-    int* diag = h->d_nonblank;
     LAUNCH(launch_tokenize_vcf(h->d_text, h->d_textoff, n_snp, h->n_ind, h->ind_offset, h->n_input ? h->d_local : nullptr,
-                               h->n_input, dst, diag, diag + n_snp, diag + 2 * n_snp, h->stream));
+                               h->n_input, dst, diag, diag + n_snp, diag + 2 * n_snp, cf, h->stream));
     LAUNCH(launch_first_allele(dst, n_snp, h->n_ind, h->ind_offset, 255, h->d_key + snp0, h->stream));
     h->missing_char = 255;
-    int32_t* out[3] = {n_cols, max_allele, bad_col};
-    for (int k = 0; k < 3; ++k)
+    int32_t* out[4] = {n_cols, max_allele, bad_col, filter ? bad_value : nullptr};
+    for (int k = 0; k < 4; ++k)
         if (out[k]) CK(cudaMemcpyAsync(out[k], diag + (size_t)k * n_snp, (size_t)n_snp * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    if (filter) CK(cudaMemcpyAsync(&h->n_set_missing, h->d_n_set, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));   // the caller may reuse its text buffer
+    if (bad_value && !filter) std::fill(bad_value, bad_value + n_snp, -1);
     return 0;
 }
 
-int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec_off, const uint8_t* gt_type,
-                          int n_samples, int64_t snp0, int n_snp, int32_t* max_allele, int32_t* bad_sample)
+int garlic_gpu_put_vcf_text(garlic_gpu_t* h, const char* text, const int64_t* line_off, int64_t snp0, int n_snp,
+                            int32_t* n_cols, int32_t* max_allele, int32_t* bad_col)
+{
+    return put_vcf_common(h, text, line_off, snp0, n_snp, nullptr, n_cols, max_allele, bad_col, nullptr);
+}
+
+int garlic_gpu_put_vcf_text_filtered(garlic_gpu_t* h, const char* text, const int64_t* line_off, int64_t snp0, int n_snp,
+                                     const int32_t* fmt_index, int32_t* n_cols, int32_t* max_allele, int32_t* bad_col,
+                                     int32_t* bad_value)
+{
+    if (!h) return 1;
+    if (!fmt_index) FAIL("put_vcf_text_filtered: fmt_index is NULL");
+    for (int l = 0; l < 2 * n_snp; ++l)
+        if (fmt_index[l] == 0 || fmt_index[l] < -1)
+            FAIL("put_vcf_text_filtered: record " + std::to_string(l / 2) + ": FORMAT index " + std::to_string(fmt_index[l]) +
+                 " is not -1 (absent) or 1 or more");
+    return put_vcf_common(h, text, line_off, snp0, n_snp, fmt_index, n_cols, max_allele, bad_col, bad_value);
+}
+
+// put_bcf_gt and put_bcf_gt_filtered: fv_off = nullptr decodes without the call filter (fv may be nullptr while the
+// block's records hold no GQ / DP vector)
+static int put_bcf_common(garlic_gpu* h, const uint8_t* gt, const int64_t* rec_off, const uint8_t* gt_type, int n_samples,
+                          int64_t snp0, int n_snp, const uint8_t* fv, const int64_t* fv_off, const int32_t* fv_pos,
+                          const uint8_t* fv_type, int32_t* max_allele, int32_t* bad_sample, int32_t* bad_value)
 {
     CK(cudaSetDevice(h->device));
     if (!h->L0) FAIL("put_bcf_gt: call set_shape first");
@@ -751,6 +813,22 @@ int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec
         if (rec_off[l + 1] - rec_off[l] < need)
             FAIL("put_bcf_gt: record " + std::to_string(l) + ": payload shorter than its descriptor needs");
     }
+    const bool filter = fv_off && (h->min_gq || h->min_dp);
+    for (int l = 0; l < n_snp && filter; ++l) {
+        if (fv_off[l] % 4 != 0) FAIL("put_bcf_gt_filtered: record " + std::to_string(l) + ": GQ / DP offset is not a multiple of 4");
+        for (int f = 0; f < 2; ++f) {
+            const int32_t at = fv_pos[2 * l + f];
+            if (at < 0 || !(f ? h->min_dp : h->min_gq)) continue;
+            const char* key = f ? "DP" : "GQ";
+            const int count = fv_type[2 * l + f] >> 4, t = fv_type[2 * l + f] & 15;
+            if (count != 1 || !(t == 1 || t == 2 || t == 3 || t == 5))
+                FAIL("put_bcf_gt_filtered: record " + std::to_string(l) + ": " + key + " descriptor " + std::to_string(fv_type[2 * l + f]) +
+                     " is not an int8, int16, int32 or float field with a count of 1");
+            if (at % 4 != 0) FAIL("put_bcf_gt_filtered: record " + std::to_string(l) + ": " + key + " offset is not a multiple of 4");
+            if (fv_off[l] + at + (int64_t)n_samples * (t == 1 ? 1 : t == 2 ? 2 : 4) > fv_off[l + 1])
+                FAIL("put_bcf_gt_filtered: record " + std::to_string(l) + ": " + key + " vector runs past the record's span");
+        }
+    }
     if (!h->d_alleles) {
         if (dev_alloc(h, &h->d_alleles, (size_t)h->L0 * h->n_ind * 2)) return 1;
         if (dev_alloc(h, &h->d_key, (size_t)h->L0)) return 1;
@@ -760,7 +838,7 @@ int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec
     if (dev_alloc(h, &h->d_text, (size_t)bytes + 16)) return 1;
     if (dev_alloc(h, &h->d_textoff, (size_t)n_snp + 1)) return 1;
     if (dev_alloc(h, &h->d_gt_type, (size_t)n_snp)) return 1;
-    if (dev_alloc(h, &h->d_nonblank, (size_t)2 * n_snp)) return 1;     // largest index, first bad sample
+    if (dev_alloc(h, &h->d_nonblank, (size_t)(filter ? 3 : 2) * n_snp)) return 1;   // largest index, first bad sample, bad value
     std::vector<long long> rel(n_snp + 1);
     for (int i = 0; i <= n_snp; ++i) rel[i] = (long long)(rec_off[i] - rec_off[0]);
     CK(cudaMemcpyAsync(h->d_text, gt + rec_off[0], (size_t)bytes, cudaMemcpyHostToDevice, h->stream));
@@ -768,16 +846,56 @@ int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec
     CK(cudaMemcpyAsync(h->d_gt_type, gt_type, (size_t)n_snp, cudaMemcpyHostToDevice, h->stream));
     uint8_t* dst = h->d_alleles + (size_t)snp0 * h->n_ind * 2;
     int* diag = h->d_nonblank;
+    CallFilter cf;
+    if (filter) {
+        const int64_t fbytes = fv_off[n_snp] - fv_off[0];
+        if (fbytes < 0) FAIL("put_bcf_gt_filtered: GQ / DP offsets must ascend");
+        std::vector<long long> frel(n_snp + 1);
+        for (int i = 0; i <= n_snp; ++i) frel[i] = (long long)(fv_off[i] - fv_off[0]);
+        if (dev_alloc(h, &h->d_fv, (size_t)fbytes + 16)) return 1;
+        if (dev_alloc(h, &h->d_fv_off, (size_t)n_snp + 1)) return 1;
+        if (dev_alloc(h, &h->d_fv_pos, (size_t)n_snp)) return 1;
+        if (dev_alloc(h, &h->d_fv_type, (size_t)2 * n_snp)) return 1;
+        if (fbytes) CK(cudaMemcpyAsync(h->d_fv, fv + fv_off[0], (size_t)fbytes, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(h->d_fv_off, frel.data(), frel.size() * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(h->d_fv_pos, fv_pos, (size_t)n_snp * sizeof(int2), cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(h->d_fv_type, fv_type, (size_t)2 * n_snp, cudaMemcpyHostToDevice, h->stream));
+        cf.min_gq = h->min_gq; cf.min_dp = h->min_dp;
+        cf.fv = h->d_fv; cf.fv_off = h->d_fv_off; cf.fv_pos = h->d_fv_pos; cf.fv_type = h->d_fv_type;
+        cf.bad_val = diag + 2 * n_snp; cf.n_set_missing = h->d_n_set;
+    }
     // every sample of this handle is stored (a malformed one as 255), so no pre-fill is needed
     LAUNCH(launch_decode_bcf_gt((const uint8_t*)h->d_text, h->d_textoff, h->d_gt_type, n_snp, n_samples, h->n_ind,
-                                h->ind_offset, h->n_input ? h->d_local : nullptr, h->n_input, dst, diag, diag + n_snp, h->stream));
+                                h->ind_offset, h->n_input ? h->d_local : nullptr, h->n_input, dst, diag, diag + n_snp, cf, h->stream));
     LAUNCH(launch_first_allele(dst, n_snp, h->n_ind, h->ind_offset, 255, h->d_key + snp0, h->stream));
     h->missing_char = 255;
-    int32_t* out[2] = {max_allele, bad_sample};
-    for (int k = 0; k < 2; ++k)
+    int32_t* out[3] = {max_allele, bad_sample, filter ? bad_value : nullptr};
+    for (int k = 0; k < 3; ++k)
         if (out[k]) CK(cudaMemcpyAsync(out[k], diag + (size_t)k * n_snp, (size_t)n_snp * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    if (filter) CK(cudaMemcpyAsync(&h->n_set_missing, h->d_n_set, sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));   // the caller may reuse its buffers
+    if (bad_value && !filter) std::fill(bad_value, bad_value + n_snp, -1);
     return 0;
+}
+
+int garlic_gpu_put_bcf_gt(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec_off, const uint8_t* gt_type,
+                          int n_samples, int64_t snp0, int n_snp, int32_t* max_allele, int32_t* bad_sample)
+{
+    return put_bcf_common(h, gt, rec_off, gt_type, n_samples, snp0, n_snp, nullptr, nullptr, nullptr, nullptr, max_allele,
+                          bad_sample, nullptr);
+}
+
+int garlic_gpu_put_bcf_gt_filtered(garlic_gpu_t* h, const uint8_t* gt, const int64_t* rec_off, const uint8_t* gt_type,
+                                   int n_samples, int64_t snp0, int n_snp, const uint8_t* fv, const int64_t* fv_off,
+                                   const int32_t* fv_pos, const uint8_t* fv_type, int32_t* max_allele, int32_t* bad_sample,
+                                   int32_t* bad_value)
+{
+    if (!h) return 1;
+    if (!fv_off || !fv_pos || !fv_type) FAIL("put_bcf_gt_filtered: fv_off, fv_pos or fv_type is NULL");
+    if (!fv && n_snp > 0 && fv_off[n_snp] != fv_off[0])
+        FAIL("put_bcf_gt_filtered: fv is NULL but the records hold GQ / DP vectors");
+    return put_bcf_common(h, gt, rec_off, gt_type, n_samples, snp0, n_snp, fv, fv_off, fv_pos, fv_type, max_allele,
+                          bad_sample, bad_value);
 }
 
 void* garlic_gpu_first_allele_keys_dev(garlic_gpu_t* h) { return h ? (void*)h->d_key : nullptr; }

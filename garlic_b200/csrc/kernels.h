@@ -77,16 +77,31 @@ cudaError_t launch_bucket_by_individual(RohRec* in, const unsigned* count, unsig
 // local[n_input] maps to an individual (garlic_gpu_select_columns, common.cuh:select_local)
 cudaError_t launch_tokenize_tped(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
                                  int n_input, uint8_t* alleles, int* nonblank, cudaStream_t st);
+// The call filter of the VCF / BCF ingest kernels (--vcf-min-gq / --vcf-min-dp, garlic_gpu_set_call_filter): a call whose
+// GQ is below min_gq or whose DP is below min_dp (0: that filter off) is stored as two missing alleles.  The filter is
+// off unless fk (VCF) or fv (BCF) is set.  Per record bad_val = the first sample with a malformed value (-1 if none);
+// *n_set_missing += the stored calls with a present allele that the filter set missing.
+struct CallFilter {
+    int min_gq = 0, min_dp = 0;
+    const int2* fk = nullptr;           // VCF: per record the FORMAT index of GQ (x) and DP (y), -1 if absent
+    const uint8_t* fv = nullptr;        // BCF: the GQ / DP vectors; record l's span starts at fv + fv_off[l] (a multiple of 4)
+    const long long* fv_off = nullptr;
+    const int2* fv_pos = nullptr;       // BCF: per record the offsets of GQ (x) and DP (y) in the span, -1 if absent
+    const uint8_t* fv_type = nullptr;   // BCF: per record the descriptors of GQ and DP (count 1; int8/16/32 or float)
+    int* bad_val = nullptr;
+    unsigned long long* n_set_missing = nullptr;
+};
 // vcf.cu: VCF sample columns → allele index bytes (255 = missing) and per record the column count, the largest allele
 // index (-1 if none) and the first column whose GT is malformed (-1 if none)
 cudaError_t launch_tokenize_vcf(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
-                                int n_input, uint8_t* alleles, int* n_cols, int* max_allele, int* bad_col, cudaStream_t st);
+                                int n_input, uint8_t* alleles, int* n_cols, int* max_allele, int* bad_col, const CallFilter& cf,
+                                cudaStream_t st);
 // bcf.cu: BCF GT vectors (record l: n_samples x count values at gt + off[l], type[l] = the GT's typed descriptor) →
 // allele index bytes (255 = missing) and per record the largest allele index (-1 if none) and the first malformed
 // sample (-1 if none)
 cudaError_t launch_decode_bcf_gt(const uint8_t* gt, const long long* off, const uint8_t* type, int n_snp, int n_samples,
                                  int n_ind, int ind_lo, const int* local, int n_input, uint8_t* alleles, int* max_allele,
-                                 int* bad_sample, cudaStream_t st);
+                                 int* bad_sample, const CallFilter& cf, cudaStream_t st);
 cudaError_t launch_first_allele(const uint8_t* alleles, int n_snp, int n_ind, int ind_offset, int missing,
                                 unsigned long long* key, cudaStream_t st);
 cudaError_t launch_code_alleles(const uint8_t* alleles, int n_snp, int n_ind, int missing,

@@ -6,6 +6,12 @@
 // start parses that column's GT (vcf_gt.cuh:parse_gt) from global memory.  Every rank parses every column so that the
 // per-record diagnostics are the same on all ranks; it stores only the columns of its own individuals
 // [ind_lo, ind_lo + n_ind), or with SEL the columns listed in local[n_input] (common.cuh:select_local).
+//
+// With FILTER (--vcf-min-gq / --vcf-min-dp) the thread that owns a column walks on from its GT to the record's GQ and DP
+// subfields, whose FORMAT indices fk[l] the host found (-1: absent), and applies vcf_gt.cuh:call_filter: a call below a
+// threshold is stored as two missing alleles.  Per record it reports the first column with a malformed value in
+// bad_val, and it adds the number of stored calls with a present allele that it set missing to *n_set_missing.  The
+// GT grammar and the largest allele index are checked on the calls as written, filtered or not.
 #include <climits>
 #include <cstdint>
 
@@ -18,23 +24,30 @@ namespace {
 
 constexpr int kVcfChars = 16;   // characters per thread per tile
 
-template <bool SEL>
+template <bool SEL, bool FILTER>
 __global__ void __launch_bounds__(256)
 tokenize_vcf_kernel(const char* __restrict__ text, const long long* __restrict__ off, int n_snp, int n_ind, int ind_lo,
                     const int* __restrict__ local, int n_input, uint8_t* __restrict__ alleles, int* __restrict__ n_cols,
-                    int* __restrict__ max_allele, int* __restrict__ bad_col)
+                    int* __restrict__ max_allele, int* __restrict__ bad_col, CallFilter cf)
 {
     __shared__ int s_warp[8];
-    __shared__ int s_base, s_max, s_bad;
+    __shared__ int s_base, s_max, s_bad, s_badv;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long long c_lo = ind_lo, c_hi = (long long)ind_lo + n_ind;
+    unsigned long long my_set = 0;                 // FILTER: stored calls set missing, over every record of this thread
     for (int l = blockIdx.x; l < n_snp; l += gridDim.x) {
         const char* line = text + off[l];
         const long long len = off[l + 1] - off[l];
         uint8_t* dst = alleles + (size_t)l * n_ind * 2;
-        if (threadIdx.x == 0) { s_base = 0; s_max = -1; s_bad = INT_MAX; }
+        if (threadIdx.x == 0) { s_base = 0; s_max = -1; s_bad = INT_MAX; if (FILTER) s_badv = INT_MAX; }
         __syncthreads();
-        int my_max = -1, my_bad = INT_MAX;
+        int my_max = -1, my_bad = INT_MAX, my_badv = INT_MAX;
+        int k_gq = -1, k_dp = -1;
+        if (FILTER) {
+            const int2 k = cf.fk[l];
+            k_gq = cf.min_gq ? k.x : -1;
+            k_dp = cf.min_dp ? k.y : -1;
+        }
         // position len is scanned too: a record that ends in a tab has an empty last column (an empty record has none)
         for (long long t0 = 0; t0 <= len; t0 += 256 * kVcfChars) {
             const long long i0 = t0 + (long long)threadIdx.x * kVcfChars;
@@ -62,15 +75,24 @@ tokenize_vcf_kernel(const char* __restrict__ text, const long long* __restrict__
                 const long long i = i0 + k;
                 int a, b;
                 if (parse_gt(line + i, len - i, &a, &b)) {
+                    if (a != kVcfMissing && a > my_max) my_max = a;
+                    if (b != kVcfMissing && b > my_max) my_max = b;
+                    bool drop = false;
+                    if (FILTER) {
+                        int field;
+                        const int r = call_filter(line + i, len - i, k_gq, cf.min_gq, k_dp, cf.min_dp, &field);
+                        if (r < 0 && col < my_badv) my_badv = (int)col;
+                        drop = r > 0 && (a != kVcfMissing || b != kVcfMissing);
+                        if (drop) a = b = kVcfMissing;
+                    }
                     if (SEL) {
                         const int j = select_local(local, n_input, col);
-                        if (j >= 0) { dst[2 * j] = (uint8_t)a; dst[2 * j + 1] = (uint8_t)b; }
+                        if (j >= 0) { dst[2 * j] = (uint8_t)a; dst[2 * j + 1] = (uint8_t)b; my_set += FILTER && drop; }
                     } else if (col >= c_lo && col < c_hi) {
                         dst[2 * (col - c_lo)] = (uint8_t)a;
                         dst[2 * (col - c_lo) + 1] = (uint8_t)b;
+                        my_set += FILTER && drop;
                     }
-                    if (a != kVcfMissing && a > my_max) my_max = a;
-                    if (b != kVcfMissing && b > my_max) my_max = b;
                 } else if (col < my_bad) {
                     my_bad = (int)col;
                 }
@@ -83,31 +105,48 @@ tokenize_vcf_kernel(const char* __restrict__ text, const long long* __restrict__
         for (int o = 16; o; o >>= 1) {
             my_max = max(my_max, __shfl_xor_sync(0xffffffffu, my_max, o));
             my_bad = min(my_bad, __shfl_xor_sync(0xffffffffu, my_bad, o));
+            if (FILTER) my_badv = min(my_badv, __shfl_xor_sync(0xffffffffu, my_badv, o));
         }
-        if (lane == 0) { atomicMax(&s_max, my_max); atomicMin(&s_bad, my_bad); }
+        if (lane == 0) { atomicMax(&s_max, my_max); atomicMin(&s_bad, my_bad); if (FILTER) atomicMin(&s_badv, my_badv); }
         __syncthreads();
         if (threadIdx.x == 0) {
             n_cols[l] = s_base;
             max_allele[l] = s_max;
             bad_col[l] = s_bad == INT_MAX ? -1 : s_bad;
+            if (FILTER) cf.bad_val[l] = s_badv == INT_MAX ? -1 : s_badv;
         }
         __syncthreads();
     }
+    if (FILTER) {
+        for (int o = 16; o; o >>= 1) my_set += __shfl_xor_sync(0xffffffffu, my_set, o);
+        if (lane == 0 && my_set) atomicAdd(cf.n_set_missing, my_set);
+    }
+}
+
+template <bool SEL>
+void launch_vcf(unsigned blocks, const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
+                int n_input, uint8_t* alleles, int* n_cols, int* max_allele, int* bad_col, const CallFilter& cf, cudaStream_t st)
+{
+    if (cf.fk)
+        tokenize_vcf_kernel<SEL, true><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, local, n_input, alleles, n_cols,
+                                                               max_allele, bad_col, cf);
+    else
+        tokenize_vcf_kernel<SEL, false><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, local, n_input, alleles, n_cols,
+                                                                max_allele, bad_col, cf);
 }
 
 }  // namespace
 
 cudaError_t launch_tokenize_vcf(const char* text, const long long* off, int n_snp, int n_ind, int ind_lo, const int* local,
-                                int n_input, uint8_t* alleles, int* n_cols, int* max_allele, int* bad_col, cudaStream_t st)
+                                int n_input, uint8_t* alleles, int* n_cols, int* max_allele, int* bad_col, const CallFilter& cf,
+                                cudaStream_t st)
 {
     if (!n_snp) return cudaSuccess;
     const unsigned blocks = n_snp < 148 * 8 ? n_snp : 148 * 8;
     if (local)
-        tokenize_vcf_kernel<true><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, local, n_input, alleles, n_cols,
-                                                          max_allele, bad_col);
+        launch_vcf<true>(blocks, text, off, n_snp, n_ind, ind_lo, local, n_input, alleles, n_cols, max_allele, bad_col, cf, st);
     else
-        tokenize_vcf_kernel<false><<<blocks, 256, 0, st>>>(text, off, n_snp, n_ind, ind_lo, nullptr, 0, alleles, n_cols,
-                                                           max_allele, bad_col);
+        launch_vcf<false>(blocks, text, off, n_snp, n_ind, ind_lo, nullptr, 0, alleles, n_cols, max_allele, bad_col, cf, st);
     return cudaGetLastError();
 }
 

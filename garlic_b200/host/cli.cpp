@@ -81,9 +81,12 @@ static const char* kHelp =
     "Extensions: --bfile <prefix> (PLINK 1 binary fileset prefix.bed/.bim/.fam in place of --tped/--tfam; not with --phased),\n"
     "  --vcf <file> (VCF, plain, gzip or BGZF, or BCF 2.2, uncompressed or BGZF, in place of --tped; FORMAT must start\n"
     "  with GT and every GT must be diploid, so restrict the input to the autosomes; QUAL, FILTER and INFO are ignored and\n"
-    "  no filter is applied; --tfam is optional:\n"
+    "  no filter is applied except --vcf-min-gq / --vcf-min-dp; --tfam is optional:\n"
     "  its IDs must equal the VCF samples in order and it names the population, which is VCF without it; not with\n"
     "  --host-tokenize),\n"
+    "  --vcf-min-gq <T>, --vcf-min-dp <D> (--vcf input only, integers >= 1: a call whose FORMAT GQ is below T, or whose DP\n"
+    "  is below D, is set missing, as if written ./.; a missing or absent value passes; QUAL, FILTER and INFO are still\n"
+    "  ignored),\n"
     "  --gpus <n> (shard individuals over n GPUs), --exact (whole-segment chains), --device <n>, --seed <n> (subsample RNG seed), --device-lut, --kde-direct, --kde-gpu (the KDE itself on the GPU: exact Gauss transform of the thinned windows still in HBM), --host-tokenize (tped allele columns extracted on the host instead of the GPU tokeniser)\n"
     "  --by-pop (a tfam or .fam with several population IDs, the first column: each population, in order of first\n"
     "  appearance, is analysed as a separate run with the same flags would analyse it, its outputs under <out>.<pop>;\n"
@@ -100,7 +103,7 @@ int parse_cli(int argc, char** argv, Options& o, std::string& cmdline)
     std::map<std::string, int*> fi = {{"--winsize", &o.winsize}, {"--auto-winsize-step", &o.auto_winsize_step},
         {"--max-gap", &o.max_gap}, {"--resample", &o.resample}, {"--threads", &o.threads}, {"--M", &o.M},
         {"--nclust", &o.nclust}, {"--kde-subsample", &o.kde_subsample}, {"--ld-subsample", &o.ld_subsample},
-        {"--device", &o.device}, {"--gpus", &o.gpus}};
+        {"--device", &o.device}, {"--gpus", &o.gpus}, {"--vcf-min-gq", &o.vcf_min_gq}, {"--vcf-min-dp", &o.vcf_min_dp}};
     std::map<std::string, double*> fd = {{"--error", &o.error}, {"--overlap-frac", &o.overlap_frac},
         {"--lod-cutoff", &o.lod_cutoff}, {"--mu", &o.mu}};
     std::map<std::string, std::string*> fs = {{"--tped", &o.tped}, {"--tfam", &o.tfam}, {"--tgls", &o.tgls},
@@ -123,6 +126,10 @@ int parse_cli(int argc, char** argv, Options& o, std::string& cmdline)
         if (fi.count(a)) {
             if (!good_int(v)) { fprintf(stderr, "ERROR: %s is not a valid integer.\n", v.c_str()); return -1; }
             *fi[a] = atoi(v.c_str());
+            if ((a == "--vcf-min-gq" || a == "--vcf-min-dp") && *fi[a] < 1) {
+                fprintf(stderr, "ERROR: %s must be an integer >= 1.\n", a.c_str());
+                return -1;
+            }
             ++i;
         } else if (a == "--seed") {
             if (!good_int(v)) { fprintf(stderr, "ERROR: %s is not a valid integer.\n", v.c_str()); return -1; }

@@ -53,6 +53,8 @@ struct Options {
     bool kde_direct = false;     // extension: exact (reproducible) Gauss transform for the KDE (--kde-direct)
     bool kde_gpu = false;        // extension: computeKDE on the GPU, from the thinned windows still in HBM (--kde-gpu)
     bool by_pop = false;         // extension: analyse each population of the tfam in turn, outputs under <out>.<pop> (--by-pop)
+    int vcf_min_gq = 0;          // extension: --vcf input, a call whose FORMAT GQ is below this is set missing (0 = off)
+    int vcf_min_dp = 0;          // extension: --vcf input, a call whose FORMAT DP is below this is set missing (0 = off)
     long seed = -1;              // extension: RNG seed for the KDE / LD subsamples (--seed; default time)
 };
 // returns 0 = run, 1 = help printed (exit 0), -1 = error
@@ -94,8 +96,21 @@ struct Vcf {
     std::vector<int64_t> line;                    // per record, its line number in the file, or its record number
                                                   // (1-based) in a BCF (for messages)
     std::vector<uint8_t> gt_type;                 // BCF: per record the GT's typed descriptor; empty for VCF text
+    // load_vcf with call_keys (--vcf-min-gq / --vcf-min-dp), per record l: fmt_index[2l] / [2l+1] = the FORMAT index of
+    // GQ / DP (GT = 0), -1 if the record lacks it or it was not asked for.  BCF: the asked-for GQ / DP vectors, copied
+    // out of the record into fv (not Tped::text): record l's span is fv[fv_off[l], fv_off[l+1]), the vectors at
+    // fv_pos[2l] / [2l+1] within it (multiples of 4, -1 if absent), their descriptors in fv_type[2l] / [2l+1]
+    // (garlic_gpu_put_bcf_gt_filtered).
+    std::vector<int32_t> fmt_index;
+    std::vector<uint8_t> fv;
+    std::vector<int64_t> fv_off;
+    std::vector<int32_t> fv_pos;
+    std::vector<uint8_t> fv_type;
 };
 bool load_vcf(const std::string& path, Tped& t, Vcf& v);
+// call_keys: bit 0 = record GQ, bit 1 = record DP (above).  A BCF GQ / DP asked for must have count 1 and type int8,
+// int16, int32 or float, else the record is rejected.
+bool load_vcf(const std::string& path, Tped& t, Vcf& v, unsigned call_keys);
 struct Scaffold { std::string chr; std::vector<int32_t> pos; std::vector<double> gen; };
 bool load_map(const std::string& path, std::vector<Scaffold>& s);
 // values individual-major [N][L0]

@@ -360,7 +360,7 @@ struct ChrRuns {
 // 9 tab-separated fixed columns and the sample columns.  CHROM / ID / POS take the places of the tped's columns 1 / 2 / 4;
 // the sample text is kept raw, as load_tped keeps its genotype columns, and parsed on the GPU (vcf.cu).
 template <class Lines>
-bool parse_vcf(Lines& in, const std::string& path, Tped& t, Vcf& v)
+bool parse_vcf(Lines& in, const std::string& path, Tped& t, Vcf& v, unsigned call_keys)
 {
     t = Tped();
     v = Vcf();
@@ -421,6 +421,19 @@ bool parse_vcf(Lines& in, const std::string& path, Tped& t, Vcf& v)
                 a = c + 1;
             }
         v.line.push_back(line_no);
+        if (call_keys) {                              // the FORMAT indices of GQ and DP
+            int32_t gq = -1, dp = -1, k = 0;
+            for (const char *a = f[8], *fe = f[8] + fl[8];; ++k) {
+                const char* c = (const char*)memchr(a, ':', fe - a);
+                const size_t kl = (c ? c : fe) - a;
+                if (kl == 2 && a[0] == 'G' && a[1] == 'Q' && gq < 0 && (call_keys & 1)) gq = k;
+                if (kl == 2 && a[0] == 'D' && a[1] == 'P' && dp < 0 && (call_keys & 2)) dp = k;
+                if (!c) break;
+                a = c + 1;
+            }
+            v.fmt_index.push_back(gq);
+            v.fmt_index.push_back(dp);
+        }
         if (q) t.text.insert(t.text.end(), q, e);      // the sample columns: parsed on the GPU
         t.text_off.push_back((int64_t)t.text.size());
         ++t.n_loci;
@@ -546,12 +559,13 @@ struct Typed {
 // l_shared.  The first FORMAT field must be GT, whose values are appended to Tped::text with each record's payload at
 // a multiple of 4 bytes, and its descriptor to Vcf::gt_type: decoded on the GPU (bcf.cu).
 template <class Reader>
-bool parse_bcf(Reader& in, const std::string& path, Tped& t, Vcf& v)
+bool parse_bcf(Reader& in, const std::string& path, Tped& t, Vcf& v, unsigned call_keys)
 {
     t = Tped();
     v = Vcf();
     t.chr_off.push_back(0);
     t.text_off.push_back(0);
+    if (call_keys) v.fv_off.push_back(0);
     const char* p;
     size_t got;
     auto head_bad = [&](const std::string& why) {
@@ -636,6 +650,44 @@ bool parse_bcf(Reader& in, const std::string& path, Tped& t, Vcf& v)
         const uint64_t bytes = (uint64_t)n_sample * (uint64_t)count * Typed::width(type);
         if (bytes > ind.n - ind.i)
             return bad("the GT vector (" + std::to_string(bytes) + " bytes) is longer than l_indiv (" + std::to_string(l_indiv) + ").");
+        if (call_keys) {
+            // the GQ / DP vectors: every FORMAT field after GT is stepped over through its descriptor
+            int32_t kpos[2] = {-1, -1}, kidx[2] = {-1, -1};
+            uint8_t kdesc[2] = {0, 0};
+            const size_t span0 = v.fv.size();
+            Typed f = ind;
+            f.i += bytes;
+            for (uint32_t k = 1; k < n_fmt; ++k) {
+                int64_t fkey, fcount;
+                int ftype;
+                if (!f.typed_int(fkey) || !f.desc(ftype, fcount))
+                    return bad("l_indiv (" + std::to_string(l_indiv) + ") is too small for FORMAT field " + std::to_string(k + 1) + ".");
+                const std::string name = strings.at(fkey);
+                if (name.empty()) return bad("FORMAT key " + std::to_string(fkey) + " is not in the header's dictionary of strings.");
+                if (Typed::width(ftype) == 0) return bad("the " + name + " field is of unknown type " + std::to_string(ftype) + ".");
+                const uint64_t fb = (uint64_t)n_sample * (uint64_t)fcount * Typed::width(ftype);
+                if (fb > f.n - f.i)
+                    return bad("the " + name + " vector (" + std::to_string(fb) + " bytes) runs past l_indiv (" + std::to_string(l_indiv) + ").");
+                const int which = name == "GQ" ? 0 : name == "DP" ? 1 : -1;
+                if (which >= 0 && (call_keys >> which & 1) && kpos[which] < 0) {
+                    if (fcount != 1 || !(ftype == 1 || ftype == 2 || ftype == 3 || ftype == 5))
+                        return bad("the " + name + " field has count " + std::to_string(fcount) + " and type " + std::to_string(ftype) +
+                                   "; --vcf-min-" + (which ? "dp" : "gq") + " needs count 1 and type int8, int16, int32 or float.");
+                    kpos[which] = (int32_t)(v.fv.size() - span0);
+                    kidx[which] = (int32_t)k;
+                    kdesc[which] = (uint8_t)(1 << 4 | ftype);
+                    v.fv.insert(v.fv.end(), f.p + f.i, f.p + f.i + fb);
+                    v.fv.resize((v.fv.size() + 3) & ~(size_t)3, 0);
+                }
+                f.i += fb;
+            }
+            v.fv_off.push_back((int64_t)v.fv.size());
+            for (int w = 0; w < 2; ++w) {
+                v.fmt_index.push_back(kidx[w]);
+                v.fv_pos.push_back(kpos[w]);
+                v.fv_type.push_back(kdesc[w]);
+            }
+        }
         runs.add(t, chr);
         t.snp_id.push_back(id.empty() ? "." : id);
         t.pos.push_back((int32_t)pos);
@@ -665,14 +717,16 @@ std::string head_bytes(const std::string& path)
 }
 
 template <class Reader>
-bool parse_vcf_or_bcf(Reader& in, const std::string& path, Tped& t, Vcf& v, bool bcf)
+bool parse_vcf_or_bcf(Reader& in, const std::string& path, Tped& t, Vcf& v, bool bcf, unsigned call_keys)
 {
-    return bcf ? parse_bcf(in, path, t, v) : parse_vcf(in, path, t, v);
+    return bcf ? parse_bcf(in, path, t, v, call_keys) : parse_vcf(in, path, t, v, call_keys);
 }
 
 }  // namespace
 
-bool load_vcf(const std::string& path, Tped& t, Vcf& v)
+bool load_vcf(const std::string& path, Tped& t, Vcf& v) { return load_vcf(path, t, v, 0); }
+
+bool load_vcf(const std::string& path, Tped& t, Vcf& v, unsigned call_keys)
 {
     const std::string magic = head_bytes(path);
     const bool bcf = magic.size() >= 3 && magic.compare(0, 3, "BCF") == 0;
@@ -684,11 +738,11 @@ bool load_vcf(const std::string& path, Tped& t, Vcf& v)
     if (BgzfLines::sniff(path)) {
         BgzfLines in;
         if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
-        return parse_vcf_or_bcf(in, path, t, v, bcf);
+        return parse_vcf_or_bcf(in, path, t, v, bcf, call_keys);
     }
     GzLines in;
     if (!in.open(path)) { LOG.error("ERROR: Failed to open " + path); return false; }
-    return parse_vcf_or_bcf(in, path, t, v, bcf);
+    return parse_vcf_or_bcf(in, path, t, v, bcf, call_keys);
 }
 
 // scanIndData3 / readIndData3 (garlic-data.cpp:1893-2014): single population, unique IDs.

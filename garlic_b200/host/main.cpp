@@ -19,6 +19,7 @@
 #include "../../include/garlic_b200.h"
 #include "garlic_host.h"
 #include "../csrc/bcf_gt.cuh"
+#include "../csrc/vcf_gt.cuh"
 
 using namespace gh;
 
@@ -314,11 +315,17 @@ int main(int argc, char** argv)
 
     // ---- validation and parameter log, in the reference's order (garlic-main.cpp:39-183) ----
     const bool bed = o.bfile != "none", vcf = o.vcf != "none";
+    const bool call_filter = o.vcf_min_gq > 0 || o.vcf_min_dp > 0;
     if (vcf) {
         if (o.tped != "none" || bed) { LOG.error("ERROR: Provide exactly one input: --tped/--tfam, --bfile or --vcf."); return -1; }
         if (o.host_tokenize) { LOG.error("ERROR: --host-tokenize applies to tped input only, not to --vcf."); return -1; }
         LOG.line("VCF file: " + o.vcf);
         if (o.tfam != "none") LOG.line("TFAM file: " + o.tfam);
+        if (o.vcf_min_gq > 0) LOG.line("Minimum genotype quality (GQ) of a call: " + std::to_string(o.vcf_min_gq));
+        if (o.vcf_min_dp > 0) LOG.line("Minimum read depth (DP) of a call: " + std::to_string(o.vcf_min_dp));
+    } else if (call_filter) {
+        LOG.error("ERROR: --vcf-min-gq and --vcf-min-dp apply to --vcf input (VCF or BCF) only, not to --tped or --bfile.");
+        return -1;
     } else if (bed) {
         if (o.tped != "none" || o.tfam != "none") { LOG.error("ERROR: Provide either --bfile or --tped and --tfam, not both."); return -1; }
         if (o.phased) { LOG.error("ERROR: --phased cannot be used with --bfile: a PLINK .bed stores unphased genotypes."); return -1; }
@@ -423,7 +430,8 @@ int main(int argc, char** argv)
     if (!load_centromeres(o.build, o.centromere, c.cen)) return -1;
     std::vector<std::string> a1, a2;                   // .bim allele names (--bfile)
     Vcf vc;                                            // VCF samples and allele names (--vcf)
-    if (vcf ? !load_vcf(o.vcf, c.tped, vc)
+    const unsigned call_keys = (o.vcf_min_gq > 0 ? 1u : 0u) | (o.vcf_min_dp > 0 ? 2u : 0u);
+    if (vcf ? !load_vcf(o.vcf, c.tped, vc, call_keys)
             : bed ? !load_bim(o.bfile + ".bim", c.tped, a1, a2) : !load_tped(o.tped, o.tped_missing, c.tped, o.host_tokenize)) return 1;
     Tped& t = c.tped;
     LOG.line("Total loci: " + std::to_string(t.n_loci));
@@ -543,6 +551,42 @@ int main(int argc, char** argv)
         }
         return "";
     };
+    // the message of record s's first malformed GQ / DP value, in sample bad (the rule the GPU applied, run here again)
+    auto value_error = [&](int64_t s, int bad) -> std::string {
+        const int32_t k_gq = vc.fmt_index[2 * s], k_dp = vc.fmt_index[2 * s + 1];
+        int field = 0;
+        std::string value;
+        if (bcf) {
+            const unsigned char* p = (const unsigned char*)vc.fv.data() + vc.fv_off[s];
+            for (int f = 1; f >= 0; --f) {                  // GQ is named when both are malformed
+                const int32_t at = vc.fv_pos[2 * s + f], type = vc.fv_type[2 * s + f] & 15, w = type == 1 ? 1 : type == 2 ? 2 : 4;
+                if (at < 0) continue;
+                const unsigned char* q = p + at + (int64_t)bad * w;
+                const int32_t raw = w == 1 ? (int8_t)q[0] : w == 2 ? (int16_t)(q[0] | q[1] << 8) : (int32_t)(q[0] | q[1] << 8 | q[2] << 16 | (uint32_t)q[3] << 24);
+                if (garlic::bcf_value(raw, type, f ? o.vcf_min_dp : o.vcf_min_gq) < 0) {
+                    field = f;
+                    char hex[16];
+                    snprintf(hex, sizeof(hex), "0x%08x", (unsigned)raw);
+                    value = hex;
+                }
+            }
+            return vcf_record(s) + "the " + (field ? "DP" : "GQ") + " of sample " + vc.samples[bad] + " is float " + value +
+                   ", an infinity or NaN that is not the missing value.";
+        }
+        const char* p = t.text.data() + t.text_off[s];
+        const char* e = t.text.data() + t.text_off[s + 1];
+        for (int i = 0; i < bad && p < e; ++i) { const char* tab = (const char*)memchr(p, '\t', e - p); p = tab ? tab + 1 : e; }
+        garlic::call_filter(p, e - p, k_gq, o.vcf_min_gq, k_dp, o.vcf_min_dp, &field);
+        const int k = field ? k_dp : k_gq;
+        for (int i = 0; i < k && p < e; ++i) {
+            while (p < e && *p != ':' && *p != '\t') ++p;
+            if (p < e && *p == ':') ++p;
+        }
+        const char* ve = p;
+        while (ve < e && *ve != ':' && *ve != '\t') ++ve;
+        return vcf_record(s) + "the " + (field ? "DP" : "GQ") + " of sample " + vc.samples[bad] + " (" + std::string(p, ve) +
+               ") is not a number: digits with an optional '-' and decimal part, or '.'.";
+    };
     if (!team.all([&](Rank& R) {
             if (garlic_gpu_create(o.device + R.rank, &R.g)) { R.err = "no usable CUDA device " + std::to_string(o.device + R.rank) + "; garlic_b200 has no CPU path"; return false; }
             if (G > 1 && !rank_ok(R, garlic_gpu_comm_init(R.g, comm_id, R.rank, G), "comm_init")) return false;
@@ -550,24 +594,32 @@ int main(int argc, char** argv)
             if (!rank_ok(R, garlic_gpu_set_shape(R.g, n, R.lo, t.n_loci, C, t.chr_off.data(), t.pos.data()), "set_shape")) return false;
             // --by-pop: every rank parses every input column and keeps its own individuals of the population
             if (sel && !rank_ok(R, garlic_gpu_select_columns(R.g, cols.data() + R.lo, t.n_ind), "select_columns")) return false;
+            if (call_filter && !rank_ok(R, garlic_gpu_set_call_filter(R.g, o.vcf_min_gq, o.vcf_min_dp), "set_call_filter")) return false;
             std::vector<uint8_t> slice;
             std::vector<int32_t> nb;
-            std::vector<int32_t> nc, mx, bc;
+            std::vector<int32_t> nc, mx, bc, bv;
             for (int64_t s0 = 0; s0 < t.n_loci && vcf; s0 += blk) {
                 // the VCF sample columns (or the BCF GT vectors) go to every rank, which keeps its own individuals'
                 // allele indices; every rank parses every sample, so each finds the same malformed records
                 const int ns = (int)std::min(blk, t.n_loci - s0);
-                nc.resize(ns); mx.resize(ns); bc.resize(ns);
-                if (bcf ? !rank_ok(R, garlic_gpu_put_bcf_gt(R.g, (const uint8_t*)t.text.data(), t.text_off.data() + s0, vc.gt_type.data() + s0,
-                                                            t.n_ind, s0, ns, mx.data(), bc.data()), "put_bcf_gt")
-                        : !rank_ok(R, garlic_gpu_put_vcf_text(R.g, t.text.data(), t.text_off.data() + s0, s0, ns, nc.data(), mx.data(), bc.data()),
-                                   "put_vcf_text")) return false;
+                nc.resize(ns); mx.resize(ns); bc.resize(ns); bv.assign(ns, -1);
+                const int rc = call_filter
+                    ? (bcf ? garlic_gpu_put_bcf_gt_filtered(R.g, (const uint8_t*)t.text.data(), t.text_off.data() + s0, vc.gt_type.data() + s0,
+                                                            t.n_ind, s0, ns, vc.fv.data(), vc.fv_off.data() + s0, vc.fv_pos.data() + 2 * s0,
+                                                            vc.fv_type.data() + 2 * s0, mx.data(), bc.data(), bv.data())
+                           : garlic_gpu_put_vcf_text_filtered(R.g, t.text.data(), t.text_off.data() + s0, s0, ns, vc.fmt_index.data() + 2 * s0,
+                                                              nc.data(), mx.data(), bc.data(), bv.data()))
+                    : (bcf ? garlic_gpu_put_bcf_gt(R.g, (const uint8_t*)t.text.data(), t.text_off.data() + s0, vc.gt_type.data() + s0,
+                                                   t.n_ind, s0, ns, mx.data(), bc.data())
+                           : garlic_gpu_put_vcf_text(R.g, t.text.data(), t.text_off.data() + s0, s0, ns, nc.data(), mx.data(), bc.data()));
+                if (!rank_ok(R, rc, bcf ? "put_bcf_gt" : "put_vcf_text")) return false;
                 for (int k = 0; k < ns; ++k) {
                     if (!bcf && nc[k] != t.n_ind) {
                         R.err = vcf_record(s0 + k) + std::to_string(nc[k]) + " sample columns, but the #CHROM header names " + std::to_string(t.n_ind) + " samples.";
                         return false;
                     }
                     R.err = vcf_record_error(s0 + k, bc[k], mx[k]);
+                    if (R.err.empty() && bv[k] >= 0) R.err = value_error(s0 + k, bv[k]);
                     if (!R.err.empty()) return false;
                 }
             }
@@ -660,6 +712,15 @@ int main(int argc, char** argv)
         }
     }
     c.g = team.ranks[0].g;
+    if (call_filter) {
+        uint64_t n_set = 0;
+        for (Rank& R : team.ranks) n_set += garlic_gpu_calls_set_missing(R.g);
+        int64_t lacking = 0;
+        for (int64_t s = 0; s < t.n_loci; ++s)
+            lacking += (o.vcf_min_gq > 0 && vc.fmt_index[2 * s] < 0) || (o.vcf_min_dp > 0 && vc.fmt_index[2 * s + 1] < 0);
+        LOG.line("Calls set missing by the GQ/DP filter: " + std::to_string(n_set) + "; records whose FORMAT lacks " +
+                 (o.vcf_min_gq > 0 && o.vcf_min_dp > 0 ? "GQ or DP" : o.vcf_min_gq > 0 ? "GQ" : "DP") + ": " + std::to_string(lacking));
+    }
     if (last_pop) {                                    // the parsed input stays on the host until the last population
         std::vector<uint8_t>().swap(t.alleles);
         std::vector<char>().swap(t.text);

@@ -133,6 +133,35 @@ int garlic_gpu_put_vcf_text(garlic_gpu_t *h, const char *text, const int64_t *li
  * synchronises (the caller may reuse its buffers).  garlic_gpu_code_alleles then codes the block with missing = 255. */
 int garlic_gpu_put_bcf_gt(garlic_gpu_t *h, const uint8_t *gt, const int64_t *rec_off, const uint8_t *gt_type,
                           int n_samples, int64_t snp0, int n_snp, int32_t *max_allele, int32_t *bad_sample);
+/* Call filter of VCF / BCF input (--vcf-min-gq / --vcf-min-dp): a call whose FORMAT GQ is below min_gq, or whose DP is
+ * below min_dp, is stored as two missing alleles, so a filtered put means exactly the unfiltered put of the file in
+ * which every such call is written ./. (0 = that filter off; both 0 = no filter).  A missing value passes: '.', an
+ * empty or omitted trailing subfield, a record without the key, the BCF missing and end-of-vector values.  Call it
+ * after set_shape (which turns the filter off) and before the first put_*; it resets the count of calls set missing.
+ * Only the _filtered puts below apply it; put_vcf_text and put_bcf_gt never filter. */
+int garlic_gpu_set_call_filter(garlic_gpu_t *h, int min_gq, int min_dp);
+/* put_vcf_text with the call filter.  fmt_index[2*l] / [2*l+1] = the FORMAT index (GT = 0) of GQ / DP in record l,
+ * -1 if its FORMAT lacks the key.  A value is an optional '-', digits, then optionally '.' and digits (I.F passes iff
+ * I >= the threshold), or missing; anything else is malformed while its filter is on.  bad_value[l] (may be NULL) =
+ * the first sample of record l with a malformed GQ or DP, -1 if none; the GT checks (bad_col, max_allele) apply to
+ * every call as written, filtered or not. */
+int garlic_gpu_put_vcf_text_filtered(garlic_gpu_t *h, const char *text, const int64_t *line_off, int64_t snp0, int n_snp,
+                                     const int32_t *fmt_index, int32_t *n_cols, int32_t *max_allele, int32_t *bad_col,
+                                     int32_t *bad_value);
+/* put_bcf_gt with the call filter.  Record l's GQ and DP vectors lie in fv[fv_off[l], fv_off[l+1]) (fv_off: n_snp + 1
+ * ascending entries, multiples of 4): GQ at fv + fv_off[l] + fv_pos[2*l], DP at + fv_pos[2*l+1] (multiples of 4, -1 if
+ * the record lacks the key), with descriptors fv_type[2*l] / [2*l+1].  A filtered field must have count 1 and type
+ * int8, int16, int32 or float (5), else the call fails naming the record.  Integers other than the missing / end-of-
+ * vector values compare as integers; a float must be finite or one of its two sentinels (0x7F800001, 0x7F800002), an
+ * other NaN or an infinity is malformed.  fv may be NULL when fv_off[n_snp] == fv_off[0] (no record of the block holds
+ * a GQ or DP vector: every call passes).  bad_value[l] (may be NULL) as for put_vcf_text_filtered. */
+int garlic_gpu_put_bcf_gt_filtered(garlic_gpu_t *h, const uint8_t *gt, const int64_t *rec_off, const uint8_t *gt_type,
+                                   int n_samples, int64_t snp0, int n_snp, const uint8_t *fv, const int64_t *fv_off,
+                                   const int32_t *fv_pos, const uint8_t *fv_type, int32_t *max_allele, int32_t *bad_sample,
+                                   int32_t *bad_value);
+/* calls of this handle's individuals with at least one present allele that the call filter set missing, since
+ * set_call_filter (a call already ./. is not counted) */
+uint64_t garlic_gpu_calls_set_missing(const garlic_gpu_t *h);
 int garlic_gpu_code_alleles(garlic_gpu_t *h);
 
 /* ---- pre-coded input: packed 2-bit rows (codes 0/1/2, 3 = missing) -------------------------
